@@ -806,12 +806,12 @@ bool nm_extrema_make_tma(NmBlurTma* t, const NmOctave& oc, int batch)
 }
 
 // Split pipeline (default): extrema_kernel here, gradmap_kernel after the compaction.  The fused round-1 kernel
-// stays as the path for levels TMA cannot describe and behind NM_EXTREMA_FUSED=1 (A/B measurements); it writes
-// dense gradient maps itself.  Returns through *fused which one ran.
+// stays as the path for levels TMA cannot describe; it writes dense gradient maps itself.  NM_EXTREMA_FUSED=1 forces
+// it (test hook: the parity tests are re-run on this path).  Returns through *fused which one ran.
 static bool extrema_use_fused(const NmBlurTma* tma)
 {
     static const bool forced = getenv("NM_EXTREMA_FUSED") != nullptr;
-    return forced || !(tma && tma->valid) || getenv("NM_EXTREMA_NO_TMA") != nullptr;
+    return forced || !(tma && tma->valid);
 }
 
 bool nm_extrema_is_fused(const NmBlurTma* tma) { return extrema_use_fused(tma); }
@@ -837,15 +837,14 @@ int nm_extrema_launch(const NmOctave& oc, int, int, const NmDetectParams& dp, in
         if (n_tiles >= (1LL << 31) / EX2_LIST || !oc.cand_n || !oc.cand) return NM_ERR_OVERFLOW;
         // 4x the resident count: co-resident CTAs do not advance evenly, and with exactly-resident persistent CTAs the
         // launch ends on half-empty SMs; the hardware hands an SM its next CTA as one retires (64 x 1080p: 1.27 -> 1.21 ms,
-        // 2x 1.23, 8x 1.21).  NM_EXTREMA_OVER overrides (tuning aid).
-        static const int over = getenv("NM_EXTREMA_OVER") ? atoi(getenv("NM_EXTREMA_OVER")) : 4;
-        const long long want = (long long)n_sms * ctas_per_sm * (over < 1 ? 1 : over);
+        // 2x 1.23, 8x 1.21; B200).
+        const long long want = (long long)n_sms * ctas_per_sm * 4;
         const int ctas = (int)(n_tiles < want ? n_tiles : want);
         extrema_kernel<<<ctas, block, EX2_SMEM, stream>>>(oc, dp, tma->map, (int)grid.x, (int)grid.y, (int)n_tiles, oc.cand_n, oc.cand);
         NM_LAUNCH_CHECK();
         refine_list_kernel<<<(unsigned)nm_div_up64(n_tiles, 8), 256, 0, stream>>>(oc, dp, (int)grid.x, (int)grid.y, (int)n_tiles,
                                                                                 oc.cand_n, oc.cand);
-    } else if (tma && tma->valid && getenv("NM_EXTREMA_NO_TMA") == nullptr) {
+    } else if (tma && tma->valid) {
         extrema_grad_kernel<true><<<grid, block, 0, stream>>>(oc, dp, tma->map);
     } else {
         CUtensorMap none{};

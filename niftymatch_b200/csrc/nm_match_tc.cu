@@ -38,8 +38,6 @@
 #include <cuda_fp16.h>
 #include <float.h>
 #include <math.h>
-#include <stdio.h>
-#include <stdlib.h>
 #include <string.h>
 
 namespace {
@@ -807,8 +805,6 @@ __global__ void __launch_bounds__(256) pairs_rerank_kernel(const float* __restri
     }
 }
 
-uint32_t g_lbo = TC_KSTRIDE, g_sbo = 128;
-
 } // namespace
 
 // Per device: compute capability 10.x, enough opt-in shared memory, and the scan kernel's dynamic shared memory
@@ -828,11 +824,6 @@ bool nm_match_tc_available()
               smem >= TC_SMEM_BYTES;
     if (ok) ok = cudaFuncSetAttribute(tc_scan_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, TC_SMEM_BYTES) == cudaSuccess;
     if (!ok) cudaGetLastError();
-    // bring-up aid: NM_TC_DESC="lbo,sbo" overrides the descriptor strides (bytes)
-    if (const char* env = getenv("NM_TC_DESC")) {
-        unsigned l = 0, b = 0;
-        if (sscanf(env, "%u,%u", &l, &b) == 2) { g_lbo = l; g_sbo = b; }
-    }
     if (dev >= 0 && dev < 64) state[dev].store(ok ? 1 : -1, std::memory_order_release);
     return ok;
 }
@@ -920,11 +911,11 @@ static int tc_run(const float* A, int nA, const float* B, int nB, int index_offs
         tc_absmax_kernel<<<ga + gb, 256, 0, stream>>>(A, ea4, ga, B, eb4, hdr);
         tc_pack_kernel<<<n_atiles + n_btiles, 256, 0, stream>>>(A, nA, n_atiles, a_pack, B, nB, b_pack, hdr);
         if (seed_tiles > 0) {
-            TcScanArgs ss{a_pack, b_pack, seed_s, seed_i, nullptr, nullptr, nA, 0, seed_tiles, seed_tiles, g_lbo, g_sbo, nullptr, 0};
+            TcScanArgs ss{a_pack, b_pack, seed_s, seed_i, nullptr, nullptr, nA, 0, seed_tiles, seed_tiles, TC_KSTRIDE, 128, nullptr, 0};
             tc_scan_kernel<<<dim3(n_rowblocks, 1), TC_THREADS, TC_SMEM_BYTES, stream>>>(ss);
         }
         TcScanArgs sa{a_pack, b_pack, cand_s, cand_i, seed_tiles > 0 ? seed_s : nullptr, seed_tiles > 0 ? seed_i : nullptr,
-                      nA, seed_tiles, n_btiles, tiles_per_split, g_lbo, g_sbo, nullptr, 0};
+                      nA, seed_tiles, n_btiles, tiles_per_split, TC_KSTRIDE, 128, nullptr, 0};
         tc_scan_kernel<<<dim3(n_rowblocks, n_splits), TC_THREADS, TC_SMEM_BYTES, stream>>>(sa);
         tc_rerank_kernel<<<nm_div_up(nA, 8), 256, 0, stream>>>(A, nA, B, nB, n_lists, cand_s, cand_i, hdr, index_offset, rec4,
                                                                fb_list, fb_count);
@@ -991,7 +982,7 @@ extern "C" int nm_match_pairs_f32(const float* desc, const int* counts_dev, int 
     if (e == cudaSuccess) {
         pairs_absmax_kernel<<<dim3(32, n_frames), 256, 0, stream>>>(desc, counts_dev, capacity, hdr);
         pairs_pack_kernel<<<dim3(tiles, n_frames), 256, 0, stream>>>(desc, counts_dev, capacity, ws + off_ap, ws + off_bp, hdr, fhdr);
-        TcScanArgs sa{ws + off_ap, ws + off_bp, cand_s, cand_i, nullptr, nullptr, 0, 0, 0, 0, g_lbo, g_sbo, counts_dev, capacity};
+        TcScanArgs sa{ws + off_ap, ws + off_bp, cand_s, cand_i, nullptr, nullptr, 0, 0, 0, 0, TC_KSTRIDE, 128, counts_dev, capacity};
         tc_scan_kernel<<<dim3(rowblocks, n_splits, n_pairs), TC_THREADS, TC_SMEM_BYTES, stream>>>(sa);
         pairs_rerank_kernel<<<dim3(capacity / 8, n_pairs), 256, 0, stream>>>(desc, counts_dev, capacity, n_lists, cand_s, cand_i, hdr,
                                                                             fhdr, ambiguity, match_out,

@@ -14,7 +14,6 @@
 // 16x16 chunks of the descriptor window, no normalisation (SURVEY.md Q5,Q6,Q10,Q12,Q16).
 #include "nm_sift_internal.cuh"
 #include "nm_kpgeom.cuh"
-#include <cstdlib>
 
 namespace {
 
@@ -24,18 +23,6 @@ __device__ __forceinline__ float exp2f_approx(float x)
     asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(x));
     return r;
 }
-
-// Packed fp32 pairs (Blackwell FADD2 / FMUL2 / FFMA2: two independent IEEE operations per instruction).  A packed
-// instruction holds the FMA pipe for two cycles but takes ONE issue slot, and instructions of the other pipes issue
-// in its shadow (tools/fma_probe.cu: 8 FFMA2 + 8 LOP3 per round take 17 cycles, 16 FFMA + 8 LOP3 take 26) -- in the
-// issue-bound gather kernels that is where the floating-point half of the instruction count goes.
-typedef unsigned long long nm_f2;
-__device__ __forceinline__ nm_f2 pk2(float lo, float hi) { nm_f2 r; asm("mov.b64 %0, {%1, %2};" : "=l"(r) : "f"(lo), "f"(hi)); return r; }
-__device__ __forceinline__ void upk2(nm_f2 v, float& lo, float& hi) { asm("mov.b64 {%0, %1}, %2;" : "=f"(lo), "=f"(hi) : "l"(v)); }
-__device__ __forceinline__ nm_f2 fma2(nm_f2 a, nm_f2 b, nm_f2 c) { nm_f2 d; asm("fma.rn.f32x2 %0, %1, %2, %3;" : "=l"(d) : "l"(a), "l"(b), "l"(c)); return d; }
-__device__ __forceinline__ nm_f2 add2(nm_f2 a, nm_f2 b) { nm_f2 d; asm("add.rn.f32x2 %0, %1, %2;" : "=l"(d) : "l"(a), "l"(b)); return d; }
-__device__ __forceinline__ nm_f2 sub2(nm_f2 a, nm_f2 b) { nm_f2 d; asm("sub.rn.f32x2 %0, %1, %2;" : "=l"(d) : "l"(a), "l"(b)); return d; }
-__device__ __forceinline__ nm_f2 mul2(nm_f2 a, nm_f2 b) { nm_f2 d; asm("mul.rn.f32x2 %0, %1, %2;" : "=l"(d) : "l"(a), "l"(b)); return d; }
 
 constexpr int OR_WARPS = 8;      // warps per block, orientation
 constexpr int NBINS = 36;
@@ -205,11 +192,10 @@ constexpr int DE_BINS = 128;
 constexpr int DE_COPIES = 16;    // private histogram copies per warp (lanes l, l + 16 share one): 8 KB per keypoint
                                  // in flight instead of 16 -> twice the resident warps (the kernel is latency bound)
 
-// EXACT = the reference's mixed double/float expression shapes (descriptor.cu:98-115, with
-// the DFMA contractions of its sm_100a SASS); !EXACT = the same formulas in fp32 (the bins
-// and trilinear weights are continuous in nx, ny, nt, so the fp32 evaluation stays within
-// ~1e-6 relative of the exact one; the tolerance is 1e-3, BASELINE.json).
-template <bool EXACT>
+// Exact mode: the reference's mixed double/float expression shapes (descriptor.cu:98-115, with
+// the DFMA contractions of its sm_100a SASS).  describe_fast_kernel below evaluates the same
+// formulas in fp32 (the bins and trilinear weights are continuous in nx, ny, nt, so the fp32
+// evaluation stays within ~1e-6 relative of the exact one; the tolerance is 1e-3, BASELINE.json).
 __global__ void __launch_bounds__(DE_WARPS * 32) describe_kernel(const NmOctaveTable tab, int capacity,
                                                                  const int* __restrict__ counts,
                                                                  const float4* __restrict__ kpts,
@@ -242,7 +228,6 @@ __global__ void __launch_bounds__(DE_WARPS * 32) describe_kernel(const NmOctaveT
                                                                                          // so gradient angle - th0 is in (-2 pi, 2 pi + 1]
     const float st0f = sinf(th0), ct0f = cosf(th0);                                      // :90-91 (float overloads)
     const double st0 = (double)st0f, ct0 = (double)ct0f;
-    const float inv_sbp = __fdiv_rn(1.0f, SBP);
     const float2* __restrict__ G = oc.grad + ((long long)f * 3 + g.level) * oc.level_elems +
                                    (long long)g.yi * oc.pitch + g.xi;
     const int total = chunks * 256;
@@ -256,37 +241,19 @@ __global__ void __launch_bounds__(DE_WARPS * 32) describe_kernel(const NmOctaveT
         return s < total && cx <= xmax && cy <= ymax;             // :96
     };
     // one sample: rotate into the keypoint frame, weight, spread into the 2 x 2 x 2 neighbouring bins
-    auto process = [&](const int cx, const int cy, const float2 gv, const bool valid) {
-        bool act = valid;
+    auto process = [&](const int cx, const int cy, const float2 gv, const bool act) {
         const float mod = gv.x;
         const float dx = __fsub_rn((float)(g.xi + cx), g.x);          // :102-103
         const float dy = __fsub_rn((float)(g.yi + cy), g.y);
-        float nx, ny, nt, win, rbinx, rbiny;
-        int binx, biny;
-        if (EXACT) {
-            const float theta = nm_mod_2pi_once(__fsub_rn(gv.y, th0));                                       // :100
-            nx = (float)__ddiv_rn(__fma_rn(ct0, (double)dx, __dmul_rn(st0, (double)dy)), (double)SBP);    // :104
-            ny = (float)__ddiv_rn(__fma_rn(ct0, (double)dy, -__dmul_rn(st0, (double)dx)), (double)SBP);   // :105
-            nt = (float)__ddiv_rn((double)__fmul_rn(8.0f, theta), NM_TWO_PI_D);                           // :107
-            win = (float)exp(__dmul_rn((double)__fmaf_rn(nx, nx, __fmul_rn(ny, ny)), 0.125));             // :108
-            binx = (int)floor(__dadd_rn((double)nx, -0.5));                                               // :110
-            biny = (int)floor(__dadd_rn((double)ny, -0.5));
-            rbinx = (float)__dsub_rn((double)nx, __dadd_rn((double)binx, 0.5));                           // :113
-            rbiny = (float)__dsub_rn((double)ny, __dadd_rn((double)biny, 0.5));
-        } else {
-            nx = __fmul_rn(__fmaf_rn(ct0f, dx, __fmul_rn(st0f, dy)), inv_sbp);
-            ny = __fmul_rn(__fmaf_rn(ct0f, dy, -__fmul_rn(st0f, dx)), inv_sbp);
-            const float fx = floorf(__fsub_rn(nx, 0.5f)), fy = floorf(__fsub_rn(ny, 0.5f));
-            binx = (int)fx; biny = (int)fy;
-            // about a third of the window (corners outside the rotated 4x4 cell grid) lands in no
-            // bin (:122-125 rejects all four cells): skip before the exponential and the angle
-            act = act && !(binx < -3 || binx > 1 || biny < -3 || biny > 1);
-            const float theta = nm_mod_2pi_once(__fsub_rn(gv.y, th0));   // :100
-            nt = __fmul_rn(theta, 1.2732395447351628f);               // 8 / (2 pi)
-            win = expf(__fmul_rn(__fmaf_rn(nx, nx, __fmul_rn(ny, ny)), 0.125f));
-            rbinx = __fsub_rn(nx, __fadd_rn(fx, 0.5f));
-            rbiny = __fsub_rn(ny, __fadd_rn(fy, 0.5f));
-        }
+        const float theta = nm_mod_2pi_once(__fsub_rn(gv.y, th0));                                             // :100
+        const float nx = (float)__ddiv_rn(__fma_rn(ct0, (double)dx, __dmul_rn(st0, (double)dy)), (double)SBP);  // :104
+        const float ny = (float)__ddiv_rn(__fma_rn(ct0, (double)dy, -__dmul_rn(st0, (double)dx)), (double)SBP); // :105
+        const float nt = (float)__ddiv_rn((double)__fmul_rn(8.0f, theta), NM_TWO_PI_D);                         // :107
+        const float win = (float)exp(__dmul_rn((double)__fmaf_rn(nx, nx, __fmul_rn(ny, ny)), 0.125));           // :108
+        const int binx = (int)floor(__dadd_rn((double)nx, -0.5));                                               // :110
+        const int biny = (int)floor(__dadd_rn((double)ny, -0.5));
+        const float rbinx = (float)__dsub_rn((double)nx, __dadd_rn((double)binx, 0.5));                         // :113
+        const float rbiny = (float)__dsub_rn((double)ny, __dadd_rn((double)biny, 0.5));
         const int bint = (int)floorf(nt);                             // :112
         const float rbint = __fsub_rn(nt, (float)bint);               // :115
         const float wm = __fmul_rn(win, mod);                         // :128-129 (left to right)
@@ -368,32 +335,35 @@ __global__ void __launch_bounds__(DE_WARPS * 32) describe_kernel(const NmOctaveT
     if (lane == 0) { xo[kidx] = kp.x; yo[kidx] = kp.y; }              // :76
 }
 
-// ------------------------------- descriptor, fp32 mode, restructured -----------------------------------
-// Same formulas as describe_kernel<false>; what changes is the instruction count per sample (the kernel is
-// issue bound: ncu counted 135 warp instructions per 32 samples, 5 350 per keypoint):
+// ------------------------------- descriptor, fp32 mode -----------------------------------
+// The descriptor formulas in fp32, arranged for a low instruction count per sample (the kernel is issue bound: the
+// round-1 fp32 kernel, which walked the window one flat sample index at a time, took 135 warp instructions per 32
+// samples, 5 350 per keypoint):
 //   * the window is walked chunk by chunk and row by row (lane = column (0..15) + 16 * (row & 1), eight row steps
 //     per 16 x 16 chunk), so sample positions, validity and gradient addresses are increments, not a decode of a
 //     flat sample index; the eight gradient loads of the NEXT chunk are issued before the current chunk's
 //     arithmetic;
 //   * the rotation into the keypoint frame is folded with the 1 / SBP scale: nx = sn * dy + (cs * dx), one FFMA per
 //     coordinate with the per-chunk terms hoisted;
-//   * exp(r2 / 8) through ex2.approx (2 ulp; the tolerance is 1e-3), contributions added with one FFMA each;
-//   * COPIES = 32: one private histogram copy per lane, a single accumulation phase (16 KB per keypoint in flight);
-//     COPIES = 16: lanes l and l + 16 share a copy and take turns (8 KB).
+//   * exp(r2 / 8) through ex2.approx (2 ulp; the tolerance is 1e-3), contributions added with one FFMA each.
 // Reduction order over the copies is fixed, so the output is bit-reproducible run to run.
-template <int COPIES, int WARPS, bool PACKED, int MINB = 0>
-__global__ void __launch_bounds__(WARPS * 32, MINB) describe_fast_kernel(const NmOctaveTable tab, int capacity,
-                                                                      const int* __restrict__ counts,
-                                                                      const float4* __restrict__ kpts,
-                                                                      const int* __restrict__ meta,
-                                                                      const float2* __restrict__ orient,
-                                                                      float* __restrict__ desc, float* __restrict__ xo,
-                                                                      float* __restrict__ yo, int num_dogs)
+// Variants measured on a B200 with 64 x 1080p frames, against this kernel's 1.54 ms: the round-1 kernel 2.26 ms;
+// without the skip of sample rows that have no active lane 1.63; two passes of 16 lanes instead of the split by bin
+// parity 1.87; a test of the row against ymax before the sample arithmetic 1.60; packed fp32 pairs (FFMA2) for the
+// sample arithmetic 1.71 (1.84 without the row skip); 32 histogram copies, one per lane, 1.97 (2.03 packed, 1.96 in
+// two-warp CTAs); register caps for 6 / 7 CTAs per SM 1.88 - 2.28.
+__global__ void __launch_bounds__(DE_WARPS * 32) describe_fast_kernel(const NmOctaveTable tab, int capacity,
+                                                                     const int* __restrict__ counts,
+                                                                     const float4* __restrict__ kpts,
+                                                                     const int* __restrict__ meta,
+                                                                     const float2* __restrict__ orient,
+                                                                     float* __restrict__ desc, float* __restrict__ xo,
+                                                                     float* __restrict__ yo, int num_dogs)
 {
-    extern __shared__ __align__(16) float s_h[];      // [WARPS][128 bins][COPIES]
+    extern __shared__ __align__(16) float s_h[];      // [DE_WARPS][128 bins][DE_COPIES]
     const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
     const int f = blockIdx.y;
-    const int j = blockIdx.x * WARPS + wid;
+    const int j = blockIdx.x * DE_WARPS + wid;
     const long long kidx = (long long)f * capacity + j;
     const int n_kp = counts[f];                                   // fetched together with the slot's payload (see orient_kernel)
     const float4 kp = __ldg(kpts + kidx);
@@ -405,11 +375,11 @@ __global__ void __launch_bounds__(WARPS * 32, MINB) describe_fast_kernel(const N
     float* dout = desc + kidx * DE_BINS;
     if (g.xi < 0 || g.xi >= oc.w || g.yi < 0 || g.yi >= oc.h || g.level < 0 || g.level >= num_dogs)
         return;                                                   // :49 (slot left as is)
-    float* hist = s_h + wid * (DE_BINS * COPIES);
+    float* hist = s_h + wid * (DE_BINS * DE_COPIES);
     {
         float4* h4 = reinterpret_cast<float4*>(hist);
 #pragma unroll
-        for (int b = 0; b < DE_BINS * COPIES / 128; ++b) h4[b * 32 + lane] = make_float4(0.f, 0.f, 0.f, 0.f);
+        for (int b = 0; b < DE_BINS * DE_COPIES / 128; ++b) h4[b * 32 + lane] = make_float4(0.f, 0.f, 0.f, 0.f);
     }
     __syncwarp();
 
@@ -421,7 +391,7 @@ __global__ void __launch_bounds__(WARPS * 32, MINB) describe_fast_kernel(const N
     const int pitch = oc.pitch;
     const float2* __restrict__ G = oc.grad + ((long long)f * 3 + g.level) * oc.level_elems +
                                    (long long)g.yi * pitch + g.xi;             // offsets inside one level fit 32 bits
-    float* const hcopy = hist + (lane & (COPIES - 1));
+    float* const hcopy = hist + (lane & (DE_COPIES - 1));
     const int tx = lane & 15, ty = lane >> 4;
 
     // gradient samples of chunk c for this lane: column xmin + 16 c + tx, rows ymin + 16 c + ty + 2 i (:94-97, :142-143)
@@ -440,105 +410,6 @@ __global__ void __launch_bounds__(WARPS * 32, MINB) describe_fast_kernel(const N
         const float dx = __fsub_rn((float)(g.xi + bx), g.x);                   // :102
         const float ax = __fmul_rn(cs, dx), ay = -__fmul_rn(sn, dx);
         const float fy0 = (float)(g.yi + by);
-        if (PACKED) {
-            // two samples of the lane (rows 2 i and 2 i + 2 below the chunk's first row) per packed instruction
-            const nm_f2 sn2 = pk2(sn, sn), cs2 = pk2(cs, cs), ax2 = pk2(ax, ax), ay2 = pk2(ay, ay);
-            const nm_f2 gy2 = pk2(g.y, g.y), th2 = pk2(th0, th0), half2v = pk2(0.5f, 0.5f), one2 = pk2(1.f, 1.f);
-#pragma unroll
-            for (int ip = 0; ip < 4; ++ip) {
-                const int i0 = 2 * ip, i1 = 2 * ip + 1;
-                const nm_f2 dy2 = sub2(pk2(__fadd_rn(fy0, (float)(2 * i0)), __fadd_rn(fy0, (float)(2 * i1))), gy2);   // :103
-                const nm_f2 nx2 = fma2(sn2, dy2, ax2), ny2 = fma2(cs2, dy2, ay2);                            // :104-105
-                const nm_f2 ux2 = sub2(nx2, half2v), uy2 = sub2(ny2, half2v);
-                float ux[2], uy[2];
-                upk2(ux2, ux[0], ux[1]); upk2(uy2, uy[0], uy[1]);
-                const float fx[2] = {floorf(ux[0]), floorf(ux[1])}, fy[2] = {floorf(uy[0]), floorf(uy[1])};   // :110-111
-                const nm_f2 rbx2 = sub2(nx2, add2(pk2(fx[0], fx[1]), half2v));                               // :113-114
-                const nm_f2 rby2 = sub2(ny2, add2(pk2(fy[0], fy[1]), half2v));
-                // theta = mod_2pi(angle - th0) (:100), nt = 8 theta / 2 pi (:107)
-                float th[2];
-                upk2(sub2(pk2(cur[i0].y, cur[i1].y), th2), th[0], th[1]);
-                th[0] = nm_mod_2pi_once(th[0]); th[1] = nm_mod_2pi_once(th[1]);
-                const nm_f2 nt2 = mul2(pk2(th[0], th[1]), pk2(1.2732395447351628f, 1.2732395447351628f));
-                float nt[2];
-                upk2(nt2, nt[0], nt[1]);
-                const float ft[2] = {floorf(nt[0]), floorf(nt[1])};
-                const nm_f2 rbt2 = sub2(nt2, pk2(ft[0], ft[1]));                                             // :115
-                const nm_f2 r22 = fma2(nx2, nx2, mul2(ny2, ny2));
-                float e[2];
-                upk2(mul2(r22, pk2(0.18033688011112042f, 0.18033688011112042f)), e[0], e[1]);
-                const nm_f2 wm2 = mul2(pk2(exp2f_approx(e[0]), exp2f_approx(e[1])), pk2(cur[i0].x, cur[i1].x));   // :108, :128-129
-                const nm_f2 a12 = mul2(wm2, rbx2), a02 = sub2(wm2, a12);
-                const nm_f2 w012 = mul2(a02, rby2), w002 = sub2(a02, w012);
-                const nm_f2 w112 = mul2(a12, rby2), w102 = sub2(a12, w112);
-                const nm_f2 at02 = sub2(one2, rbt2);
-                float w00[2], w01[2], w10[2], w11[2], at0[2], at1[2];
-                upk2(w002, w00[0], w00[1]); upk2(w012, w01[0], w01[1]); upk2(w102, w10[0], w10[1]); upk2(w112, w11[0], w11[1]);
-                upk2(at02, at0[0], at0[1]); upk2(rbt2, at1[0], at1[1]);
-#pragma unroll
-                for (int u = 0; u < 2; ++u) {
-                    const int i = 2 * ip + u;
-                    const int bx0 = (int)fx[u] + 2, by0 = (int)fy[u] + 2, bint = (int)ft[u];
-                    const bool act = vx && by + 2 * i <= ymax && (unsigned)(bx0 + 1) <= 4u && (unsigned)(by0 + 1) <= 4u;
-                    float* hp = hcopy + (by0 * 32 + bx0 * 8) * COPIES;
-                    float* h0 = hp + (bint & 7) * COPIES;
-                    float* h1 = hp + ((bint + 1) & 7) * COPIES;
-                    constexpr int OX = 8 * COPIES, OY = 32 * COPIES;
-                    const bool vx0 = (unsigned)bx0 < 4u, vx1 = (unsigned)(bx0 + 1) < 4u;
-                    const bool vy0 = (unsigned)by0 < 4u, vy1 = (unsigned)(by0 + 1) < 4u;
-                    const bool p00 = vx0 && vy0, p01 = vx0 && vy1, p10 = vx1 && vy0, p11 = vx1 && vy1;
-                    if (COPIES == 32) {
-                        if (act) {
-                            // the two orientation bins of a cell as one packed FFMA: (v0, v1) += w * (at0, at1)
-                            const nm_f2 at2 = pk2(at0[u], at1[u]);
-                            float v0 = 0.f, v1 = 0.f, v2 = 0.f, v3 = 0.f, v4 = 0.f, v5 = 0.f, v6 = 0.f, v7 = 0.f;
-                            if (p00) { v0 = h0[0]; v1 = h1[0]; }
-                            if (p01) { v2 = h0[OY]; v3 = h1[OY]; }
-                            if (p10) { v4 = h0[OX]; v5 = h1[OX]; }
-                            if (p11) { v6 = h0[OX + OY]; v7 = h1[OX + OY]; }
-                            upk2(fma2(pk2(w00[u], w00[u]), at2, pk2(v0, v1)), v0, v1);                       // :135
-                            upk2(fma2(pk2(w01[u], w01[u]), at2, pk2(v2, v3)), v2, v3);
-                            upk2(fma2(pk2(w10[u], w10[u]), at2, pk2(v4, v5)), v4, v5);
-                            upk2(fma2(pk2(w11[u], w11[u]), at2, pk2(v6, v7)), v6, v7);
-                            if (p00) { h0[0] = v0; h1[0] = v1; }
-                            if (p01) { h0[OY] = v2; h1[OY] = v3; }
-                            if (p10) { h0[OX] = v4; h1[OX] = v5; }
-                            if (p11) { h0[OX + OY] = v6; h1[OX + OY] = v7; }
-                        }
-                    } else {
-                        // 16 copies: lanes l and l + 16 share one.  A sample's two orientation bins have different
-                        // parities, so in the first pass every lane adds to the bin whose parity is its half-warp's
-                        // and in the second to the other one: the two lanes of a copy never meet in a pass, all 32
-                        // lanes work in both (round 2 had two passes of 16 lanes with all eight bins each), and with
-                        // bank = copy + 16 * (bin & 1) each of the four accesses of a pass is conflict free.
-                        const bool sw = ((bint ^ (lane >> 4)) & 1) != 0;
-                        float* pa = sw ? h1 : h0;
-                        float* pb = sw ? h0 : h1;
-                        const float ta = sw ? at1[u] : at0[u], tb = sw ? at0[u] : at1[u];
-#pragma unroll
-                        for (int ph = 0; ph < 2; ++ph) {
-                            float* q = ph ? pb : pa;
-                            const float tq = ph ? tb : ta;
-                            if (act) {
-                                float v0 = 0.f, v1 = 0.f, v2 = 0.f, v3 = 0.f;
-                                if (p00) v0 = q[0];
-                                if (p01) v1 = q[OY];
-                                if (p10) v2 = q[OX];
-                                if (p11) v3 = q[OX + OY];
-                                v0 = __fmaf_rn(w00[u], tq, v0); v1 = __fmaf_rn(w01[u], tq, v1);             // :135
-                                v2 = __fmaf_rn(w10[u], tq, v2); v3 = __fmaf_rn(w11[u], tq, v3);
-                                if (p00) q[0] = v0;
-                                if (p01) q[OY] = v1;
-                                if (p10) q[OX] = v2;
-                                if (p11) q[OX + OY] = v3;
-                            }
-                            __syncwarp();
-                        }
-                    }
-                }
-            }
-            return;
-        }
 #pragma unroll
         for (int i = 0; i < 8; ++i) {
             const float dy = __fsub_rn(__fadd_rn(fy0, (float)(2 * i)), g.y);   // :103 (integers: the sum is exact)
@@ -563,10 +434,10 @@ __global__ void __launch_bounds__(WARPS * 32, MINB) describe_fast_kernel(const N
             const float w01 = __fmul_rn(a0, rbiny), w00 = __fsub_rn(a0, w01);
             const float w11 = __fmul_rn(a1, rbiny), w10 = __fsub_rn(a1, w11);
             const float at1 = rbint, at0 = __fsub_rn(1.f, rbint);
-            float* hp = hcopy + (by0 * 32 + bx0 * 8) * COPIES;                 // only dereferenced for valid cells
-            float* h0 = hp + (bint & 7) * COPIES;                              // :133 (bint + dbt) % 8
-            float* h1 = hp + ((bint + 1) & 7) * COPIES;
-            constexpr int OX = 8 * COPIES, OY = 32 * COPIES;
+            float* hp = hcopy + (by0 * 32 + bx0 * 8) * DE_COPIES;                 // only dereferenced for valid cells
+            float* h0 = hp + (bint & 7) * DE_COPIES;                              // :133 (bint + dbt) % 8
+            float* h1 = hp + ((bint + 1) & 7) * DE_COPIES;
+            constexpr int OX = 8 * DE_COPIES, OY = 32 * DE_COPIES;
             const bool vx0 = (unsigned)bx0 < 4u, vx1 = (unsigned)(bx0 + 1) < 4u;            // :122-125
             const bool vy0 = (unsigned)by0 < 4u, vy1 = (unsigned)(by0 + 1) < 4u;
             // The eight bins of a sample are distinct addresses: all eight loads are issued before the first store, so a
@@ -575,47 +446,32 @@ __global__ void __launch_bounds__(WARPS * 32, MINB) describe_fast_kernel(const N
             // store (the round-1 kernel was bound by exactly that chain: twice the histogram copies, i.e. half the
             // resident warps, made it 2.3x slower).
             const bool p00 = vx0 && vy0, p01 = vx0 && vy1, p10 = vx1 && vy0, p11 = vx1 && vy1;
-            if (COPIES == 32) {
-                if (act) {
-                    float v0 = 0.f, v1 = 0.f, v2 = 0.f, v3 = 0.f, v4 = 0.f, v5 = 0.f, v6 = 0.f, v7 = 0.f;
-                    if (p00) { v0 = h0[0]; v1 = h1[0]; }
-                    if (p01) { v2 = h0[OY]; v3 = h1[OY]; }
-                    if (p10) { v4 = h0[OX]; v5 = h1[OX]; }
-                    if (p11) { v6 = h0[OX + OY]; v7 = h1[OX + OY]; }
-                    v0 = __fmaf_rn(w00, at0, v0); v1 = __fmaf_rn(w00, at1, v1);                                          // :135
-                    v2 = __fmaf_rn(w01, at0, v2); v3 = __fmaf_rn(w01, at1, v3);
-                    v4 = __fmaf_rn(w10, at0, v4); v5 = __fmaf_rn(w10, at1, v5);
-                    v6 = __fmaf_rn(w11, at0, v6); v7 = __fmaf_rn(w11, at1, v7);
-                    if (p00) { h0[0] = v0; h1[0] = v1; }
-                    if (p01) { h0[OY] = v2; h1[OY] = v3; }
-                    if (p10) { h0[OX] = v4; h1[OX] = v5; }
-                    if (p11) { h0[OX + OY] = v6; h1[OX + OY] = v7; }
-                }
-            } else {
-                // 16 copies, two passes by orientation-bin parity (see the packed path above)
-                const bool sw = ((bint ^ (lane >> 4)) & 1) != 0;
-                float* pa = sw ? h1 : h0;
-                float* pb = sw ? h0 : h1;
-                const float ta = sw ? at1 : at0, tb = sw ? at0 : at1;
+            // Lanes l and l + 16 share a copy.  A sample's two orientation bins have different parities, so in the first
+            // pass every lane adds to the bin whose parity is its half-warp's and in the second to the other one: the two
+            // lanes of a copy never meet in a pass, all 32 lanes work in both (round 2 had two passes of 16 lanes with all
+            // eight bins each), and with bank = copy + 16 * (bin & 1) each of the four accesses of a pass is conflict free.
+            const bool sw = ((bint ^ (lane >> 4)) & 1) != 0;
+            float* pa = sw ? h1 : h0;
+            float* pb = sw ? h0 : h1;
+            const float ta = sw ? at1 : at0, tb = sw ? at0 : at1;
 #pragma unroll
-                for (int ph = 0; ph < 2; ++ph) {
-                    float* q = ph ? pb : pa;
-                    const float tq = ph ? tb : ta;
-                    if (act) {
-                        float v0 = 0.f, v1 = 0.f, v2 = 0.f, v3 = 0.f;
-                        if (p00) v0 = q[0];
-                        if (p01) v1 = q[OY];
-                        if (p10) v2 = q[OX];
-                        if (p11) v3 = q[OX + OY];
-                        v0 = __fmaf_rn(w00, tq, v0); v1 = __fmaf_rn(w01, tq, v1);                                        // :135
-                        v2 = __fmaf_rn(w10, tq, v2); v3 = __fmaf_rn(w11, tq, v3);
-                        if (p00) q[0] = v0;
-                        if (p01) q[OY] = v1;
-                        if (p10) q[OX] = v2;
-                        if (p11) q[OX + OY] = v3;
-                    }
-                    __syncwarp();
+            for (int ph = 0; ph < 2; ++ph) {
+                float* q = ph ? pb : pa;
+                const float tq = ph ? tb : ta;
+                if (act) {
+                    float v0 = 0.f, v1 = 0.f, v2 = 0.f, v3 = 0.f;
+                    if (p00) v0 = q[0];
+                    if (p01) v1 = q[OY];
+                    if (p10) v2 = q[OX];
+                    if (p11) v3 = q[OX + OY];
+                    v0 = __fmaf_rn(w00, tq, v0); v1 = __fmaf_rn(w01, tq, v1);                                            // :135
+                    v2 = __fmaf_rn(w10, tq, v2); v3 = __fmaf_rn(w11, tq, v3);
+                    if (p00) q[0] = v0;
+                    if (p01) q[OY] = v1;
+                    if (p10) q[OX] = v2;
+                    if (p11) q[OX + OY] = v3;
                 }
+                __syncwarp();
             }
         }
     };
@@ -636,8 +492,8 @@ __global__ void __launch_bounds__(WARPS * 32, MINB) describe_fast_kernel(const N
         const int b = lane + 32 * q;
         float acc = 0.f;
 #pragma unroll 8
-        for (int k = 0; k < COPIES; ++k)
-            acc = __fadd_rn(acc, hist[b * COPIES + ((k + lane / (32 / COPIES)) & (COPIES - 1))]);   // rotated: conflict free
+        for (int k = 0; k < DE_COPIES; ++k)
+            acc = __fadd_rn(acc, hist[b * DE_COPIES + ((k + lane / (32 / DE_COPIES)) & (DE_COPIES - 1))]);   // rotated: conflict free
         dout[b] = acc;
     }
     if (lane == 0) { xo[kidx] = kp.x; yo[kidx] = kp.y; }              // :76
@@ -668,38 +524,14 @@ int nm_describe_launch(const NmOctaveTable& tab, int batch, int capacity, const 
 {
     static NmDeviceOnce once;
     constexpr int smem = DE_WARPS * DE_BINS * DE_COPIES * (int)sizeof(float);
-    constexpr int smem16 = DE_WARPS * DE_BINS * 16 * (int)sizeof(float), smem32 = DE_WARPS * DE_BINS * 32 * (int)sizeof(float);
     if (once.first()) {
-        NM_CUDA_TRY(cudaFuncSetAttribute(describe_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-        NM_CUDA_TRY(cudaFuncSetAttribute(describe_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-        NM_CUDA_TRY(cudaFuncSetAttribute((describe_fast_kernel<16, DE_WARPS, false>), cudaFuncAttributeMaxDynamicSharedMemorySize, smem16));
-        NM_CUDA_TRY(cudaFuncSetAttribute((describe_fast_kernel<16, DE_WARPS, true>), cudaFuncAttributeMaxDynamicSharedMemorySize, smem16));
-        NM_CUDA_TRY(cudaFuncSetAttribute((describe_fast_kernel<32, DE_WARPS, false>), cudaFuncAttributeMaxDynamicSharedMemorySize, smem32));
-        NM_CUDA_TRY(cudaFuncSetAttribute((describe_fast_kernel<32, DE_WARPS, true>), cudaFuncAttributeMaxDynamicSharedMemorySize, smem32));
-        NM_CUDA_TRY(cudaFuncSetAttribute((describe_fast_kernel<32, 2, false>), cudaFuncAttributeMaxDynamicSharedMemorySize, smem32 / 2));
+        NM_CUDA_TRY(cudaFuncSetAttribute(describe_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+        NM_CUDA_TRY(cudaFuncSetAttribute(describe_fast_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
         once.done();
     }
-    // NM_DESCRIBE (tuning aid; 64 x 1080p): 0: round-1 kernel 2.26 ms; 16 (default): restructured kernel, 16 histogram
-    // copies, two passes by orientation-bin parity, sample rows without an active lane skipped 1.54 (1.63 without the skip; two
-    // passes of 16 lanes: 1.87; a test of the row against ymax before the sample arithmetic: 1.60); 162: the same with packed fp32
-    // pairs for the sample arithmetic 1.71 (1.84); 32 / 323: 32 copies 1.97 / 2.03; 322: 32 copies in two-warp CTAs 1.96;
-    // register caps for 6 / 7 CTAs per SM: 1.88 - 2.28
-    static const int variant = getenv("NM_DESCRIBE") ? atoi(getenv("NM_DESCRIBE")) : 16;
+    const auto kernel = exact ? describe_kernel : describe_fast_kernel;
     dim3 grid(nm_div_up(capacity, DE_WARPS), batch);
-    if (exact)
-        describe_kernel<true><<<grid, DE_WARPS * 32, smem, stream>>>(tab, capacity, counts, kpts, meta, orient, desc, x, y, num_dogs);
-    else if (variant == 32)
-        describe_fast_kernel<32, DE_WARPS, false><<<grid, DE_WARPS * 32, smem32, stream>>>(tab, capacity, counts, kpts, meta, orient, desc, x, y, num_dogs);
-    else if (variant == 322)          // 32 copies, two-warp CTAs: 14 instead of 12 warps per SM
-        describe_fast_kernel<32, 2, false><<<dim3(nm_div_up(capacity, 2), batch), 64, smem32 / 2, stream>>>(tab, capacity, counts, kpts, meta, orient, desc, x, y, num_dogs);
-    else if (variant == 16)
-        describe_fast_kernel<16, DE_WARPS, false><<<grid, DE_WARPS * 32, smem16, stream>>>(tab, capacity, counts, kpts, meta, orient, desc, x, y, num_dogs);
-    else if (variant == 162)          // 16 copies, packed fp32 pairs
-        describe_fast_kernel<16, DE_WARPS, true><<<grid, DE_WARPS * 32, smem16, stream>>>(tab, capacity, counts, kpts, meta, orient, desc, x, y, num_dogs);
-    else if (variant == 323)          // 32 copies, packed fp32 pairs
-        describe_fast_kernel<32, DE_WARPS, true><<<grid, DE_WARPS * 32, smem32, stream>>>(tab, capacity, counts, kpts, meta, orient, desc, x, y, num_dogs);
-    else
-        describe_kernel<false><<<grid, DE_WARPS * 32, smem, stream>>>(tab, capacity, counts, kpts, meta, orient, desc, x, y, num_dogs);
+    kernel<<<grid, DE_WARPS * 32, smem, stream>>>(tab, capacity, counts, kpts, meta, orient, desc, x, y, num_dogs);
     NM_LAUNCH_CHECK();
     return NM_OK;
 }

@@ -27,9 +27,6 @@
 // kernel with plain loads.
 #include "nm_pyramid.cuh"
 #include <mutex>
-#include <vector>
-#include <algorithm>
-#include <cstdio>
 #include <cstring>
 #include <cstdlib>
 
@@ -470,15 +467,9 @@ __global__ void __launch_bounds__(kThreads, 2) blur_strip_kernel(const NmBlurArg
 //   oversubscribed launch, two CTAs per strip (see launch_tile)               1.96 ms
 // Per launch (octave 0, ncu, final): R = 5 188 us, 7 201, 8 (+ decimated copy) 248, 10 247, 13 312 against
 // 216 / 245 / 282 / 303 / 368 for blur_strip_kernel; the HBM floor of a level is 165 us, the FMA floor of R = 13 192 us.
-// The role rotation (rot_div) stays as a tuning aid; the default divisor is so large that no CTA rotates.
-#ifndef NM_STREAM_GR
-#define NM_STREAM_GR 16
-#define NM_STREAM_NS 2
-#define NM_STREAM_NG 2
-#endif
-constexpr int kGR = NM_STREAM_GR;  // rows per group (8 or 16)
-constexpr int kNS = NM_STREAM_NS;  // TMA stages
-constexpr int kNG = NM_STREAM_NG;  // ring slots (2 + 2 of 16 rows: 38 KB of shared memory per CTA, 5 CTAs per SM)
+constexpr int kGR = 16;            // rows per group
+constexpr int kNS = 2;             // TMA stages
+constexpr int kNG = 2;             // ring slots (2 + 2 of 16 rows: 38 KB of shared memory per CTA, 5 CTAs per SM)
 constexpr int kStreamThreads = 128;
 constexpr int kStreamPieces = 32;  // pieces per CTA the schedule table holds
 constexpr int kStreamMaxR = 13;    // 2R+1 float2 accumulators + the row-pass window fit 128 registers up to here
@@ -560,13 +551,10 @@ __host__ __device__ constexpr int stream_min_ctas(int R) { return R <= 10 ? 5 : 
 template <int R, bool DST2>
 __global__ void __launch_bounds__(kStreamThreads, stream_min_ctas(R)) blur_stream_kernel(const NmBlurArgs a, const __grid_constant__ CUtensorMap tmap,
                                                                          const __grid_constant__ StreamTaps taps,
-                                                                         int tiles_x, int cg, int full_rounds, int total,
-                                                                         int rot_div, unsigned long long* trace)
+                                                                         int tiles_x, int cg, int full_rounds, int total)
 {
     constexpr int RA = radius_aligned(R), IP = in_pitch(R), NT = 2 * R + 1;
     constexpr int PRE = (2 * R + kGR - 1) / kGR;
-    unsigned long long t_begin = 0;
-    if (trace != nullptr) asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t_begin));
     extern __shared__ __align__(128) float smem[];
     float* s_in = smem;                                  // [kNS][kGR][IP]
     float* s_ring = smem + kNS * kGR * IP;               // [kNG][kGR][kRowPitch]
@@ -615,8 +603,8 @@ __global__ void __launch_bounds__(kStreamThreads, stream_min_ctas(R)) blur_strea
 
     const float* __restrict__ t = taps.v;
 
-    // roles rotate with the CTA's residency slot so that every SM sub-partition hosts both kinds of warp
-    const int role = ((tid >> 5) + (blockIdx.x / rot_div)) & 3;
+    // fixed roles: warps 0-1 produce, 2-3 consume in every CTA (each SM sub-partition's instruction cache sees one role)
+    const int role = (tid >> 5) & 3;
     if (role < 2) {
         // ---------------- producer: row pass ----------------
         StreamWalk wi;                                    // TMA cursor (meaningful in role 0 only)
@@ -714,13 +702,6 @@ __global__ void __launch_bounds__(kStreamThreads, stream_min_ctas(R)) blur_strea
             if (lane == 0) mbar_arrive(ring_empty + q);
             wk.next(tab, live_pieces, cg, tiles_x);
         }
-        if (trace != nullptr && role == 3 && lane == 0) {     // tuning aid: CTA residency interval and SM
-            unsigned long long t_end;
-            unsigned smid;
-            asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t_end));
-            asm volatile("mov.u32 %0, %%smid;" : "=r"(smid));
-            trace[3 * blockIdx.x] = t_begin; trace[3 * blockIdx.x + 1] = t_end; trace[3 * blockIdx.x + 2] = smid;
-        }
     }
 }
 
@@ -814,12 +795,11 @@ int sm_count() { return nm_sm_count(); }
 
 // The strip-walking kernel is taken for TMA-describable sources with enough chunks: below ~8 chunks per CTA the
 // lead-in row pass of a piece that starts inside a strip costs more than the tile kernels' halo rows.
-// NM_BLUR_STRIP_MIN overrides the threshold (tests force 1); NM_BLUR_WALK / NM_BLUR_TILE disable it (tuning aids).
+// NM_BLUR_STRIP_MIN overrides the threshold (test hook: the tests force 1).
 bool strip_eligible(const NmBlurArgs& a, const NmBlurTma* tma)
 {
-    static const bool no_strip = getenv("NM_BLUR_TILE") != nullptr || getenv("NM_BLUR_WALK") != nullptr;
     const int n_sms = sm_count();
-    if (no_strip || !tma || !tma->valid || !tma->valid_strip || n_sms <= 0 || a.radius < 1 || a.radius > 16) return false;
+    if (!tma || !tma->valid || !tma->valid_strip || n_sms <= 0 || a.radius < 1 || a.radius > 16) return false;
     static const long long strip_min_env = getenv("NM_BLUR_STRIP_MIN") ? atoll(getenv("NM_BLUR_STRIP_MIN")) : -1;
     const long long strip_min = strip_min_env >= 0 ? strip_min_env : 16LL * n_sms;
     const long long strips = (long long)nm_div_up(a.w, kTW) * a.batch;
@@ -828,13 +808,8 @@ bool strip_eligible(const NmBlurArgs& a, const NmBlurTma* tma)
 }
 
 // The streaming kernel takes what the strip kernel takes when the destination allows 8-byte stores, the source is
-// float (BGRA conversion stays with the strip kernel) and the CTA's piece table fits.  NM_BLUR_STREAM=0 disables it.
-int stream_ctas_per_sm(int R)
-{
-    static const int cap = getenv("NM_BLUR_STREAM_CTAS") ? atoi(getenv("NM_BLUR_STREAM_CTAS")) : 8;   // tuning aid
-    const int n = stream_min_ctas(R);
-    return cap < 1 ? 1 : n > cap ? cap : n;
-}
+// float (BGRA conversion stays with the strip kernel) and the CTA's piece table fits.  NM_BLUR_STREAM=0 disables it
+// (test hook: the tests use it to reach the strip kernel).
 bool stream_eligible(const NmBlurArgs& a, const NmBlurTma* tma)
 {
     static const bool off = getenv("NM_BLUR_STREAM") != nullptr && atoi(getenv("NM_BLUR_STREAM")) == 0;
@@ -842,39 +817,9 @@ bool stream_eligible(const NmBlurArgs& a, const NmBlurTma* tma)
     if (a.radius > kStreamMaxR || (a.w & 1)) return false;
     if ((a.dst_pitch & 1) || (a.dst_fstride & 1) || (reinterpret_cast<uintptr_t>(a.dst) & 7)) return false;
     if (a.dst2 != nullptr && (a.dst2_pitch & 1)) return false;
-    const long long strips = (long long)nm_div_up(a.w, kTW) * a.batch, G = (long long)stream_ctas_per_sm(a.radius) * sm_count();
+    const long long strips = (long long)nm_div_up(a.w, kTW) * a.batch, G = (long long)stream_min_ctas(a.radius) * sm_count();
     const long long total = strips * nm_div_up(a.h + 2 * a.radius, kGR);
     return total < (1LL << 31) && strips / G + 1 <= kStreamPieces;
-}
-
-// NM_BLUR_STREAM_TRACE: per-CTA residency intervals of one launch (synchronises; tuning aid only)
-void stream_trace_report(unsigned long long* trace, int G, int R, const NmBlurArgs& a, cudaStream_t stream)
-{
-    cudaStreamSynchronize(stream);
-    std::vector<unsigned long long> h(3 * (size_t)G);
-    cudaMemcpy(h.data(), trace, h.size() * sizeof(unsigned long long), cudaMemcpyDeviceToHost);
-    cudaFree(trace);
-    unsigned long long t0 = ~0ULL, t1 = 0;
-    for (int i = 0; i < G; ++i) if (h[3 * i + 1]) { t0 = std::min(t0, h[3 * i]); t1 = std::max(t1, h[3 * i + 1]); }
-    std::vector<double> dur, endrel;
-    std::vector<double> sm_first(256, 1e30), sm_last(256, 0);
-    for (int i = 0; i < G; ++i) {
-        if (!h[3 * i + 1]) continue;
-        dur.push_back((h[3 * i + 1] - h[3 * i]) * 1e-3);
-        const double e = (h[3 * i + 1] - t0) * 1e-3;
-        endrel.push_back(e);
-        const int sm = (int)h[3 * i + 2] & 255;
-        sm_first[sm] = std::min(sm_first[sm], e); sm_last[sm] = std::max(sm_last[sm], e);
-    }
-    std::sort(dur.begin(), dur.end()); std::sort(endrel.begin(), endrel.end());
-    double gap = 0; int ns = 0;
-    for (int s = 0; s < 256; ++s) if (sm_last[s] > 0) { gap += sm_last[s] - sm_first[s]; ++ns; }
-    const size_t n = dur.size();
-    if (n)
-        fprintf(stderr, "[stream R=%d %dx%dx%d] span %.1f us; CTA duration min %.1f med %.1f max %.1f; CTA end (from launch) "
-                        "10%% %.1f 50%% %.1f 90%% %.1f; per-SM first-to-last CTA end: mean %.1f us over %d SMs\n",
-                R, a.w, a.h, a.batch, (t1 - t0) * 1e-3, dur[0], dur[n / 2], dur[n - 1], endrel[n / 10], endrel[n / 2],
-                endrel[n * 9 / 10], ns ? gap / ns : 0.0, ns);
 }
 
 template <int R>
@@ -895,7 +840,6 @@ int launch_tile(const NmBlurArgs& a, cudaStream_t stream, const NmBlurTma* tma)
         const int n_sms = nm_sm_count();
         if (n_sms <= 0) return NM_ERR_NO_DEVICE;
         const long long n_tiles = (long long)grid.x * grid.y * grid.z;
-        static const bool no_walk = getenv("NM_BLUR_TILE") != nullptr;        // tuning aid
         const int chunks = nm_div_up(a.h + 2 * R, kCH);
         const long long total = (long long)grid.x * a.batch * chunks;
         if constexpr (R <= kStreamMaxR) if (stream_eligible(a, tma)) {
@@ -908,51 +852,40 @@ int launch_tile(const NmBlurArgs& a, cudaStream_t stream, const NmBlurTma* tma)
                 once_stream.done();
             }
             const long long n_strips = (long long)grid.x * a.batch;
-            // Co-resident CTAs do not advance evenly (the same work takes 45 to 105 us, NM_BLUR_STREAM_TRACE), so a launch
+            // Co-resident CTAs do not advance evenly (the same work takes 45 to 105 us), so a launch
             // of exactly-resident persistent CTAs ends with a long tail of half-empty SMs.  When there are enough strips
             // the launch is OVERSUBSCRIBED instead: P CTAs per strip (part b / strips of strip b % strips, so CTAs that
             // start together are neighbours in the image), about 2.5x the resident count, and the hardware hands an SM
-            // its next CTA as soon as one retires.  64 x 1080p: P = 2, pyramid 2.06 -> 1.96 ms (P = 1: 2.11, 3: 2.00).
-            // NM_BLUR_STREAM_PARTS forces P (0: always the persistent split).
-            static const int parts_env = getenv("NM_BLUR_STREAM_PARTS") ? atoi(getenv("NM_BLUR_STREAM_PARTS")) : -1;
+            // its next CTA as soon as one retires.  64 x 1080p (B200): P = 2, pyramid 2.06 -> 1.96 ms (P = 1: 2.11, 3: 2.00).
             const int cg = nm_div_up(a.h + 2 * R, kGR);
-            const long long resident = (long long)stream_ctas_per_sm(R) * n_sms;
-            int parts = parts_env;
-            if (parts_env < 0) {
-                // smallest P that reaches 2.5x the resident count with parts of >= 16 groups (the lead-in of a part is
-                // ceil(2R / 16) groups), else the largest such P that still reaches 1.5x, else the persistent split
-                parts = 0;
-                for (int p = 1; p <= 8 && cg >= 16 * p; ++p) {
-                    if (2 * n_strips * p >= 3 * resident) parts = p;
-                    if (2 * n_strips * p >= 5 * resident) break;
-                }
+            const long long resident = (long long)stream_min_ctas(R) * n_sms;
+            // smallest P that reaches 2.5x the resident count with parts of >= 16 groups (the lead-in of a part is
+            // ceil(2R / 16) groups), else the largest such P that still reaches 1.5x, else the persistent split
+            int parts = 0;
+            for (int p = 1; p <= 8 && cg >= 16 * p; ++p) {
+                if (2 * n_strips * p >= 3 * resident) parts = p;
+                if (2 * n_strips * p >= 5 * resident) break;
             }
             const bool over = parts > 0 && n_strips * parts > resident && n_strips * parts < (1 << 20) && cg >= 4 * parts;
             const int G = over ? (int)(n_strips * parts) : (int)resident;
             const int rounds_arg = over ? -parts : (int)(n_strips / G);
-            static const int rot_env = getenv("NM_BLUR_STREAM_ROT") ? atoi(getenv("NM_BLUR_STREAM_ROT")) : 0;   // tuning aid
-            const int rot_div = rot_env > 0 ? rot_env : (1 << 30);
             StreamTaps tp;
             memset(&tp, 0, sizeof(tp));
             memcpy(tp.v, a.taps_host, sizeof(float) * (2 * R + 1));
-            static const bool trace_on = getenv("NM_BLUR_STREAM_TRACE") != nullptr;                            // tuning aid
-            unsigned long long* trace = nullptr;
-            if (trace_on) cudaMalloc(&trace, sizeof(unsigned long long) * 3 * G);
             if (a.dst2 != nullptr)
                 blur_stream_kernel<R, true><<<G, kStreamThreads, stream_smem_bytes(R), stream>>>(
-                        a, tma->map_stream, tp, (int)grid.x, cg, rounds_arg, (int)(n_strips * cg), rot_div, trace);
+                        a, tma->map_stream, tp, (int)grid.x, cg, rounds_arg, (int)(n_strips * cg));
             else
                 blur_stream_kernel<R, false><<<G, kStreamThreads, stream_smem_bytes(R), stream>>>(
-                    a, tma->map_stream, tp, (int)grid.x, cg, rounds_arg, (int)(n_strips * cg), rot_div, trace);
+                    a, tma->map_stream, tp, (int)grid.x, cg, rounds_arg, (int)(n_strips * cg));
             NM_LAUNCH_CHECK();
-            if (trace_on) stream_trace_report(trace, G, R, a, stream);
             return NM_OK;
         }
         if (strip_eligible(a, tma)) {
             const long long n_strips = (long long)grid.x * a.batch;
             blur_strip_kernel<R><<<2 * n_sms, kThreads, strip_smem_bytes(R), stream>>>(a, tma->map_strip, (int)grid.x, chunks,
                                                                                       (int)(n_strips / (2 * n_sms)), total);
-        } else if (!no_walk && n_tiles >= 4LL * n_sms && n_tiles < (1LL << 31))
+        } else if (n_tiles >= 4LL * n_sms && n_tiles < (1LL << 31))
             blur_walk_kernel<R><<<2 * n_sms, kThreads, smem, stream>>>(a, tma->map, (int)grid.x, (int)grid.y, (int)n_tiles);
         else
             blur_tile_kernel<R, true><<<grid, kThreads, smem, stream>>>(a, tma->map);

@@ -10,8 +10,6 @@
 #include <atomic>
 #include <cmath>
 #include <cstring>
-#include <cstdlib>
-#include <cstdio>
 #include <new>
 #include <vector>
 
@@ -457,12 +455,11 @@ extern "C" int nm_sift_run_bgra(nm_sift_ctx* c, const void* frames_bgra_dev, int
 extern "C" int nm_sift_run(nm_sift_ctx* c, const float* frames_dev, int n_frames, nm_stream_t stream)
 {
     if (!c || !frames_dev || n_frames <= 0 || n_frames > c->B) return NM_ERR_INVALID;
-    // octaves 1.. beside octave 0's last levels when octave 0 alone fills the device for a while (NM_SIDE_OCTAVES=0 disables)
-    static const bool side_off = getenv("NM_SIDE_OCTAVES") && getenv("NM_SIDE_OCTAVES")[0] == '0';
+    // octaves 1.. beside octave 0's last levels when octave 0 alone fills the device for a while
     cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
     const bool cap_ok = cudaStreamIsCapturing((cudaStream_t)stream, &cap) == cudaSuccess;
     if (!cap_ok) cudaGetLastError();
-    const bool side = !side_off && cap_ok && cap == cudaStreamCaptureStatusNone &&
+    const bool side = cap_ok && cap == cudaStreamCaptureStatusNone &&
                       (long long)n_frames * c->P.width * c->P.height >= 16LL * 1920 * 1080;
     // (measured and not kept: the two halves of the batch as two ranges on two streams, 7.24 -> 7.16 ms per 64 frames)
     return sift_run_range(c, frames_dev, 0, n_frames, (cudaStream_t)stream, c->timing != 0, false, side);
@@ -484,28 +481,22 @@ extern "C" int nm_sift_run_host(nm_sift_ctx* c, const float* frames_host, int n_
     // fraction of a wave) are covered by running up to four stages concurrently on separate streams, and their
     // launch cost by replaying each stage as one CUDA graph.  Measured at 64 x 1080p, 4 streams, graphs:
     // stages of 3 frames 11.45 ms, 4: 11.67, 5: 11.60, 6: 11.73, 8: 12.16 (uploads alone: 9.58 ms);
-    // without graphs 6-frame stages were best at 12.33.
-    // NM_HOST_CHUNK=<n> / NM_HOST_STREAMS=<1..4> / NM_HOST_GRAPH=0 override (tuning aids).
-    static const int forced = [] {
-        const char* e = getenv("NM_HOST_CHUNK");
-        return e ? atoi(e) : 0;
-    }();
-    const int stage = forced > 0 ? forced : 3;
+    // without graphs 6-frame stages were best at 12.33 (B200).
+    constexpr int stage = 3;
     int bounds[NM_MAX_CHUNKS + 1];
     int n_chunks = 0;
     bounds[0] = 0;
-    if (n_frames <= 8 && forced <= 0) {
+    if (n_frames <= 8) {
         bounds[++n_chunks] = n_frames;
     } else {
         // uniform stages, tapered at the end (2, 1, 1 frames): what remains to be done when the LAST frame has landed
-        // is that frame's kernels and its result copy, not a whole 3-frame stage (NM_HOST_TAPER=0 disables)
-        static const bool taper = !(getenv("NM_HOST_TAPER") && getenv("NM_HOST_TAPER")[0] == '0');
+        // is that frame's kernels and its result copy, not a whole 3-frame stage
         const int per = std::max(stage, nm_div_up(n_frames, NM_MAX_CHUNKS - 4));
         int f = 0;
         while (f < n_frames) {
             const int left = n_frames - f;
             int take = per;
-            if (taper && per >= 2 && left <= per + 1) take = left >= 4 ? 2 : left >= 3 ? 2 : 1;
+            if (left <= per + 1) take = left >= 3 ? 2 : 1;
             if (take > left) take = left;
             f += take;
             bounds[++n_chunks] = f;
@@ -513,14 +504,6 @@ extern "C" int nm_sift_run_host(nm_sift_ctx* c, const float* frames_host, int n_
     }
     if (n_chunks > NM_MAX_CHUNKS) return NM_ERR_INVALID;
     int launches = 0;
-    // NM_HOST_TRACE=1: device timeline of the stages on stderr (development aid)
-    static const bool trace = getenv("NM_HOST_TRACE") != nullptr;
-    cudaEvent_t tr0 = nullptr, tr_in[NM_MAX_CHUNKS], tr_k0[NM_MAX_CHUNKS], tr_k1[NM_MAX_CHUNKS], tr_out[NM_MAX_CHUNKS];
-    if (trace) {
-        cudaEventCreate(&tr0);
-        for (int k = 0; k < n_chunks; ++k) { cudaEventCreate(&tr_in[k]); cudaEventCreate(&tr_k0[k]); cudaEventCreate(&tr_k1[k]); cudaEventCreate(&tr_out[k]); }
-        cudaEventRecord(tr0, c->s_in);
-    }
     auto drain = [&](int k) -> int {
         // results of chunk k: wait for its counts, then copy the filled part of every frame
         NM_CUDA_TRY(cudaEventSynchronize(c->ev_done[k]));
@@ -531,7 +514,6 @@ extern "C" int nm_sift_run_host(nm_sift_ctx* c, const float* frames_host, int n_
             if (x_host) NM_CUDA_TRY(cudaMemcpyAsync(x_host + off, c->x + off, n * sizeof(float), cudaMemcpyDeviceToHost, c->s_out));
             if (y_host) NM_CUDA_TRY(cudaMemcpyAsync(y_host + off, c->y + off, n * sizeof(float), cudaMemcpyDeviceToHost, c->s_out));
         }
-        if (trace) cudaEventRecord(tr_out[k], c->s_out);
         return NM_OK;
     };
     for (int k = 0; k < n_chunks; ++k) {        // the uploads do not depend on anything: queue them all
@@ -539,22 +521,14 @@ extern "C" int nm_sift_run_host(nm_sift_ctx* c, const float* frames_host, int n_
         NM_CUDA_TRY(cudaMemcpyAsync(c->frames_stage + f0 * fpix, frames_host + f0 * fpix, fpix * n * sizeof(float),
                                     cudaMemcpyHostToDevice, c->s_in));
         NM_CUDA_TRY(cudaEventRecord(c->ev_in[k], c->s_in));
-        if (trace) cudaEventRecord(tr_in[k], c->s_in);
     }
     // stages rotate over the internal compute streams: the launch-bound tail of one stage (small octaves,
-    // orientation) overlaps the big blur kernels of the next
-    static const int n_streams = [] {
-        const char* e = getenv("NM_HOST_STREAMS");
-        const int v = e ? atoi(e) : 4;
-        return v < 1 ? 1 : v > NM_AUX_STREAMS ? NM_AUX_STREAMS : v;
-    }();
-    // NM_HOST_GRAPH=0: launch the stages kernel by kernel (tuning aid); with several stages the launches of a stage
-    // are replayed as one CUDA graph (11 stages x 47 launches per 64-frame call otherwise)
-    static const bool graphs_on = [] {
-        const char* e = getenv("NM_HOST_GRAPH");
-        return !(e && e[0] == '0');
-    }();
-    const bool use_graphs = graphs_on && n_chunks > 1 && !trace;
+    // orientation) overlaps the big blur kernels of the next; the host may only block on a stage once the next
+    // n_streams - 1 stages are queued behind it
+    constexpr int n_streams = NM_AUX_STREAMS, lag = n_streams > 1 ? n_streams - 1 : 1;
+    // with several stages the launches of a stage are replayed as one CUDA graph (11 stages x 47 launches per
+    // 64-frame call otherwise)
+    const bool use_graphs = n_chunks > 1;
     NM_CUDA_TRY(cudaEventRecord(c->ev_fork, st));
     // every stage runs on an internal stream (the caller's may be the legacy default stream, which cannot be captured)
     for (int i = 0; i < n_streams; ++i) NM_CUDA_TRY(cudaStreamWaitEvent(c->s_aux[i], c->ev_fork, 0));
@@ -562,7 +536,6 @@ extern "C" int nm_sift_run_host(nm_sift_ctx* c, const float* frames_host, int n_
         const int f0 = bounds[k], n = bounds[k + 1] - bounds[k];
         cudaStream_t sk = c->s_aux[k % n_streams];
         NM_CUDA_TRY(cudaStreamWaitEvent(sk, c->ev_in[k], 0));
-        if (trace) cudaEventRecord(tr_k0[k], sk);
         int rc;
         if (use_graphs) {
             nm_sift_ctx::StageGraph& g = c->stage_graph[k];
@@ -590,12 +563,9 @@ extern "C" int nm_sift_run_host(nm_sift_ctx* c, const float* frames_host, int n_
         }
         NM_CUDA_TRY(cudaMemcpyAsync(counts_host + f0, c->counts + f0, sizeof(int) * n, cudaMemcpyDeviceToHost, sk));
         NM_CUDA_TRY(cudaEventRecord(c->ev_done[k], sk));
-        if (trace) cudaEventRecord(tr_k1[k], sk);
-        // the host may only block on a stage once the next n_streams - 1 stages are queued behind it
-        const int lag = n_streams > 1 ? n_streams - 1 : 1;
         if (k >= lag && (rc = drain(k - lag)) != NM_OK) return rc;
     }
-    for (int k = n_chunks - (n_streams > 1 ? n_streams - 1 : 1); k < n_chunks; ++k) {
+    for (int k = n_chunks - lag; k < n_chunks; ++k) {
         if (k < 0) continue;
         int rc = drain(k);
         if (rc != NM_OK) return rc;
@@ -608,17 +578,6 @@ extern "C" int nm_sift_run_host(nm_sift_ctx* c, const float* frames_host, int n_
     NM_CUDA_TRY(cudaEventRecord(c->ev_out, c->s_out));
     NM_CUDA_TRY(cudaStreamWaitEvent(st, c->ev_out, 0));
     NM_CUDA_TRY(cudaStreamSynchronize(st));
-    if (trace) {
-        for (int k = 0; k < n_chunks; ++k) {
-            float a = 0, b = 0, d = 0, e = 0;
-            cudaEventElapsedTime(&a, tr0, tr_in[k]); cudaEventElapsedTime(&b, tr0, tr_k0[k]);
-            cudaEventElapsedTime(&d, tr0, tr_k1[k]); cudaEventElapsedTime(&e, tr0, tr_out[k]);
-            fprintf(stderr, "[nm trace] stage %d frames %d..%d: uploaded %.2f  kernels %.2f..%.2f  downloaded %.2f ms\n",
-                    k, bounds[k], bounds[k + 1], a, b, d, e);
-            cudaEventDestroy(tr_in[k]); cudaEventDestroy(tr_k0[k]); cudaEventDestroy(tr_k1[k]); cudaEventDestroy(tr_out[k]);
-        }
-        cudaEventDestroy(tr0);
-    }
     c->last_launches = launches;
     return NM_OK;
 }
