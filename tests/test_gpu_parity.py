@@ -51,20 +51,25 @@ def run_product(nm, frames, peak=0.0, capacity=8192, exact=False, num_octaves=-1
     sb.set_dense_gradients(dense_grad)
     sb.run(_cu(frames))
     torch.cuda.synchronize()
-    r = sb.results()
-    out = []
-    for f in range(n):
-        c = int(r["counts"][f].item())
-        seg = r["seg_counts"][f].cpu().numpy()
-        nk = min(int(seg.sum()), capacity)
-        out.append({
-            "n": c, "seg_counts": seg, "desc": r["desc"][f, :c].cpu().numpy(), "x": r["x"][f, :c].cpu().numpy(),
-            "y": r["y"][f, :c].cpu().numpy(), "kpts": r["kpts"][f, :nk].cpu().numpy(),
-            "orient": r["orient"][f, :nk].cpu().numpy(),
-            "levels": [[sb.level(f, o, l).cpu().numpy() for l in range(6)] for o in range(P._num_octaves)],
-            "grad": [np.stack([sb.grad(f, o, l).cpu().numpy() for l in range(3)]) for o in range(P._num_octaves)],
-        })
+    out = [read_frame(sb, f, grad=True) for f in range(n)]
     sb.close()
+    return out
+
+
+def read_frame(sb, f, grad=False):
+    """Frame f of the last run of `sb` as host arrays: results, all Gaussian levels and (grad=True) gradient maps."""
+    r = sb.results()
+    c = int(r["counts"][f].item())
+    seg = r["seg_counts"][f].cpu().numpy()
+    nk = min(int(seg.sum()), sb.capacity)
+    out = {
+        "n": c, "seg_counts": seg, "desc": r["desc"][f, :c].cpu().numpy(), "x": r["x"][f, :c].cpu().numpy(),
+        "y": r["y"][f, :c].cpu().numpy(), "kpts": r["kpts"][f, :nk].cpu().numpy(),
+        "orient": r["orient"][f, :nk].cpu().numpy(),
+        "levels": [[sb.level(f, o, l).cpu().numpy() for l in range(6)] for o in range(sb.n_oct)],
+    }
+    if grad:
+        out["grad"] = [np.stack([sb.grad(f, o, l).cpu().numpy() for l in range(3)]) for o in range(sb.n_oct)]
     return out
 
 
@@ -111,9 +116,16 @@ def test_blur_vs_reference_golden(nm):
     assert np.array_equal(out.cpu().numpy(), g["result"])
 
 
-@pytest.mark.parametrize("shape", [(77, 131), (64, 128), (1, 5), (200, 33), (130, 260), (700, 300)])
-@pytest.mark.parametrize("radius", [1, 4, 5, 7, 8, 10, 13, 16, 20])
+@pytest.mark.parametrize("shape", [(77, 131), (64, 128), (1, 5), (200, 33), (130, 260), (700, 300), (2304, 2560)])
+@pytest.mark.parametrize("radius", list(range(1, 17)) + [17, 20, 45])
 def test_blur_vs_oracle_bitwise(nm, oracle, shape, radius):
+    """nm_blur_f32 at every radius the tiled kernels are instantiated for (1..16) and the generic two-pass blur above
+    them, up to the reference's largest kernel (radius 45).  Odd widths take the tile kernel with plain loads, the
+    other small shapes the TMA tile kernel, 2304 x 2560 (720 tiles, 740 strip chunks) the persistent tile-walking
+    kernel; test_forced_strip_blur_parity_suite re-runs every case through the strip-walking kernel.  Bitwise against
+    the oracle, and within the fp32 rounding bound of a float64 convolution: the taps are random and asymmetric, so
+    that check pins the direction (out[x] = sum_k in[x + k] * taps[R - k]) and the zero border independently."""
+    from scipy.ndimage import convolve1d
     from niftymatch_b200 import sift as S
     h, w = shape
     rng = np.random.default_rng(radius * 1000 + h)
@@ -124,8 +136,12 @@ def test_blur_vs_oracle_bitwise(nm, oracle, shape, radius):
     oracle.lib.orc_convolve(res.ctypes.data_as(C.c_void_p), img.ctypes.data_as(C.c_void_p), buf.ctypes.data_as(C.c_void_p),
                             w, h, taps.ctypes.data_as(C.c_void_p), radius)
     scratch = torch.empty((h, w), dtype=torch.float32, device="cuda")
-    out = S.blur(_cu(img), _cu(taps), radius, buffer=scratch)
-    assert np.array_equal(out.cpu().numpy(), res)
+    out = S.blur(_cu(img), _cu(taps), radius, buffer=scratch).cpu().numpy()
+    assert np.array_equal(out, res)
+    t64 = taps.astype(np.float64)
+    ref = convolve1d(convolve1d(img.astype(np.float64), t64, axis=1, mode="constant"), t64, axis=0, mode="constant")
+    # two chains of 2R+1 fp32 multiply-adds over non-negative terms summing to <= max|img|
+    assert np.abs(out - ref).max() <= 4 * (2 * radius + 1) * 2.0 ** -24 * np.abs(img).max()
 
 
 def test_downsample_subtract_gradient_vs_oracle(nm, oracle):
@@ -352,10 +368,10 @@ def test_1080p_single_frame_vs_oracle(nm, oracle):
 
 
 def test_1080p_batch_strip_blur_vs_oracle(nm, oracle):
-    """Twenty 1080p frames = 300 column strips in octave 0: the strip-walking blur kernel (nm_pyramid.cu,
-    blur_strip_kernel) runs one round of whole strips on its 296 CTAs and splits the 4 strips left over as a flat
-    chunk list (most pieces empty, some starting inside a strip).  First, a middle and the last frame against the
-    CPU oracle, levels bitwise."""
+    """Twenty 1080p frames = 300 column strips in octave 0: every octave-0 blur takes the streaming blur kernel
+    (nm_pyramid.cu, blur_stream_kernel) oversubscribed with 4 CTAs per strip, each walking a quarter of the strip's
+    16-row groups (the parts that start inside the strip after lead-in groups whose outputs are not stored).  First,
+    a middle and the last frame against the CPU oracle, levels bitwise."""
     frames = np.stack([synth.scene(1920, 1080, synth.SEED_BASE + (i % 2)) for i in range(20)])
     out = run_product(nm, frames, capacity=16384)
     ref = [oracle.sift_frame(frames[f], capacity=16384) for f in (0, 1)]
