@@ -247,6 +247,52 @@ int nm_transform_blend_bgra(void* canvas, int cw, int ch, unsigned long long fra
                             unsigned long long frame_wts_tex, nm_stream_t stream);
 
 /* ------------------------------------------------------------------------ */
+/* Mosaic of a frame stream: the pairwise homographies of a registered        */
+/* stream chained and laid out on a canvas, and a chunk of frames blended in  */
+/* one pass over the canvas.  No host synchronisation inside.                 */
+/* ------------------------------------------------------------------------ */
+typedef struct nm_mosaic_ctx nm_mosaic_ctx;
+
+/* frame_w x frame_h BGRA frames, up to max_frames (<= 1024) per blend call.  mask: frame_w*frame_h bytes, weights:
+ * frame_w*frame_h floats, host or device memory; bound as textures with the reference's CudaTex2D settings
+ * (cudaArray, linear filter, border addressing, unnormalised coordinates; frame and mask read as normalised floats,
+ * weights as elements), like the textures a reference client hands to transform_blend.  The context owns one such
+ * frame texture per slot.  Calls on one context are ordered by their stream: use one stream per context. */
+int nm_mosaic_create(nm_mosaic_ctx** m, int frame_w, int frame_h, int max_frames, const unsigned char* mask, const float* weights);
+int nm_mosaic_destroy(nm_mosaic_ctx* m);
+
+/* Placement, one CTA, fp64.  All pointers are device memory.
+ *   H_pairs   [n_frames-1][9] row-major: H[p] maps frame p coordinates to frame p+1 (nm_ransac_batch_f32)
+ *   status    [n_frames-1][3] as nm_ransac_batch_f32 writes it, or NULL (every pair valid)
+ *   anchor9   G[0] (frame 0 -> mosaic), NULL = identity;  G[p+1] = G[p] . H[p]^-1, where H[p] is replaced by the identity
+ *             when status[p*3] == 0 or H[p] is singular or non-finite (flag bit 0 of frame p+1).  After each step G is
+ *             divided by the power of two at its largest absolute entry (exact; the blend is scale invariant).
+ *   footprint of frame k: the bounding box, floor / ceil, of the sampling box [-1, fw] x [-1, fh] mapped through G[k]
+ *             (a bilinear sample with non-zero mask weight comes from inside it); empty, flag bit 1, when a corner has
+ *             w <= 0, is non-finite or lies beyond 2^30 pixels
+ *   origin2   canvas origin (ox, oy) in mosaic pixels, NULL = the least corner over all non-empty footprints
+ *   bounds_out  (ox, oy, width, height): the canvas from that origin that holds every footprint
+ *   rects_out [n_frames][4] (tx, ty, nw, nh) in canvas pixels ((0, 0, 0, 0) when empty), 16-byte aligned
+ *   mats_out  [n_frames][9] canvas-local -> frame coordinates, G[k]^-1 . T(tx + ox, ty + oy) rounded to float: the
+ *             mat3x3 of nm_transform_blend_bgra
+ *   flags_out [n_frames];  chain_out  [n_frames][9] doubles, G[k], or NULL */
+int nm_mosaic_place_f32(const float* H_pairs, const int* status, int n_frames, int frame_w, int frame_h, const float* anchor9,
+                        const int* origin2, float* mats_out, int* rects_out, int* flags_out, int* bounds_out, double* chain_out,
+                        nm_stream_t stream);
+
+/* frames_bgra: n_frames x frame_h x frame_w uchar4 on the device (the buffer nm_sift_run_bgra takes), frame size equal to
+ * the context's; mats / rects as nm_mosaic_place_f32 writes them (rects 16-byte aligned; a rect with nw or nh <= 0 is
+ * empty).  Copies frame i into slot i (one cudaMemcpy2DToArrayAsync each) and blends all n frames in one pass over
+ * the cw x ch canvas: bitwise equal to n calls of nm_transform_blend_bgra, in frame order, on the context's textures. */
+int nm_mosaic_blend_bgra(nm_mosaic_ctx* m, const void* frames_bgra, int n_frames, int frame_w, int frame_h, const float* mats,
+                         const int* rects, void* canvas, int cw, int ch, float* canvas_wts, nm_stream_t stream);
+
+/* The context's texture objects (frame slot i -> frame_tex_host[i], max_frames of them; mask; weights), for callers
+ * that drive nm_transform_blend_bgra themselves.  Any output may be NULL. */
+int nm_mosaic_textures(nm_mosaic_ctx* m, unsigned long long* frame_tex_host, unsigned long long* mask_tex,
+                       unsigned long long* wts_tex);
+
+/* ------------------------------------------------------------------------ */
 /* Registration after matching (SURVEY.md 8f rank 1): align_points and the    */
 /* three RANSAC estimators of gpu/kernels/ransac.h, Jacobi SVD of svd.cu.      */
 /* ------------------------------------------------------------------------ */

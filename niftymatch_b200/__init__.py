@@ -11,3 +11,4 @@ from .sift import SiftParams, SiftBatch, gaussian_taps, grayscale, cast_u8, undi
 from .match import match, match_top2, merge_top2, match_pairs, set_engine, get_engine, tc_probe  # noqa: F401
 from .ransac import align_points, ransac, ransac_batch, ransac_hypotheses, TRANSLATION, SIMILARITY, HOMOGRAPHY  # noqa: F401
 from .dist import shard_bounds, match_sharded, frame_range, register_stream  # noqa: F401
+from .mosaic import Mosaic, Placement, place, render_stream  # noqa: F401

@@ -72,6 +72,11 @@ SIGNATURES = {
     "nm_resample_perspective_bgra": (_i, [_vp, _ull, _i, _i, _vp, _vp, _vp, _i, _vp]),
     "nm_resample_mask_tex_u8": (_i, [_vp, _ull, _i, _i, _vp, _vp, _f, _vp]),
     "nm_transform_blend_bgra": (_i, [_vp, _i, _i, _ull, _i, _i, _i, _i, _vp, _i, _i, _ull, _vp, _ull, _vp]),
+    "nm_mosaic_create": (_i, [C.POINTER(_vp), _i, _i, _i, _vp, _vp]),
+    "nm_mosaic_destroy": (_i, [_vp]),
+    "nm_mosaic_place_f32": (_i, [_vp, _vp, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "nm_mosaic_blend_bgra": (_i, [_vp, _vp, _i, _i, _i, _vp, _vp, _vp, _i, _i, _vp, _vp]),
+    "nm_mosaic_textures": (_i, [_vp, C.POINTER(_ull), C.POINTER(_ull), C.POINTER(_ull)]),
     "nm_sift_run_bgra": (_i, [_vp, _vp, _i, _vp]),
     "nm_align_points_f32": (_i, [_vp] * 9 + [_i, _vp]),
     "nm_align_pairs_f32": (_i, [_vp, _vp, _vp, _vp, _i, _i, _vp, _vp, _vp, _vp, _vp]),

@@ -138,8 +138,10 @@ class StreamRegistrar:
         self.corr = [torch.empty((n, cap), dtype=torch.float32, device=dev) for _ in range(4)]
 
     def run(self, frames_of, lo: int, hi: int):
-        """frames_of(t0, t1) -> cuda float32 (t1 - t0, h, w) = frames [t0, t1) of the stream.  Registers every pair
-        (t, t + 1) with lo <= t < hi - 1.  Returns (homographies (hi - lo - 1, 9), status (hi - lo - 1, 3)) on the device."""
+        """frames_of(t0, t1) -> frames [t0, t1) of the stream on the device: cuda float32 (t1 - t0, h, w), or BGRA video
+        frames, cuda uint8 (t1 - t0, h, w, 4), whose grey conversion is fused into the base blur (nm_sift_run_bgra) --
+        the same colour buffer then feeds the mosaic (mosaic.render_stream).  Registers every pair (t, t + 1) with
+        lo <= t < hi - 1.  Returns (homographies (hi - lo - 1, 9), status (hi - lo - 1, 3)) on the device."""
         import ctypes as C
         import torch
         from . import _lib
@@ -158,7 +160,11 @@ class StreamRegistrar:
         while c0 < hi - 1:
             c1 = min(hi, c0 + self.chunk)
             n = c1 - c0
-            sb.run(frames_of(c0, c1))
+            chunk = frames_of(c0, c1)
+            if chunk.dtype == torch.uint8 and chunk.dim() == 4 and chunk.shape[-1] == 4:
+                sb.run_bgra(chunk)
+            else:
+                sb.run(chunk)
             self.match[: n - 1].fill_(-1)
             check(lib.nm_match_pairs_f32(p(r["desc"]), p(r["counts"]), n, cap, self.ambiguity, p(self.match), None, None,
                                          _stream_ptr()), "nm_match_pairs_f32")
