@@ -345,6 +345,24 @@ int nm_ransac_batch_f32(int kind, const float* src_x, const float* src_y, const 
                         long long pair_stride, const int* counts, int max_pts, int n_pairs, float inlier_threshold,
                         int iterations, unsigned long long seed, float* homographies, int* status, nm_stream_t stream);
 
+/* Refit of RANSAC models on their inlier sets, and the inlier masks (no reference counterpart).  Arguments as
+ * nm_ransac_batch_f32 (the same correspondence buffers; H_in / status_in as it writes them, status_in NULL = every pair
+ * has a model).  Pair p: S0 = the inliers of H_in[p] under the RANSAC rule; round r = 1..rounds fits H_r to S(r-1) by
+ * least squares (fp64; translation: mean displacement; similarity: linear in Hartley-normalised coordinates;
+ * homography: normalised DLT, then Levenberg-Marquardt on the forward transfer error), rounded to float, and keeps it
+ * unless it is degenerate, not finite or has fewer inliers than S(r-1); it stops when the inlier set no longer changes.
+ * Sets of no more than 1 / 2 / 4 points are not refitted.  rounds = 0 computes the masks only (H_out = H_in).
+ *   H_out      [n_pairs][9], may alias H_in; not written for a pair with status_in[p*3] == 0
+ *   status_out [n_pairs][3], may alias status_in: {status_in[p][0], inliers of the returned model, refits kept}; {0, 0, 0}
+ *              for a pair without a model.  The layout nm_mosaic_place_f32 reads.
+ *   inlier_mask [n_pairs][max_pts] bytes 0 / 1 for the returned model (0 at i >= counts[p]), or NULL.
+ * One CTA per pair, no workspace and no host synchronisation (the call can be captured in a CUDA graph); pair p's
+ * result is bit-reproducible and does not depend on the other pairs. */
+int nm_ransac_refine_batch_f32(int kind, const float* src_x, const float* src_y, const float* dst_x, const float* dst_y,
+                               long long pair_stride, const int* counts, int max_pts, int n_pairs, float inlier_threshold,
+                               const float* H_in, const int* status_in, int rounds,
+                               float* H_out, int* status_out, unsigned char* inlier_mask, nm_stream_t stream);
+
 /* ------------------------------------------------------------------------ */
 /* Batched SIFT detect+describe: the client loop of the reference             */
 /* (compute_dog/_gradients/_keypoints/_orientations/_descriptors,             */

@@ -454,6 +454,473 @@ __global__ void __launch_bounds__(256) select_kernel(const int* __restrict__ inl
     if (tid == 0) { status[0] = 1; status[1] = (int)(best[0] >> 32); status[2] = idx; }
 }
 
+// score_kernel's inlier rule, expression for expression: q = (src_x, src_y, dst_x, dst_y) is an inlier of H when
+// src_x >= 0 and the squared forward transfer error is < thr.  The mask of a RANSAC model therefore has exactly as many
+// bits set as the model's score (tests/test_gpu_ransac_refine.py).  score_kernel keeps its own copy of the loop body:
+// calling any helper there, this one included, changes how its loop is unrolled.
+__device__ __forceinline__ bool transfer_inlier(const float* H, const float4 q, float thr)
+{
+    if (!(q.x >= 0.f)) return false;
+    float x = H[0] * q.x + H[1] * q.y + H[2];
+    float y = H[3] * q.x + H[4] * q.y + H[5];
+    const float z = H[6] * q.x + H[7] * q.y + H[8];
+    x /= z;
+    y /= z;
+    const float d2 = (q.z - x) * (q.z - x) + (q.w - y) * (q.w - y);
+    return d2 < thr;
+}
+
+// ---- refit of a model on its inlier set (no reference counterpart) ------------------------------------------------
+// One CTA per pair.  An inlier set is never stored: every pass over it applies transfer_inlier with the set's fp32
+// model to the pair's correspondences (read from L2 after the first pass), so no workspace is needed and sets of any
+// size take the same path.  Sums are fp64: each thread adds its correspondences in index order, each warp folds its
+// lanes in a fixed butterfly, then the warps are added in order -- bit-reproducible, and pair p depends on nothing
+// but its own inputs.
+constexpr int kRefineThreads = 256, kRefineWarps = kRefineThreads / 32, kRefineSums = 29;
+constexpr int kLmIterations = 20, kJacobiSweeps = 30;
+
+struct RefineShared {
+    float H[2][9];                              // [0] model of the current inlier set, [1] the refit
+    double red[kRefineWarps][kRefineSums];      // per-warp partial sums
+    double tot[kRefineSums];                    // block sums
+    double A[81], V[81];                        // DLT normal matrix (eigenvalues on its diagonal after Jacobi), eigenvectors
+    double J[64], g[8], L[64];                  // LM normal equations J^T J, J^T r, Cholesky factor
+    double prm[2][8];                           // LM point and trial point (normalised homography, h8 = 1)
+    int ok;
+};
+
+template <int K>
+__device__ void block_sum(double (&v)[K], RefineShared& S)
+{
+    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+#pragma unroll
+    for (int k = 0; k < K; ++k) {
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) v[k] += __shfl_xor_sync(0xffffffffu, v[k], o);
+        if (lane == 0) S.red[wid][k] = v[k];
+    }
+    __syncthreads();
+    for (int k = threadIdx.x; k < K; k += kRefineThreads) {
+        double s = S.red[0][k];
+        for (int w = 1; w < kRefineWarps; ++w) s += S.red[w][k];
+        S.tot[k] = s;
+    }
+    __syncthreads();
+}
+
+// f(q) for every correspondence q of pair p that is an inlier of the fp32 model Hsh
+template <class F>
+__device__ __forceinline__ void for_each_inlier(const Pairs& P, int p, int n, const float* Hsh, float thr, F f)
+{
+    float H[9];
+#pragma unroll
+    for (int k = 0; k < 9; ++k) H[k] = Hsh[k];
+    const long long off = (long long)p * P.stride;
+    for (int i = threadIdx.x; i < n; i += kRefineThreads) {
+        const float4 q = make_float4(P.sx[off + i], P.sy[off + i], P.dx[off + i], P.dy[off + i]);
+        if (transfer_inlier(H, q, thr)) f(q);
+    }
+}
+
+// Hartley normalisation of both point sets: src (x - mx) * s, dst likewise, RMS distance from the centroid sqrt(2)
+struct Norm {
+    double smx, smy, s1, dmx, dmy, s2;
+    __device__ void apply(const float4 q, double& a, double& b, double& u, double& v) const
+    {
+        a = ((double)q.x - smx) * s1;
+        b = ((double)q.y - smy) * s1;
+        u = ((double)q.z - dmx) * s2;
+        v = ((double)q.w - dmy) * s2;
+    }
+};
+
+// Solves A x = b for a symmetric positive definite N x N matrix whose lower triangle is in L (overwritten by the
+// factor).  False when a pivot is not positive or the solution is not finite.
+template <int N>
+__device__ bool cholesky_solve(double* L, const double* b, double* x)
+{
+    for (int j = 0; j < N; ++j) {
+        double d = L[j * N + j];
+        for (int k = 0; k < j; ++k) d -= L[j * N + k] * L[j * N + k];
+        if (!(d > 0.0)) return false;
+        d = sqrt(d);
+        L[j * N + j] = d;
+        for (int i = j + 1; i < N; ++i) {
+            double s = L[i * N + j];
+            for (int k = 0; k < j; ++k) s -= L[i * N + k] * L[j * N + k];
+            L[i * N + j] = s / d;
+        }
+    }
+    for (int i = 0; i < N; ++i) {
+        double s = b[i];
+        for (int k = 0; k < i; ++k) s -= L[i * N + k] * x[k];
+        x[i] = s / L[i * N + i];
+    }
+    bool ok = true;
+    for (int i = N - 1; i >= 0; --i) {
+        double s = x[i];
+        for (int k = i + 1; k < N; ++k) s -= L[k * N + i] * x[k];
+        x[i] = s / L[i * N + i];
+        ok &= isfinite(x[i]);
+    }
+    return ok;
+}
+
+// Cyclic Jacobi on the symmetric 9 x 9 matrix A (eigenvalues on its diagonal afterwards), eigenvectors to the columns
+// of V.  Called by warp 0: every lane decides the same rotations, lane k < 9 rotates row and column k.
+__device__ void jacobi_eigen9(double* A, double* V)
+{
+    const int k = threadIdx.x;
+    for (int i = k; i < 81; i += 32) V[i] = i % 10 == 0 ? 1.0 : 0.0;
+    __syncwarp();
+    for (int sweep = 0; sweep < kJacobiSweeps; ++sweep) {
+        bool rotated = false;
+        for (int p = 0; p < 8; ++p)
+            for (int q = p + 1; q < 9; ++q) {
+                const double apq = A[p * 9 + q], app = A[p * 9 + p], aqq = A[q * 9 + q];
+                __syncwarp();
+                if (!(fabs(apq) > 1e-18 * sqrt(fabs(app * aqq)))) continue;
+                const double theta = (aqq - app) / (2.0 * apq), at = fabs(theta);
+                const double t = at > 1e100 ? 0.5 / theta : (theta >= 0.0 ? 1.0 : -1.0) / (at + sqrt(theta * theta + 1.0));
+                const double c = 1.0 / sqrt(t * t + 1.0), s = t * c;
+                if (k < 9) {
+                    const double akp = A[k * 9 + p], akq = A[k * 9 + q];
+                    A[k * 9 + p] = c * akp - s * akq;
+                    A[k * 9 + q] = s * akp + c * akq;
+                }
+                __syncwarp();
+                if (k < 9) {
+                    const double apk = A[p * 9 + k], aqk = A[q * 9 + k];
+                    A[p * 9 + k] = c * apk - s * aqk;
+                    A[q * 9 + k] = s * apk + c * aqk;
+                    const double vkp = V[k * 9 + p], vkq = V[k * 9 + q];
+                    V[k * 9 + p] = c * vkp - s * vkq;
+                    V[k * 9 + q] = s * vkp + c * vkq;
+                }
+                __syncwarp();
+                if (k == 0) A[p * 9 + q] = A[q * 9 + p] = 0.0;
+                __syncwarp();
+                rotated = true;
+            }
+        if (!rotated) break;
+    }
+}
+
+// out = fp32 of Td^-1 . Hn . Ts divided by its [8]; false when not finite
+__device__ bool denormalise_store(const double* Hn, const Norm& nm, float* out)
+{
+    double T[9], R[9];
+    for (int r = 0; r < 3; ++r) {
+        T[r * 3 + 0] = Hn[r * 3 + 0] * nm.s1;
+        T[r * 3 + 1] = Hn[r * 3 + 1] * nm.s1;
+        T[r * 3 + 2] = Hn[r * 3 + 2] - Hn[r * 3 + 0] * nm.s1 * nm.smx - Hn[r * 3 + 1] * nm.s1 * nm.smy;
+    }
+    for (int c = 0; c < 3; ++c) {
+        R[c] = T[c] / nm.s2 + nm.dmx * T[6 + c];
+        R[3 + c] = T[3 + c] / nm.s2 + nm.dmy * T[6 + c];
+        R[6 + c] = T[6 + c];
+    }
+    bool ok = true;
+    for (int e = 0; e < 9; ++e) {
+        out[e] = (float)(R[e] / R[8]);
+        ok &= isfinite(out[e]);
+    }
+    return ok;
+}
+
+// sum of squared forward transfer errors in normalised coordinates at the normalised homography h (h8 = 1)
+__device__ double lm_cost(const Pairs& P, int p, int n, float thr, const Norm& nm, const double* hs, RefineShared& S)
+{
+    double h[8];
+#pragma unroll
+    for (int e = 0; e < 8; ++e) h[e] = hs[e];
+    double v[1] = {0.0};
+    for_each_inlier(P, p, n, S.H[0], thr, [&](const float4 q) {
+        double a, b, u, w;
+        nm.apply(q, a, b, u, w);
+        const double iw = 1.0 / (h[6] * a + h[7] * b + 1.0);
+        const double rx = (h[0] * a + h[1] * b + h[2]) * iw - u, ry = (h[3] * a + h[4] * b + h[5]) * iw - w;
+        v[0] += rx * rx + ry * ry;
+    });
+    block_sum(v, S);
+    return S.tot[0];
+}
+
+// J^T J and J^T r of the transfer error at h: with g = (a, b, 1) / w, c = (a, b) / w and the mapped point (X, Y), the
+// Jacobian rows are [g, 0, -X c] and [0, g, -Y c], so 29 sums make up the 8 x 8 system (written by thread 0).
+__device__ void lm_normal(const Pairs& P, int p, int n, float thr, const Norm& nm, const double* hs, RefineShared& S)
+{
+    double h[8];
+#pragma unroll
+    for (int e = 0; e < 8; ++e) h[e] = hs[e];
+    double v[kRefineSums];
+#pragma unroll
+    for (int e = 0; e < kRefineSums; ++e) v[e] = 0.0;
+    for_each_inlier(P, p, n, S.H[0], thr, [&](const float4 q) {
+        double a, b, u, w;
+        nm.apply(q, a, b, u, w);
+        const double iw = 1.0 / (h[6] * a + h[7] * b + 1.0);
+        const double X = (h[0] * a + h[1] * b + h[2]) * iw, Y = (h[3] * a + h[4] * b + h[5]) * iw;
+        const double rx = X - u, ry = Y - w;
+        const double g[3] = {a * iw, b * iw, iw};
+        v[0] += g[0] * g[0]; v[1] += g[0] * g[1]; v[2] += g[0] * g[2];
+        v[3] += g[1] * g[1]; v[4] += g[1] * g[2]; v[5] += g[2] * g[2];
+#pragma unroll
+        for (int i = 0; i < 3; ++i) {
+            const double xg = X * g[i], yg = Y * g[i];
+            v[6 + 2 * i] += xg * g[0]; v[7 + 2 * i] += xg * g[1];
+            v[12 + 2 * i] += yg * g[0]; v[13 + 2 * i] += yg * g[1];
+            v[21 + i] += rx * g[i];
+            v[24 + i] += ry * g[i];
+        }
+        const double q2 = X * X + Y * Y, e = X * rx + Y * ry;
+        v[18] += q2 * g[0] * g[0]; v[19] += q2 * g[0] * g[1]; v[20] += q2 * g[1] * g[1];
+        v[27] -= e * g[0]; v[28] -= e * g[1];
+    });
+    block_sum(v, S);
+    if (threadIdx.x == 0) {
+        const double* t = S.tot;
+        const int s3[9] = {0, 1, 2, 1, 3, 4, 2, 4, 5};
+        for (int e = 0; e < 64; ++e) S.J[e] = 0.0;
+        for (int i = 0; i < 3; ++i) {
+            for (int j = 0; j < 3; ++j) S.J[i * 8 + j] = S.J[(3 + i) * 8 + 3 + j] = t[s3[i * 3 + j]];
+            for (int j = 0; j < 2; ++j) {
+                S.J[i * 8 + 6 + j] = S.J[(6 + j) * 8 + i] = -t[6 + 2 * i + j];
+                S.J[(3 + i) * 8 + 6 + j] = S.J[(6 + j) * 8 + 3 + i] = -t[12 + 2 * i + j];
+            }
+        }
+        S.J[6 * 8 + 6] = t[18];
+        S.J[6 * 8 + 7] = S.J[7 * 8 + 6] = t[19];
+        S.J[7 * 8 + 7] = t[20];
+        for (int e = 0; e < 8; ++e) S.g[e] = t[21 + e];
+    }
+}
+
+// Least-squares refit on the inlier set of S.H[0] (cnt correspondences) into S.H[1].  False when the fit is degenerate
+// or its fp32 result is not finite; S.H[1] is then not used.
+template <int KIND>
+__device__ bool refit(const Pairs& P, int p, int n, float thr, int cnt, RefineShared& S)
+{
+    const int tid = threadIdx.x;
+    const double N = (double)cnt;
+    if constexpr (KIND == 0) {                                   // the mean displacement
+        double v[2] = {0.0, 0.0};
+        for_each_inlier(P, p, n, S.H[0], thr, [&](const float4 q) {
+            v[0] += (double)q.z - (double)q.x;
+            v[1] += (double)q.w - (double)q.y;
+        });
+        block_sum(v, S);
+        if (tid == 0) {
+            const float H[9] = {1.f, 0.f, (float)(S.tot[0] / N), 0.f, 1.f, (float)(S.tot[1] / N), 0.f, 0.f, 1.f};
+            for (int e = 0; e < 9; ++e) S.H[1][e] = H[e];
+            S.ok = isfinite(H[2]) && isfinite(H[5]);
+        }
+        __syncthreads();
+        return S.ok;
+    } else {
+    Norm nm;
+    {
+        double v[4] = {0.0, 0.0, 0.0, 0.0};
+        for_each_inlier(P, p, n, S.H[0], thr, [&](const float4 q) { v[0] += q.x; v[1] += q.y; v[2] += q.z; v[3] += q.w; });
+        block_sum(v, S);
+        nm.smx = S.tot[0] / N; nm.smy = S.tot[1] / N; nm.dmx = S.tot[2] / N; nm.dmy = S.tot[3] / N;
+        nm.s1 = nm.s2 = 1.0;
+        double r[2] = {0.0, 0.0};
+        for_each_inlier(P, p, n, S.H[0], thr, [&](const float4 q) {
+            double a, b, u, w;
+            nm.apply(q, a, b, u, w);
+            r[0] += a * a + b * b;
+            r[1] += u * u + w * w;
+        });
+        block_sum(r, S);
+        nm.s1 = sqrt(2.0) / sqrt(S.tot[0] / N);
+        nm.s2 = sqrt(2.0) / sqrt(S.tot[1] / N);
+    }
+    if constexpr (KIND == 1) {
+        // u = a' x - b' y + tx, v = b' x + a' y + ty is linear in (a', b', tx, ty): 4 x 4 normal equations
+        double v[7];
+#pragma unroll
+        for (int e = 0; e < 7; ++e) v[e] = 0.0;
+        for_each_inlier(P, p, n, S.H[0], thr, [&](const float4 q) {
+            double x, y, u, w;
+            nm.apply(q, x, y, u, w);
+            v[0] += x * x + y * y; v[1] += x; v[2] += y;
+            v[3] += x * u + y * w; v[4] += x * w - y * u; v[5] += u; v[6] += w;
+        });
+        block_sum(v, S);
+        if (tid == 0) {
+            const double* t = S.tot;
+            const double A[16] = {t[0], 0.0, t[1], t[2], 0.0, t[0], -t[2], t[1], t[1], -t[2], N, 0.0, t[2], t[1], 0.0, N};
+            for (int e = 0; e < 16; ++e) S.L[e] = A[e];
+            double x[4];
+            bool ok = cholesky_solve<4>(S.L, t + 3, x);
+            const double Hn[9] = {x[0], -x[1], x[2], x[1], x[0], x[3], 0.0, 0.0, 1.0};
+            S.ok = ok && denormalise_store(Hn, nm, S.H[1]);
+        }
+        __syncthreads();
+        return S.ok;
+    } else {
+    // homography: normalised DLT, the two rows per point of homography4, M = sum r^T r from 24 sums of t t^T, t = (a, b, 1)
+    {
+        double v[24];
+#pragma unroll
+        for (int e = 0; e < 24; ++e) v[e] = 0.0;
+        for_each_inlier(P, p, n, S.H[0], thr, [&](const float4 q) {
+            double a, b, u, w;
+            nm.apply(q, a, b, u, w);
+            const double tt[6] = {a * a, a * b, a, b * b, b, 1.0};
+            const double q2 = u * u + w * w;
+#pragma unroll
+            for (int e = 0; e < 6; ++e) {
+                v[e] += tt[e];
+                v[6 + e] += u * tt[e];
+                v[12 + e] += w * tt[e];
+                v[18 + e] += q2 * tt[e];
+            }
+        });
+        block_sum(v, S);
+        if (tid < 81) {
+            const int i = tid / 9, j = tid % 9, bi = i / 3, bj = j / 3;
+            const int s3[9] = {0, 1, 2, 1, 3, 4, 2, 4, 5};
+            const double m = S.tot[s3[(i % 3) * 3 + j % 3]], mu = S.tot[6 + s3[(i % 3) * 3 + j % 3]];
+            const double mw = S.tot[12 + s3[(i % 3) * 3 + j % 3]], mq = S.tot[18 + s3[(i % 3) * 3 + j % 3]];
+            double x = 0.0;                                    // blocks of M: [S0 0 -Su; 0 S0 -Sw; -Su -Sw Sq]
+            if (bi == bj) x = bi == 2 ? mq : m;
+            else if (bi == 2 || bj == 2) x = (bi == 0 || bj == 0) ? -mu : -mw;
+            S.A[tid] = x;
+        }
+        __syncthreads();
+        if (tid < 32) {
+            jacobi_eigen9(S.A, S.V);
+            if (tid == 0) {
+                int lo = 0;
+                double hi = S.A[0];
+                for (int e = 1; e < 9; ++e) {
+                    if (S.A[e * 10] < S.A[lo * 10]) lo = e;
+                    hi = fmax(hi, S.A[e * 10]);
+                }
+                double second = INFINITY;
+                for (int e = 0; e < 9; ++e)
+                    if (e != lo) second = fmin(second, S.A[e * 10]);
+                const double h8 = S.V[8 * 9 + lo];
+                // a null space of more than one dimension (collinear points, ...) or a model at infinity
+                S.ok = second > 1e-12 * hi && fabs(h8) > 1e-12;
+                for (int e = 0; e < 8; ++e) S.prm[0][e] = S.V[e * 9 + lo] / h8;
+            }
+        }
+        __syncthreads();
+        if (!S.ok) return false;
+    }
+    // Levenberg-Marquardt on the transfer error: lambda0 = 1e-3 max diag(J^T J), (J^T J + lambda diag) d = -J^T r,
+    // accepted step -> lambda / 10, rejected -> lambda * 10; at most kLmIterations steps, stop when an accepted step
+    // gains less than 1e-12 of the cost or when lambda > 1e16.  Every thread keeps the same (cur, cost, lambda).
+    int cur = 0;
+    double cost = lm_cost(P, p, n, thr, nm, S.prm[0], S);
+    lm_normal(P, p, n, thr, nm, S.prm[0], S);
+    double lambda = 1e-3 * fmax(fmax(fmax(S.tot[0], S.tot[3]), fmax(S.tot[5], S.tot[18])), S.tot[20]);
+    for (int it = 0; it < kLmIterations; ++it) {
+        if (tid == 0) {
+            for (int e = 0; e < 64; ++e) S.L[e] = S.J[e];
+            for (int e = 0; e < 8; ++e) S.L[e * 9] += lambda * S.J[e * 9];
+            double d[8], rhs[8];
+            for (int e = 0; e < 8; ++e) rhs[e] = -S.g[e];
+            S.ok = cholesky_solve<8>(S.L, rhs, d);
+            for (int e = 0; e < 8; ++e) S.prm[cur ^ 1][e] = S.prm[cur][e] + d[e];
+        }
+        __syncthreads();
+        const bool solved = S.ok;
+        __syncthreads();                                   // S.ok is rewritten by the next step
+        const double trial = solved ? lm_cost(P, p, n, thr, nm, S.prm[cur ^ 1], S) : INFINITY;
+        if (trial < cost) {
+            const bool done = cost - trial < 1e-12 * cost;
+            cost = trial;
+            cur ^= 1;
+            lambda *= 0.1;
+            if (done) break;
+            lm_normal(P, p, n, thr, nm, S.prm[cur], S);
+        } else {
+            lambda *= 10.0;
+            if (lambda > 1e16) break;
+        }
+    }
+    if (tid == 0) {
+        double Hn[9];
+        for (int e = 0; e < 8; ++e) Hn[e] = S.prm[cur][e];
+        Hn[8] = 1.0;
+        S.ok = denormalise_store(Hn, nm, S.H[1]);
+    }
+    __syncthreads();
+    return S.ok;
+    }
+    }
+}
+
+// Pair p: the inlier set S0 of H_in[p]; round r refits on S(r-1), and keeps the refit unless it is degenerate or has
+// fewer inliers than S(r-1); it stops early when the set no longer changes.  status_out[p] = {status_in[p][0],
+// inliers of the returned model, refits kept}; mask row p = the returned model's inliers.  Pairs without a model
+// (status_in[p][0] == 0) get status {0, 0, 0}, a zero mask row, and H_out[p] is not written.
+template <int KIND>
+__global__ void __launch_bounds__(kRefineThreads, 1) refine_kernel(const Pairs P, float thr, const float* __restrict__ H_in,
+                                                                const int* __restrict__ status_in, int rounds, float* H_out,
+                                                                int* status_out, unsigned char* __restrict__ mask_all)
+{
+    constexpr int M = KIND == 0 ? 1 : KIND == 1 ? 2 : 4;     // minimal sample: no refit with no more points than this
+    __shared__ RefineShared S;
+    const int p = blockIdx.x, n = pair_n(P, p), tid = threadIdx.x;
+    const int has = status_in == nullptr ? 1 : status_in[p * 3];
+    if (tid < 9) S.H[0][tid] = H_in[p * 9 + tid];
+    __syncthreads();                                        // read before written: H_out / status_out may alias the inputs
+    unsigned char* mask = mask_all == nullptr ? nullptr : mask_all + (long long)p * P.max_pts;
+    if (has == 0) {
+        if (mask != nullptr)
+            for (int i = tid; i < P.max_pts; i += kRefineThreads) mask[i] = 0;
+        if (tid == 0) status_out[p * 3] = status_out[p * 3 + 1] = status_out[p * 3 + 2] = 0;
+        return;
+    }
+    double c[1] = {0.0};
+    for_each_inlier(P, p, n, S.H[0], thr, [&](const float4) { c[0] += 1.0; });
+    block_sum(c, S);
+    int cnt = (int)S.tot[0], kept = 0;
+    for (int r = 1; r <= rounds && cnt > M; ++r) {
+        if (!refit<KIND>(P, p, n, thr, cnt, S)) break;
+        double v[2] = {0.0, 0.0};                           // |S_r| and |S_r xor S_(r-1)|
+        {
+            float H0[9], H1[9];
+#pragma unroll
+            for (int e = 0; e < 9; ++e) { H0[e] = S.H[0][e]; H1[e] = S.H[1][e]; }
+            const long long off = (long long)p * P.stride;
+            for (int i = tid; i < n; i += kRefineThreads) {
+                const float4 q = make_float4(P.sx[off + i], P.sy[off + i], P.dx[off + i], P.dy[off + i]);
+                const bool a = transfer_inlier(H0, q, thr), b = transfer_inlier(H1, q, thr);
+                v[0] += b ? 1.0 : 0.0;
+                v[1] += a != b ? 1.0 : 0.0;
+            }
+        }
+        block_sum(v, S);
+        const int cnt_r = (int)S.tot[0], changed = (int)S.tot[1];
+        if (cnt_r < cnt) break;
+        if (tid < 9) S.H[0][tid] = S.H[1][tid];
+        __syncthreads();
+        cnt = cnt_r;
+        kept = r;
+        if (changed == 0) break;
+    }
+    if (mask != nullptr) {
+        float H[9];
+#pragma unroll
+        for (int e = 0; e < 9; ++e) H[e] = S.H[0][e];
+        const long long off = (long long)p * P.stride;
+        for (int i = tid; i < P.max_pts; i += kRefineThreads)
+            mask[i] = i < n && transfer_inlier(H, make_float4(P.sx[off + i], P.sy[off + i], P.dx[off + i], P.dy[off + i]), thr);
+    }
+    if (tid < 9) H_out[p * 9 + tid] = S.H[0][tid];
+    if (tid == 0) {
+        status_out[p * 3] = has;
+        status_out[p * 3 + 1] = cnt;
+        status_out[p * 3 + 2] = kept;
+    }
+}
+
 int min_points(int kind) { return kind == 2 ? 4 : 2; }        // ransac.cu:541, :606, :656 (translation also asks for 2)
 int sample_size(int kind) { return kind == 0 ? 1 : kind == 1 ? 2 : 4; }
 
@@ -563,4 +1030,20 @@ extern "C" int nm_ransac_batch_f32(int kind, const float* src_x, const float* sr
     if (!src_x || !src_y || !dst_x || !dst_y || !homographies || !status) return NM_ERR_INVALID;
     const Pairs P{src_x, src_y, dst_x, dst_y, pair_stride, counts, max_pts};
     return ransac_batch(kind, P, n_pairs, inlier_threshold, iterations, seed, homographies, status, (cudaStream_t)stream);
+}
+
+extern "C" int nm_ransac_refine_batch_f32(int kind, const float* src_x, const float* src_y, const float* dst_x, const float* dst_y,
+                                          long long pair_stride, const int* counts, int max_pts, int n_pairs,
+                                          float inlier_threshold, const float* H_in, const int* status_in, int rounds,
+                                          float* H_out, int* status_out, unsigned char* inlier_mask, nm_stream_t stream)
+{
+    if (kind < 0 || kind > 2 || max_pts <= 0 || n_pairs <= 0 || rounds < 0 || pair_stride < 0) return NM_ERR_INVALID;
+    if (!src_x || !src_y || !dst_x || !dst_y || !H_in || !H_out || !status_out) return NM_ERR_INVALID;
+    const Pairs P{src_x, src_y, dst_x, dst_y, pair_stride, counts, max_pts};
+    cudaStream_t st = (cudaStream_t)stream;
+    if (kind == 0) refine_kernel<0><<<n_pairs, kRefineThreads, 0, st>>>(P, inlier_threshold, H_in, status_in, rounds, H_out, status_out, inlier_mask);
+    else if (kind == 1) refine_kernel<1><<<n_pairs, kRefineThreads, 0, st>>>(P, inlier_threshold, H_in, status_in, rounds, H_out, status_out, inlier_mask);
+    else refine_kernel<2><<<n_pairs, kRefineThreads, 0, st>>>(P, inlier_threshold, H_in, status_in, rounds, H_out, status_out, inlier_mask);
+    NM_LAUNCH_CHECK();
+    return NM_OK;
 }

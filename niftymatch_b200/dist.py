@@ -78,14 +78,16 @@ def match_stream(sift_batch, frames, ambiguity: float = 0.8, world: int = 1, ran
 
 
 def register_stream(sift_batch, frames, kind: int = 2, ambiguity: float = 0.8, inlier_threshold: float = 4.0,
-                    iterations: int = 1024, seed: int = 0, world: int = 1, rank: int = 0, chunk: int = 16):
+                    iterations: int = 1024, seed: int = 0, world: int = 1, rank: int = 0, chunk: int = 16,
+                    refine_rounds: int = 0):
     """BASELINE.json configs[4] with its consumer: SIFT on this rank's frames of a stream, every frame matched to
     its successor, correspondences aligned (align_points) and ONE batched RANSAC over all the rank's pairs.
     Returns (pairs, homographies (n_pairs, 9) cuda, status (n_pairs, 3) cuda); pair t -> t+1 maps frame t's
-    coordinates to frame t+1's.  Pair t uses the seed `seed + t` (independent of the sharding)."""
+    coordinates to frame t+1's.  Pair t uses the seed `seed + t` (independent of the sharding).  refine_rounds > 0
+    refits every model on its inliers (ransac.refine_batch, in place); status[:, 2] is then the refits kept."""
     import torch
     from .match import match as _match
-    from .ransac import align_points, ransac_batch
+    from .ransac import align_points, ransac_batch, refine_batch
     n = frames.shape[0]
     lo, hi, pairs = stream_pairs(n, world, rank)
     cap = sift_batch.capacity
@@ -114,6 +116,8 @@ def register_stream(sift_batch, frames, kind: int = 2, ambiguity: float = 0.8, i
         return pairs, torch.zeros((0, 9), device=dev), torch.zeros((0, 3), dtype=torch.int32, device=dev)
     # one seed per PAIR INDEX of the whole stream, so a sharded run reproduces the single-rank run
     H, st = ransac_batch(kind, *c, counts, inlier_threshold, iterations, seed + lo)
+    if refine_rounds > 0:
+        refine_batch(kind, *c, counts, H, st, inlier_threshold, refine_rounds, out=(H, st))
     return pairs, H, st
 
 
@@ -123,15 +127,17 @@ class StreamRegistrar:
     (nm_align_pairs_f32) and all pairs registered by one batched RANSAC (nm_ransac_batch_f32).  Keypoint counts never
     leave the device and nothing synchronises; consecutive chunks share one frame (recomputed), so no state is carried
     between chunks or between GPUs.  Pair t -> t + 1 draws with seed + t: the result does not depend on the chunking or
-    on how the stream is sharded over ranks (frame_range(..., overlap=1))."""
+    on how the stream is sharded over ranks (frame_range(..., overlap=1)).  refine_rounds > 0 refits each chunk's models
+    on their inliers in place (nm_ransac_refine_batch_f32) right after its RANSAC; status[:, 2] is then the refits kept."""
 
     def __init__(self, sift_batch, chunk=None, kind: int = 2, ambiguity: float = 0.8, inlier_threshold: float = 4.0,
-                 iterations: int = 1024, seed: int = 0):
+                 iterations: int = 1024, seed: int = 0, refine_rounds: int = 0):
         import torch
         self.sb = sift_batch
         self.chunk = min(chunk or sift_batch.max_batch, sift_batch.max_batch)
         assert self.chunk >= 2 and sift_batch.capacity % 256 == 0
         self.kind, self.ambiguity, self.thr, self.iters, self.seed = kind, ambiguity, inlier_threshold, iterations, seed
+        self.refine_rounds = refine_rounds
         cap, n = sift_batch.capacity, self.chunk - 1
         dev = torch.device("cuda", torch.cuda.current_device())
         self.match = torch.empty((n, cap), dtype=torch.int32, device=dev)
@@ -174,5 +180,9 @@ class StreamRegistrar:
             check(lib.nm_ransac_batch_f32(self.kind, *[p(c) for c in self.corr], cap, p(r["counts"]), cap, n - 1, self.thr,
                                           self.iters, (self.seed + c0) & 0xFFFFFFFFFFFFFFFF, p(H[k:]), p(st[k:]), _stream_ptr()),
                   "nm_ransac_batch_f32")
+            if self.refine_rounds > 0:
+                check(lib.nm_ransac_refine_batch_f32(self.kind, *[p(c) for c in self.corr], cap, p(r["counts"]), cap, n - 1,
+                                                     self.thr, p(H[k:]), p(st[k:]), self.refine_rounds, p(H[k:]), p(st[k:]),
+                                                     None, _stream_ptr()), "nm_ransac_refine_batch_f32")
             c0 = c1 - 1
         return H[:n_pairs], st[:n_pairs]

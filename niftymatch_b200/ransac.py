@@ -86,3 +86,43 @@ def ransac_batch(kind, src_x, src_y, dst_x, dst_y, counts, inlier_threshold, ite
                                           iterations, seed & 0xFFFFFFFFFFFFFFFF, _p(H), _p(status), _stream_ptr()),
           "nm_ransac_batch_f32")
     return H, status
+
+
+def refine_batch(kind, src_x, src_y, dst_x, dst_y, counts, H, status, inlier_threshold, rounds=2, out=None):
+    """nm_ransac_refine_batch_f32: least-squares refits of the models H (n_pairs, 9) on their inlier sets, and the inlier
+    masks.  Correspondences and counts as for ransac_batch; status (n_pairs, 3) cuda int32 as ransac_batch returns it, or
+    None.  out = (H_out, status_out) writes there (they may be H and status: in place).  Returns (H (n_pairs, 9),
+    status (n_pairs, 3) = [ok, inliers, refits kept], mask (n_pairs, max_pts) bool)."""
+    import torch
+    _f32(src_x, src_y, dst_x, dst_y)
+    if counts is not None:
+        _int32(counts, "counts")
+    n_pairs, max_pts = src_x.shape
+    if not (isinstance(H, torch.Tensor) and H.is_cuda and H.dtype == torch.float32 and H.is_contiguous()
+            and tuple(H.shape) == (n_pairs, 9)):
+        raise TypeError("H: expected a contiguous cuda float32 tensor of shape (n_pairs, 9)")
+    if status is not None:
+        _int32(status, "status")
+        assert tuple(status.shape) == (n_pairs, 3)
+    if out is None:
+        H_out = torch.empty_like(H)
+        st_out = torch.zeros((n_pairs, 3), dtype=torch.int32, device=src_x.device)
+    else:
+        H_out, st_out = out
+        _f32(H_out, H); _int32(st_out, "status_out")
+        assert tuple(st_out.shape) == (n_pairs, 3)
+    mask = torch.empty((n_pairs, max_pts), dtype=torch.bool, device=src_x.device)
+    check(_lib.load().nm_ransac_refine_batch_f32(kind, _p(src_x), _p(src_y), _p(dst_x), _p(dst_y), max_pts,
+                                                 _p(counts) if counts is not None else None, max_pts, n_pairs,
+                                                 inlier_threshold, _p(H), _p(status) if status is not None else None,
+                                                 rounds, _p(H_out), _p(st_out), _p(mask), _stream_ptr()),
+          "nm_ransac_refine_batch_f32")
+    return H_out, st_out, mask
+
+
+def refine(kind, src_x, src_y, dst_x, dst_y, H, status, inlier_threshold, rounds=2):
+    """refine_batch for one pair: src_x ... dst_y (n,), H (9,), status (3,) or None.  Returns (H (9,), status (3,),
+    mask (n,) bool)."""
+    Hb, sb, mb = refine_batch(kind, src_x[None], src_y[None], dst_x[None], dst_y[None], None, H.reshape(1, 9),
+                              None if status is None else status.reshape(1, 3), inlier_threshold, rounds)
+    return Hb[0], sb[0], mb[0]

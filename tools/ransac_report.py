@@ -1,12 +1,103 @@
 """Registration parity report on a GPU box: product (C-ABI) vs the reference's kernels (oracle/_ref) vs the CPU
-oracle on the fixture scene of tests/_util.py (development aid)."""
+oracle on the fixture scene of tests/_util.py (development aid).
+
+--refine: the refit leg instead (nm_ransac_refine_batch_f32): time of the batched RANSAC alone and followed by 1 or 2
+refit rounds (64 pairs x 8 192 correspondences, 70 % inliers, 1 024 hypotheses; CUDA events, the three variants in
+alternating windows), corner error against the ground truth of the RANSAC model, the refit and a float64 fit to the
+true inliers, and the 2 048-frame 1080p StreamRegistrar rate of bench.py with refine_rounds 0 and 2."""
 import os
+import subprocess
 import sys
 import numpy as np
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 import torch  # noqa: E402
 import niftymatch_b200 as nm  # noqa: E402
+
+
+def refine_leg():
+    import bench
+    from tests.test_gpu_ransac_refine import scene, true_model, fit_homography, corner_error
+    from niftymatch_b200.dist import StreamRegistrar
+    stream_np = bench.render_frames(bench.stream_jobs(0, 32))
+    card = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit", "--format=csv,noheader", "-i", "0"],
+                          capture_output=True, text=True).stdout.strip()
+    print("card:", card)
+    rng = np.random.default_rng(12)
+    n_pairs, n, thr = 64, 8192, 4.0
+    arrs = [np.empty((n_pairs, n), np.float32) for _ in range(4)]
+    truth, floor = [], []
+    for p in range(n_pairs):
+        Ht = true_model(2, rng)
+        sc = scene(Ht, n, rng)
+        for a, v in zip(arrs, sc[:4]):
+            a[p] = v
+        m = sc[4]
+        floor.append(corner_error(fit_homography(np.stack([sc[0][m], sc[1][m]], 1).astype(np.float64),
+                                                 np.stack([sc[2][m], sc[3][m]], 1).astype(np.float64)), Ht))
+        truth.append(Ht)
+    d = [torch.from_numpy(a).cuda() for a in arrs]
+    H, st = nm.ransac_batch(2, *d, None, thr, 1024, 1)
+    outs = {r: nm.refine_batch(2, *d, None, H, st, thr, rounds=r) for r in (1, 2)}
+    Hn, stn = H.cpu().numpy(), st.cpu().numpy()
+    rows = [("RANSAC model", [corner_error(Hn[p], truth[p]) for p in range(n_pairs)])]
+    for r in (1, 2):
+        Hr = outs[r][0].cpu().numpy()
+        rows.append((f"refined, rounds = {r}", [corner_error(Hr[p], truth[p]) for p in range(n_pairs)]))
+        print(f"rounds {r}: refits kept {np.bincount(outs[r][1][:, 2].cpu().numpy()).tolist()}, inliers "
+              f"{stn[:, 1].sum()} -> {int(outs[r][1][:, 1].sum())}")
+    rows.append(("float64 fit to the true inliers", floor))
+    for name, e in rows:
+        e = np.array(e)
+        print(f"corner error, {name}: mean {e[:, 1].mean():.4f} px, max {e[:, 0].max():.4f} px")
+
+    def run(rounds):
+        H, st = nm.ransac_batch(2, *d, None, thr, 1024, 1)
+        if rounds:
+            nm.refine_batch(2, *d, None, H, st, thr, rounds=rounds, out=(H, st))
+    for r in (0, 1, 2):
+        for _ in range(3):
+            run(r)
+    torch.cuda.synchronize()
+    times = {0: [], 1: [], 2: []}
+    for _ in range(8):
+        for r in (0, 1, 2):
+            e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+            e0.record()
+            for _ in range(10):
+                run(r)
+            e1.record()
+            torch.cuda.synchronize()
+            times[r].append(e0.elapsed_time(e1) / 10 * 1e3)
+    for r in (0, 1, 2):
+        t = np.array(times[r])
+        print(f"nm_ransac_batch_f32{'' if r == 0 else f' + refine rounds = {r}'}: median {np.median(t):.0f} us "
+              f"(windows {t.min():.0f} - {t.max():.0f}); refine share {np.median(t) - np.median(times[0]):.0f} us")
+    # the stream leg of bench.py on one GPU, with and without the refit
+    P = nm.SiftParams(bench.W, bench.H)
+    sb = nm.SiftBatch(P, bench.BATCH, bench.CAPACITY)
+    base = torch.from_numpy(stream_np).cuda()
+    frames_of = lambda t0, t1: base.index_select(0, torch.arange(t0, t1, device="cuda") % base.shape[0])
+    n_stream = 2048
+    for rep in range(2):
+        for rounds in (0, 2):
+            reg = StreamRegistrar(sb, chunk=sb.max_batch, refine_rounds=rounds)
+            reg.run(frames_of, 0, sb.max_batch + 1)
+            torch.cuda.synchronize()
+            e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+            e0.record()
+            Hs, sts = reg.run(frames_of, 0, n_stream)
+            e1.record()
+            torch.cuda.synchronize()
+            ms = e0.elapsed_time(e1)
+            print(f"stream {n_stream} frames 1080p, refine_rounds {rounds}: {n_stream / ms * 1e3:.0f} frames/s "
+                  f"({ms:.1f} ms), registered pairs {int((sts[:, 0] == 1).sum())}")
+    sb.close()
+
+
+if "--refine" in sys.argv:
+    refine_leg()
+    sys.exit(0)
 from tests._util import (load_oracle, load_reflib, ransac_scene, ransac_rand_lists, checker_ransac_hypotheses,  # noqa: E402
                          normalise_h)
 
