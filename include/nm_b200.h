@@ -181,6 +181,17 @@ int nm_match_merge_top2_strided(const float* recs4, int n_shards, long long shar
 int nm_match_pairs_f32(const float* desc, const int* counts_dev, int n_frames, int capacity, float ambiguity,
                        int* match_out, float* rec_out4, int* fallback_rows_dev, nm_stream_t stream);
 
+/* The SPAN LAYOUT of a window of n frames, 1 <= span <= min(8, n - 1): its links are the pairs (t, t + d), 1 <= d <= span,
+ * 0 <= t < n - d, stored d-major -- link (t, d) is row l = sum_{e<d} (n - e) + t, and there are
+ * L = span * n - span * (span + 1) / 2 rows.  Rows 0 .. n-2 are the consecutive pairs, in the layout of nm_match_pairs_f32.
+ * Correspondence i of a link is (frame t point, frame t + d point); a link's model maps frame t to frame t + d.
+ *
+ * nm_match_pairs_f32 for every link of the layout: match_out and rec_out4 are [L][capacity], entry (l, a) gets the
+ * index into frame t + d.  Link (t, d) is bitwise nm_match_f32(frame t, frame t + d); span 1 is bitwise
+ * nm_match_pairs_f32.  Every frame is still packed once; sizes are read on the device and nothing synchronises. */
+int nm_match_pairs_span_f32(const float* desc, const int* counts_dev, int n_frames, int capacity, int span, float ambiguity,
+                            int* match_out, float* rec_out4, int* fallback_rows_dev, nm_stream_t stream);
+
 /* Which candidate-search engine nm_match_* uses: 0 = exact fp32 SIMT scan,
  * 1 = tcgen05 contraction + fp32 re-rank (default when the device is sm_100). */
 int nm_match_set_engine(int engine);
@@ -310,6 +321,13 @@ int nm_align_points_f32(const float* src_x, const float* src_y, const float* dst
 int nm_align_pairs_f32(const float* x, const float* y, const int* matches, const int* counts_dev, int n_frames,
                        int capacity, float* c_src_x, float* c_src_y, float* c_dst_x, float* c_dst_y, nm_stream_t stream);
 
+/* nm_align_pairs_f32 for every link of the span layout (see nm_match_pairs_span_f32): matches and the outputs are
+ * [L][capacity]; correspondence (l, i) = (frame t point i, frame t + d point matches[l][i]), or (-1,-1,-1,-1) when
+ * unmatched or i >= counts[t].  Span 1 is bitwise nm_align_pairs_f32. */
+int nm_align_pairs_span_f32(const float* x, const float* y, const int* matches, const int* counts_dev, int n_frames,
+                            int capacity, int span, float* c_src_x, float* c_src_y, float* c_dst_x, float* c_dst_y,
+                            nm_stream_t stream);
+
 /* Estimator kinds. */
 #define NM_RANSAC_TRANSLATION 0   /* 1 correspondence / hypothesis (ransac.cu:467-486) */
 #define NM_RANSAC_SIMILARITY  1   /* 2 (ransac.cu:437-464, :322-435) */
@@ -362,6 +380,34 @@ int nm_ransac_refine_batch_f32(int kind, const float* src_x, const float* src_y,
                                long long pair_stride, const int* counts, int max_pts, int n_pairs, float inlier_threshold,
                                const float* H_in, const int* status_in, int rounds,
                                float* H_out, int* status_out, unsigned char* inlier_mask, nm_stream_t stream);
+
+/* Joint adjustment of the chain of a window of n_frames frames registered with skip links (no reference counterpart).
+ * The window's L links are in the span layout (nm_match_pairs_span_f32): correspondences, pair_stride, counts (per
+ * link, NULL = max_pts) and max_pts as nm_ransac_refine_batch_f32 reads them; H_links [L][9], link_status [L][3] and
+ * masks [L][max_pts] as it writes them (RANSAC per d with nm_ransac_batch_f32, then the refit or rounds = 0 for the masks).
+ *   Unknowns: G_k maps frame k into frame-0 pixels, G_0 = I; G_k = N^-1 Gn_k N, N centres the frame and scales it by
+ *     2 / max(frame_w, frame_h), Gn_k in the family of `kind` (2 / 4 / 8 parameters, homography Gn[8] = 1).  fp64.
+ *   Initial poses: for k = 1 .. n-1 the smallest d <= span with frame k-d connected, link_status[(k-d, d)][0] == 1 and
+ *     at least 1 / 2 / 4 mask points gives G_k = G_(k-d) . H^-1 (the chaining rule of nm_mosaic_place_f32); without one
+ *     frame k is disconnected: G_k = G_(k-1), fixed, and its links are ignored.
+ *   Cost: sum over the links usable that way (both frames connected) and their mask points of
+ *     |pi(G_t s_i) - pi(G_(t+d) d_i)|^2, in frame-0 pixels.
+ *   Solver: Levenberg-Marquardt, lambda0 = 1e-3 max diag(J^T J), / 10 after an accepted step, * 10 after a rejected one,
+ *     at most `iterations` (>= 1) builds of the banded normal equations, banded Cholesky in one CTA; the final cost is
+ *     never above the initial one.
+ *   H_out [n-1][9] (may alias H_links): G_(p+1)^-1 G_p rounded to float, divided by its [8], when frame p+1 is connected
+ *     (a disconnected frame p gives the pair out of it that reproduces G_(p+1) in nm_mosaic_place_f32), else H_links[p].
+ *   status_out [n-1][3] (may alias link_status): {1, inliers of H_out[p] under the RANSAC rule on link (p, 1), LM steps
+ *     accepted} for a connected frame p+1, {0, 0, 0} for a disconnected one.
+ *   chain_out [n][9] doubles G_k, or NULL;  report_out [4] doubles, or NULL: mean squared residual (px^2) before and
+ *     after, residual points, links used.
+ * Limits n_frames <= 1024, span <= 8, span < n_frames.  Stream-ordered workspace, no host synchronisation (the call can
+ * be captured in a CUDA graph); the result is bit-reproducible. */
+int nm_ransac_adjust_chain_f32(int kind, const float* src_x, const float* src_y, const float* dst_x, const float* dst_y,
+                               long long pair_stride, const int* counts, int max_pts, float inlier_threshold,
+                               int n_frames, int span, int frame_w, int frame_h, const unsigned char* masks,
+                               const float* H_links, const int* link_status, int iterations, float* H_out,
+                               int* status_out, double* chain_out, double* report_out, nm_stream_t stream);
 
 /* ------------------------------------------------------------------------ */
 /* Batched SIFT detect+describe: the client loop of the reference             */

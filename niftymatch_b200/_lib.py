@@ -61,6 +61,7 @@ SIGNATURES = {
     "nm_match_merge_top2": (_i, [_vp, _i, _i, _f, _vp, _vp]),
     "nm_match_merge_top2_strided": (_i, [_vp, _i, C.c_longlong, _i, _f, _vp, _vp]),
     "nm_match_pairs_f32": (_i, [_vp, _vp, _i, _i, _f, _vp, _vp, _vp, _vp]),
+    "nm_match_pairs_span_f32": (_i, [_vp, _vp, _i, _i, _i, _f, _vp, _vp, _vp, _vp]),
     "nm_match_tc_probe": (_i, [_vp, _i, _vp, _i, _vp, C.POINTER(_i), _vp, _vp, C.POINTER(_i), C.POINTER(_f), _vp]),
     "nm_grayscale_bgra_f32": (_i, [_vp, _vp, _i, _i, _vp]),
     "nm_bgra_extract_channel_f32": (_i, [_vp, _vp, _i, _i, _i, _vp]),
@@ -80,10 +81,13 @@ SIGNATURES = {
     "nm_sift_run_bgra": (_i, [_vp, _vp, _i, _vp]),
     "nm_align_points_f32": (_i, [_vp] * 9 + [_i, _vp]),
     "nm_align_pairs_f32": (_i, [_vp, _vp, _vp, _vp, _i, _i, _vp, _vp, _vp, _vp, _vp]),
+    "nm_align_pairs_span_f32": (_i, [_vp, _vp, _vp, _vp, _i, _i, _i, _vp, _vp, _vp, _vp, _vp]),
     "nm_ransac_hypotheses_f32": (_i, [_i, _vp, _vp, _vp, _vp, _i, _vp, _i, _f, _vp, _vp, _vp]),
     "nm_ransac_f32": (_i, [_i, _vp, _vp, _vp, _vp, _i, _f, _i, _ull, _vp, _vp, _vp]),
     "nm_ransac_batch_f32": (_i, [_i, _vp, _vp, _vp, _vp, C.c_longlong, _vp, _i, _i, _f, _i, _ull, _vp, _vp, _vp]),
     "nm_ransac_refine_batch_f32": (_i, [_i, _vp, _vp, _vp, _vp, C.c_longlong, _vp, _i, _i, _f, _vp, _vp, _i, _vp, _vp, _vp, _vp]),
+    "nm_ransac_adjust_chain_f32": (_i, [_i, _vp, _vp, _vp, _vp, C.c_longlong, _vp, _i, _f, _i, _i, _i, _i, _vp, _vp, _vp, _i,
+                                        _vp, _vp, _vp, _vp, _vp]),
     "nm_match_set_engine": (_i, [_i]),
     "nm_match_get_engine": (_i, []),
     "nm_sift_create": (_i, [C.POINTER(_vp), C.POINTER(SiftParamsC), _i, _i]),

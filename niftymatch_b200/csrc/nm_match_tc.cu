@@ -280,11 +280,12 @@ struct TcScanArgs {
     const int4*    seed_i;
     int            nA, tile_first, tile_end, tiles_per_split;   // split s scans tiles tile_first + s*tps ...
     uint32_t       lbo, sbo;    // descriptor strides in bytes (k-chunk stride, 8-row-group stride)
-    // batched mode (nm_match_pairs_f32; counts != null): blockIdx.z = frame pair z, queries = frame z, database =
-    // frame z + 1; every size is read on the device.  a_pack / b_pack hold `capacity / 128` tiles per frame,
-    // the candidate lists are [pair][2 * gridDim.y][capacity].
+    // batched mode (nm_match_pairs_span_f32; counts != null): blockIdx.z = link z of the span layout over n_frames
+    // frames, queries = frame t, database = frame t + d (SPAN = false: t = z, d = 1); every size is read on the
+    // device.  a_pack / b_pack hold `capacity / 128` tiles per frame, the candidate lists are [link][2 * gridDim.y][capacity].
     const int*     counts;
     int            capacity;
+    int            n_frames;
 };
 
 #define TC_INSERT(val, idx)                                                                        \
@@ -328,6 +329,8 @@ struct TcScanArgs {
         }                                                                                          \
     } while (0)
 
+// SPAN is a template parameter so that the single-pair and consecutive-pair instantiations carry no link decode.
+template <bool SPAN>
 __global__ void __launch_bounds__(TC_THREADS, 1) tc_scan_kernel(const TcScanArgs p)
 {
     extern __shared__ __align__(128) uint8_t smem_raw[];
@@ -353,17 +356,18 @@ __global__ void __launch_bounds__(TC_THREADS, 1) tc_scan_kernel(const TcScanArgs
     size_t list_base = 0;
     int list_rows = p.nA;
     if (p.counts != nullptr) {
-        const int pair = blockIdx.z;
-        nA = min(p.counts[pair], p.capacity);
-        const int nB = min(p.counts[pair + 1], p.capacity);
+        int fa = blockIdx.z, d = 1;
+        if (SPAN) nm_link_decode(blockIdx.z, p.n_frames, fa, d);
+        nA = min(p.counts[fa], p.capacity);
+        const int nB = min(p.counts[fa + d], p.capacity);
         if (rb * TC_ROWBLK >= nA || nB <= 0) return;             // the whole CTA: nothing allocated or initialised yet
         const size_t frame_bytes = (size_t)(p.capacity / TC_TROWS) * TC_TILE_BYTES;
-        a_pack += (size_t)pair * frame_bytes;
-        b_pack += (size_t)(pair + 1) * frame_bytes;
+        a_pack += (size_t)fa * frame_bytes;
+        b_pack += (size_t)(fa + d) * frame_bytes;
         tile_first = 0;
         tile_end = (nB + TC_TROWS - 1) / TC_TROWS;
         tiles_per_split = (tile_end + (int)gridDim.y - 1) / (int)gridDim.y;
-        list_base = (size_t)pair * (2 * gridDim.y) * p.capacity;
+        list_base = (size_t)blockIdx.z * (2 * gridDim.y) * p.capacity;
         list_rows = p.capacity;
     }
     const int t0 = tile_first + split * tiles_per_split;
@@ -742,29 +746,34 @@ __global__ void __launch_bounds__(256) pairs_pack_kernel(const float* __restrict
     }
 }
 
-// One warp per (query row, pair): exact re-rank with the certificate; a row that is not certified is scanned
+// One warp per (query row, link (t, t + d) of the span layout; SPAN = false: link = pair (p, p + 1)): exact re-rank with
+// the certificate; a row that is not certified is scanned
 // exactly against the whole database frame BY THIS WARP (lanes stride over the rows; a few thousand rows: microseconds,
 // and it happens to a fraction of a per cent of the rows), so the record is exact either way.  Then the reference's
 // ratio rule (match.cu:88-116) writes the match index.
+template <bool SPAN>
 __global__ void __launch_bounds__(256) pairs_rerank_kernel(const float* __restrict__ desc, const int* __restrict__ counts,
                                                            int capacity, int n_lists, const float4* __restrict__ cand_s,
                                                            const int4* __restrict__ cand_i, const unsigned* __restrict__ hdr,
                                                            const unsigned* __restrict__ fhdr, float ambiguity,
                                                            int* __restrict__ match_out, float4* __restrict__ rec_out,
-                                                           int* __restrict__ fallback_rows)
+                                                           int* __restrict__ fallback_rows, int n_frames)
 {
     __shared__ __align__(16) float s_a[8][128];
     const int wid = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int a = blockIdx.x * 8 + wid, pair = blockIdx.y;
-    const int nA = min(counts[pair], capacity), nB = min(counts[pair + 1], capacity);
+    int fa = pair, d = 1;
+    if (SPAN) nm_link_decode(pair, n_frames, fa, d);
+    const int fb = fa + d;
+    const int nA = min(counts[fa], capacity), nB = min(counts[fb], capacity);
     if (a >= nA || nB <= 0) return;                               // warp uniform
-    const float* __restrict__ A = desc + (size_t)pair * capacity * 128;
-    const float* __restrict__ B = desc + (size_t)(pair + 1) * capacity * 128;
+    const float* __restrict__ A = desc + (size_t)fa * capacity * 128;
+    const float* __restrict__ B = desc + (size_t)fb * capacity * 128;
     const size_t lists = (size_t)pair * n_lists * capacity + a;
     float t1, t2;
     int i1;
     const bool certified = tc_rerank_row(A + (size_t)a * 128, s_a[wid], B, nB, n_lists, cand_s + lists, cand_i + lists,
-                                         (size_t)capacity, hdr[0], fhdr[2 * (pair + 1)], fhdr[2 * (pair + 1) + 1], t1, i1, t2);
+                                         (size_t)capacity, hdr[0], fhdr[2 * fb], fhdr[2 * fb + 1], t1, i1, t2);
     if (!certified) {
         // exact scan: match.cu:36-42 per column, ties to the lowest index
         float d1 = INFINITY, d2 = INFINITY;
@@ -822,7 +831,8 @@ bool nm_match_tc_available()
     bool ok = cudaDeviceGetAttribute(&major, cudaDevAttrComputeCapabilityMajor, dev) == cudaSuccess && major == 10 &&
               cudaDeviceGetAttribute(&smem, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev) == cudaSuccess &&
               smem >= TC_SMEM_BYTES;
-    if (ok) ok = cudaFuncSetAttribute(tc_scan_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, TC_SMEM_BYTES) == cudaSuccess;
+    if (ok) ok = cudaFuncSetAttribute(tc_scan_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, TC_SMEM_BYTES) == cudaSuccess;
+    if (ok) ok = cudaFuncSetAttribute(tc_scan_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, TC_SMEM_BYTES) == cudaSuccess;
     if (!ok) cudaGetLastError();
     if (dev >= 0 && dev < 64) state[dev].store(ok ? 1 : -1, std::memory_order_release);
     return ok;
@@ -911,12 +921,12 @@ static int tc_run(const float* A, int nA, const float* B, int nB, int index_offs
         tc_absmax_kernel<<<ga + gb, 256, 0, stream>>>(A, ea4, ga, B, eb4, hdr);
         tc_pack_kernel<<<n_atiles + n_btiles, 256, 0, stream>>>(A, nA, n_atiles, a_pack, B, nB, b_pack, hdr);
         if (seed_tiles > 0) {
-            TcScanArgs ss{a_pack, b_pack, seed_s, seed_i, nullptr, nullptr, nA, 0, seed_tiles, seed_tiles, TC_KSTRIDE, 128, nullptr, 0};
-            tc_scan_kernel<<<dim3(n_rowblocks, 1), TC_THREADS, TC_SMEM_BYTES, stream>>>(ss);
+            TcScanArgs ss{a_pack, b_pack, seed_s, seed_i, nullptr, nullptr, nA, 0, seed_tiles, seed_tiles, TC_KSTRIDE, 128, nullptr, 0, 0};
+            tc_scan_kernel<false><<<dim3(n_rowblocks, 1), TC_THREADS, TC_SMEM_BYTES, stream>>>(ss);
         }
         TcScanArgs sa{a_pack, b_pack, cand_s, cand_i, seed_tiles > 0 ? seed_s : nullptr, seed_tiles > 0 ? seed_i : nullptr,
-                      nA, seed_tiles, n_btiles, tiles_per_split, TC_KSTRIDE, 128, nullptr, 0};
-        tc_scan_kernel<<<dim3(n_rowblocks, n_splits), TC_THREADS, TC_SMEM_BYTES, stream>>>(sa);
+                      nA, seed_tiles, n_btiles, tiles_per_split, TC_KSTRIDE, 128, nullptr, 0, 0};
+        tc_scan_kernel<false><<<dim3(n_rowblocks, n_splits), TC_THREADS, TC_SMEM_BYTES, stream>>>(sa);
         tc_rerank_kernel<<<nm_div_up(nA, 8), 256, 0, stream>>>(A, nA, B, nB, n_lists, cand_s, cand_i, hdr, index_offset, rec4,
                                                                fb_list, fb_count);
         e = cudaGetLastError();
@@ -945,31 +955,33 @@ static int tc_run(const float* A, int nA, const float* B, int nB, int index_offs
     return rc;
 }
 
-// compute_sift_matches (gpu/sift/siftfunctions.cu:15-40) for every consecutive pair of a SIFT batch, in one launch
-// sequence with no host synchronisation: BASELINE.json configs[4] (frame t matched to t + 1).
+// compute_sift_matches (gpu/sift/siftfunctions.cu:15-40) for every link (t, t + d), d <= span, of a SIFT batch in the
+// span layout (nm_span_links), in one launch sequence with no host synchronisation; span 1 = the consecutive pairs,
+// BASELINE.json configs[4] (frame t matched to t + 1).
 //   desc       [n_frames][capacity][128] floats (the layout of nm_sift_results)
 //   counts_dev [n_frames] descriptors per frame (device)
-//   match_out  [n_frames - 1][capacity] ints: entry (p, a), a < counts[p], gets the index into frame p + 1 or -1;
-//              entries whose second distance is <= 0 keep their previous value (match.cu:107), rows >= counts[p] too
-//   rec_out    optional [n_frames - 1][capacity] float4 records (d1, bits(i1), d2, 0); fallback_rows_dev optional
+//   match_out  [links][capacity] ints: entry (l, a), a < counts[t], gets the index into frame t + d or -1;
+//              entries whose second distance is <= 0 keep their previous value (match.cu:107), rows >= counts[t] too
+//   rec_out    optional [links][capacity] float4 records (d1, bits(i1), d2, 0); fallback_rows_dev optional
 //              device counter of the rows that were scanned exactly
-extern "C" int nm_match_pairs_f32(const float* desc, const int* counts_dev, int n_frames, int capacity, float ambiguity,
-                                  int* match_out, float* rec_out4, int* fallback_rows_dev, nm_stream_t stream_)
+static int match_links(const float* desc, const int* counts_dev, int n_frames, int capacity, int span, float ambiguity,
+                       int* match_out, float* rec_out4, int* fallback_rows_dev, cudaStream_t stream)
 {
     if (!desc || !counts_dev || !match_out || n_frames < 2 || capacity <= 0) return NM_ERR_INVALID;
+    if (span < 1 || span > 8 || span > n_frames - 1) return NM_ERR_INVALID;
     if (capacity % TC_ROWBLK) return NM_ERR_INVALID;             // whole 256-row blocks per frame
     if (reinterpret_cast<uintptr_t>(desc) & 15) return NM_ERR_INVALID;
     if (!nm_match_tc_available()) return NM_ERR_UNSUPPORTED;
-    cudaStream_t stream = (cudaStream_t)stream_;
-    const int n_pairs = n_frames - 1;
+    const int n_links = nm_span_links(n_frames, span);
+    if (n_links > 65535) return NM_ERR_INVALID;
     const int tiles = capacity / TC_TROWS, rowblocks = capacity / TC_ROWBLK;
     // splits: a frame pair is small (a few thousand rows each way), so the database is cut in up to 4 pieces to get
     // enough CTAs per pair and 8 candidate lists (32 candidates) per row for the certificate
     const int n_splits = 4, n_lists = 2 * n_splits;
     const size_t off_f = 256;                                                                   // per-frame headers
     const size_t off_cs = (off_f + sizeof(unsigned) * 2 * (size_t)n_frames + 255) & ~size_t(255);
-    const size_t off_ci = off_cs + sizeof(float4) * (size_t)n_pairs * n_lists * capacity;
-    const size_t off_ap = (off_ci + sizeof(int4) * (size_t)n_pairs * n_lists * capacity + 255) & ~size_t(255);
+    const size_t off_ci = off_cs + sizeof(float4) * (size_t)n_links * n_lists * capacity;
+    const size_t off_ap = (off_ci + sizeof(int4) * (size_t)n_links * n_lists * capacity + 255) & ~size_t(255);
     const size_t off_bp = off_ap + (size_t)n_frames * tiles * TC_TILE_BYTES;
     const size_t total = off_bp + (size_t)n_frames * tiles * TC_TILE_BYTES;
     uint8_t* ws = nullptr;
@@ -982,15 +994,37 @@ extern "C" int nm_match_pairs_f32(const float* desc, const int* counts_dev, int 
     if (e == cudaSuccess) {
         pairs_absmax_kernel<<<dim3(32, n_frames), 256, 0, stream>>>(desc, counts_dev, capacity, hdr);
         pairs_pack_kernel<<<dim3(tiles, n_frames), 256, 0, stream>>>(desc, counts_dev, capacity, ws + off_ap, ws + off_bp, hdr, fhdr);
-        TcScanArgs sa{ws + off_ap, ws + off_bp, cand_s, cand_i, nullptr, nullptr, 0, 0, 0, 0, TC_KSTRIDE, 128, counts_dev, capacity};
-        tc_scan_kernel<<<dim3(rowblocks, n_splits, n_pairs), TC_THREADS, TC_SMEM_BYTES, stream>>>(sa);
-        pairs_rerank_kernel<<<dim3(capacity / 8, n_pairs), 256, 0, stream>>>(desc, counts_dev, capacity, n_lists, cand_s, cand_i, hdr,
-                                                                            fhdr, ambiguity, match_out,
-                                                                            reinterpret_cast<float4*>(rec_out4), fallback_rows_dev);
+        TcScanArgs sa{ws + off_ap, ws + off_bp, cand_s, cand_i, nullptr, nullptr, 0, 0, 0, 0, TC_KSTRIDE, 128, counts_dev, capacity,
+                      n_frames};
+        const dim3 sg(rowblocks, n_splits, n_links), rg(capacity / 8, n_links);
+        float4* rec = reinterpret_cast<float4*>(rec_out4);
+        if (span == 1) {
+            tc_scan_kernel<false><<<sg, TC_THREADS, TC_SMEM_BYTES, stream>>>(sa);
+            pairs_rerank_kernel<false><<<rg, 256, 0, stream>>>(desc, counts_dev, capacity, n_lists, cand_s, cand_i, hdr, fhdr, ambiguity,
+                                                               match_out, rec, fallback_rows_dev, n_frames);
+        } else {
+            tc_scan_kernel<true><<<sg, TC_THREADS, TC_SMEM_BYTES, stream>>>(sa);
+            pairs_rerank_kernel<true><<<rg, 256, 0, stream>>>(desc, counts_dev, capacity, n_lists, cand_s, cand_i, hdr, fhdr, ambiguity,
+                                                              match_out, rec, fallback_rows_dev, n_frames);
+        }
         e = cudaGetLastError();
     }
     cudaFreeAsync(ws, stream);
     return nm_cuda_err(e);
+}
+
+extern "C" int nm_match_pairs_f32(const float* desc, const int* counts_dev, int n_frames, int capacity, float ambiguity,
+                                  int* match_out, float* rec_out4, int* fallback_rows_dev, nm_stream_t stream)
+{
+    return match_links(desc, counts_dev, n_frames, capacity, 1, ambiguity, match_out, rec_out4, fallback_rows_dev,
+                       (cudaStream_t)stream);
+}
+
+extern "C" int nm_match_pairs_span_f32(const float* desc, const int* counts_dev, int n_frames, int capacity, int span,
+                                       float ambiguity, int* match_out, float* rec_out4, int* fallback_rows_dev, nm_stream_t stream)
+{
+    return match_links(desc, counts_dev, n_frames, capacity, span, ambiguity, match_out, rec_out4, fallback_rows_dev,
+                       (cudaStream_t)stream);
 }
 
 int nm_match_scan_tc(const float* A, int nA, const float* B, int nB, int index_offset, float4* rec4, cudaStream_t stream)

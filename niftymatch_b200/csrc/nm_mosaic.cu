@@ -10,7 +10,7 @@
 // The mosaic of a registered frame stream (nm_mosaic_*): place_kernel chains the pairwise homographies into
 // frame -> mosaic transforms and lays the frames out on a canvas; blend_stream_kernel blends a chunk of frames
 // in one pass over the canvas, bitwise what one transform_blend call per frame, in frame order, produces.
-#include "nm_common.cuh"
+#include "nm_chain.cuh"
 #include <climits>
 #include <cstdint>
 #include <cstring>
@@ -266,42 +266,7 @@ __global__ void __launch_bounds__(kMosaicThreads) blend_stream_kernel(uchar4* __
     }
 }
 
-// Placement of a registered stream, fp64.  3x3 helpers, row-major.
-__device__ __forceinline__ double det3d(const double* a)
-{
-    return a[0] * (a[4] * a[8] - a[5] * a[7]) - a[1] * (a[3] * a[8] - a[5] * a[6]) + a[2] * (a[3] * a[7] - a[4] * a[6]);
-}
-// r = a^-1 (adjugate over the determinant)
-__device__ __forceinline__ void inv3d(const double* a, double det, double* r)
-{
-    r[0] = (a[4] * a[8] - a[5] * a[7]) / det;
-    r[1] = (a[2] * a[7] - a[1] * a[8]) / det;
-    r[2] = (a[1] * a[5] - a[2] * a[4]) / det;
-    r[3] = (a[5] * a[6] - a[3] * a[8]) / det;
-    r[4] = (a[0] * a[8] - a[2] * a[6]) / det;
-    r[5] = (a[2] * a[3] - a[0] * a[5]) / det;
-    r[6] = (a[3] * a[7] - a[4] * a[6]) / det;
-    r[7] = (a[1] * a[6] - a[0] * a[7]) / det;
-    r[8] = (a[0] * a[4] - a[1] * a[3]) / det;
-}
-__device__ __forceinline__ double max_abs9(const double* a)
-{
-    double m = 0.0;
-    for (int i = 0; i < 9; ++i) m = fmax(m, fabs(a[i]));
-    return m;
-}
-// divide by the power of two at the largest absolute entry (max in [0.5, 1) afterwards): exact, so a chain of
-// thousands of frames neither overflows nor picks up rounding from the rescaling
-__device__ __forceinline__ void renormalise(double* a)
-{
-    const double m = max_abs9(a);
-    if (!(m > 0.0) || !isfinite(m)) return;
-    int e;
-    frexp(m, &e);
-    const double s = ldexp(1.0, -e);
-    for (int i = 0; i < 9; ++i) a[i] *= s;
-}
-
+// Placement of a registered stream, fp64, row-major 3x3 (helpers in nm_chain.cuh).
 constexpr int kPlaceThreads = 256;
 constexpr int kPlaceBlock = 128;            // frames whose transforms are staged in shared memory at a time
 constexpr double kPlaceMaxCoord = 1073741824.0;   // 2^30: footprints beyond this are not representable as rects
@@ -319,15 +284,8 @@ __global__ void __launch_bounds__(kPlaceThreads) place_kernel(const float* __res
     const int tid = threadIdx.x;
     // steps H[p]^-1 in parallel, written where G[p + 1] will go
     for (int p = tid; p < n - 1; p += kPlaceThreads) {
-        double h[9], r[9];
-        bool ok = status == nullptr || status[(long long)p * 3] != 0;
-        for (int i = 0; i < 9; ++i) { h[i] = (double)H[(long long)p * 9 + i]; ok = ok && isfinite(h[i]); }
-        if (ok) {
-            const double m = max_abs9(h), det = det3d(h);
-            ok = fabs(det) > 1e-12 * m * m * m;
-            if (ok) inv3d(h, det, r);
-        }
-        if (!ok) for (int i = 0; i < 9; ++i) r[i] = (i % 4 == 0) ? 1.0 : 0.0;
+        double r[9];
+        const bool ok = nm_chain_step(H + (long long)p * 9, status == nullptr || status[(long long)p * 3] != 0, r);
         for (int i = 0; i < 9; ++i) G[(long long)(p + 1) * 9 + i] = r[i];
         flags[p + 1] = ok ? 0 : 1;
     }
@@ -350,7 +308,7 @@ __global__ void __launch_bounds__(kPlaceThreads) place_kernel(const float* __res
                     for (int r = 0; r < 3; ++r)
                         for (int c = 0; c < 3; ++c) nx[r * 3 + c] = g[r * 3] * s[c] + g[r * 3 + 1] * s[3 + c] + g[r * 3 + 2] * s[6 + c];
                 }
-                renormalise(nx);
+                nm_renormalise(nx);
                 for (int i = 0; i < 9; ++i) g[i] = s_g[k][i] = nx[i];
             }
         }
@@ -405,14 +363,14 @@ __global__ void __launch_bounds__(kPlaceThreads) place_kernel(const float* __res
         rects[k] = r;
         double a[9], gi[9], m[9];
         for (int i = 0; i < 9; ++i) a[i] = G[(long long)k * 9 + i];
-        inv3d(a, det3d(a), gi);
+        nm_inv3d(a, nm_det3d(a), gi);
         const double sx = (double)r.x + ox, sy = (double)r.y + oy;
         for (int row = 0; row < 3; ++row) {
             m[row * 3] = gi[row * 3];
             m[row * 3 + 1] = gi[row * 3 + 1];
             m[row * 3 + 2] = gi[row * 3] * sx + gi[row * 3 + 1] * sy + gi[row * 3 + 2];
         }
-        renormalise(m);
+        nm_renormalise(m);
         for (int i = 0; i < 9; ++i) mats[(long long)k * 9 + i] = (float)m[i];
     }
 }

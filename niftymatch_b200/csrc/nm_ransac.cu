@@ -31,7 +31,7 @@
 //  * nm_ransac_hypotheses_f32 takes the caller's index list: that is the entry the parity tests drive with
 //    the list they also hand to the reference's own kernels (homographies and inlier counts are bitwise the
 //    reference's on the same lists, tests/test_gpu_ransac.py).
-#include "nm_common.cuh"
+#include "nm_chain.cuh"
 
 namespace {
 
@@ -242,21 +242,24 @@ __global__ void align_kernel(const float* __restrict__ src_x, const float* __res
     c_dst_y[i] = ok ? dst_y[m] : -1.f;
 }
 
-// align_points for the consecutive pairs of a SIFT batch: pair p = (frame p, frame p + 1), sizes on the device
+// align_points for the links of a SIFT batch in the span layout (nm_span_links): link l = (frame t, frame t + d), sizes
+// on the device; span 1 = the consecutive pairs
 __global__ void align_pairs_kernel(const float* __restrict__ x, const float* __restrict__ y, const int* __restrict__ matches,
-                                   const int* __restrict__ counts, int capacity, float* __restrict__ c_src_x,
+                                   const int* __restrict__ counts, int n_frames, int capacity, float* __restrict__ c_src_x,
                                    float* __restrict__ c_src_y, float* __restrict__ c_dst_x, float* __restrict__ c_dst_y)
 {
-    const int i = blockIdx.x * blockDim.x + threadIdx.x, p = blockIdx.y;
+    const int i = blockIdx.x * blockDim.x + threadIdx.x, l = blockIdx.y;
     if (i >= capacity) return;
-    const long long o = (long long)p * capacity + i;
-    const int nA = min(counts[p], capacity), nB = min(counts[p + 1], capacity);
+    int t, d;
+    nm_link_decode(l, n_frames, t, d);
+    const long long o = (long long)l * capacity + i, a = (long long)t * capacity + i;
+    const int nA = min(counts[t], capacity), nB = min(counts[t + d], capacity);
     const int m = i < nA ? matches[o] : -1;
     const bool ok = m >= 0 && m < nB;
-    c_src_x[o] = ok ? x[o] : -1.f;
-    c_src_y[o] = ok ? y[o] : -1.f;
-    c_dst_x[o] = ok ? x[o + capacity - i + m] : -1.f;
-    c_dst_y[o] = ok ? y[o + capacity - i + m] : -1.f;
+    c_src_x[o] = ok ? x[a] : -1.f;
+    c_src_y[o] = ok ? y[a] : -1.f;
+    c_dst_x[o] = ok ? x[a + (long long)d * capacity - i + m] : -1.f;
+    c_dst_y[o] = ok ? y[a + (long long)d * capacity - i + m] : -1.f;
 }
 
 // ---- batched estimator: every kernel indexes a PAIR of frames by a grid dimension ------------------------
@@ -921,6 +924,536 @@ __global__ void __launch_bounds__(kRefineThreads, 1) refine_kernel(const Pairs P
     }
 }
 
+// ---- joint adjustment of a window's chain (nm_ransac_adjust_chain_f32; no reference counterpart) -------------------
+// Unknowns: G_k, frame k -> frame-0 pixels, k = 1 .. n-1, G_0 = I.  G_k = N^-1 Gn_k N with N = the frame centred and
+// scaled by 2 / max(w, h); Gn_k has P = 2 / 4 / 8 parameters (translation / similarity / homography with Gn[8] = 1).
+// Every sum below is fp64 and is formed in a fixed order, so a window's result is bit-reproducible.
+constexpr int kAdjMaxFrames = 1024, kAdjMaxSpan = 8;
+constexpr int kAdjSlices = 4;               // CTAs per link in the normal-equation build
+constexpr int kAdjThreads = 128;            // threads of a build CTA = correspondences staged per pass
+constexpr int kAdjSolveThreads = 256;
+
+template <int KIND> struct AdjFam {
+    static constexpr int P = KIND == 0 ? 2 : KIND == 1 ? 4 : 8;
+    static constexpr int M = KIND == 0 ? 1 : KIND == 1 ? 2 : 4;       // mask points a link needs
+    static constexpr int E = 3 * P * P + 2 * P + 1;                     // J^T J blocks (t,t), (u,u), (t,u), J^T r of t, u, cost
+    static constexpr int W = 2 + 4 * P;                                 // staged per point: r, dpi_t (2 x P), dpi_u (2 x P)
+};
+
+struct AdjState {
+    double lambda, cost, cost0;             // lambda < 0: not initialised yet
+    int first, done, accepted, pad;
+};
+
+struct AdjGeom {
+    double cx, cy, s;                       // normalised point = (p - c) * s
+    __device__ double2 norm(float x, float y) const { return make_double2(((double)x - cx) * s, ((double)y - cy) * s); }
+};
+
+__device__ __forceinline__ int adj_link(int t, int d, int n) { return (d - 1) * n - (d - 1) * d / 2 + t; }
+
+template <int KIND>
+__device__ void adj_identity(double* th)
+{
+    for (int i = 0; i < AdjFam<KIND>::P; ++i) th[i] = 0.0;
+    if (KIND == 1) th[0] = 1.0;
+    if (KIND == 2) th[0] = th[4] = 1.0;
+}
+
+template <int KIND>
+__device__ void adj_matrix(const double* th, double* G)
+{
+    if (KIND == 0) {
+        const double g[9] = {1.0, 0.0, th[0], 0.0, 1.0, th[1], 0.0, 0.0, 1.0};
+        for (int i = 0; i < 9; ++i) G[i] = g[i];
+    } else if (KIND == 1) {
+        const double g[9] = {th[0], -th[1], th[2], th[1], th[0], th[3], 0.0, 0.0, 1.0};
+        for (int i = 0; i < 9; ++i) G[i] = g[i];
+    } else {
+        for (int i = 0; i < 8; ++i) G[i] = th[i];
+        G[8] = 1.0;
+    }
+}
+
+// parameters of a normalised matrix, divided by its [8] first
+template <int KIND>
+__device__ void adj_params(const double* G, double* th)
+{
+    const double w = G[8];
+    if (KIND == 0) { th[0] = G[2] / w; th[1] = G[5] / w; }
+    else if (KIND == 1) { th[0] = G[0] / w; th[1] = G[3] / w; th[2] = G[2] / w; th[3] = G[5] / w; }
+    else for (int i = 0; i < 8; ++i) th[i] = G[i] / w;
+}
+
+// N G N^-1 (to = 1) or N^-1 G N (to = 0)
+__device__ void adj_conj(const AdjGeom& g, const double* G, double* R, bool to)
+{
+    const double s = to ? g.s : 1.0 / g.s, cx = to ? g.cx : -g.cx * g.s, cy = to ? g.cy : -g.cy * g.s;
+    // N = [s 0 -s cx; 0 s -s cy; 0 0 1] and N^-1 = [1/s 0 cx; 0 1/s cy; 0 0 1] are both S'(x) = s' (x - c')
+    double T[9];                                     // T = G . S'^-1, S'^-1 x = x / s' + c'
+    for (int r = 0; r < 3; ++r) {
+        T[r * 3 + 0] = G[r * 3 + 0] / s;
+        T[r * 3 + 1] = G[r * 3 + 1] / s;
+        T[r * 3 + 2] = G[r * 3 + 0] * cx + G[r * 3 + 1] * cy + G[r * 3 + 2];
+    }
+    for (int c = 0; c < 3; ++c) {                    // R = S' . T, S' x = s' (x - c')
+        R[c] = s * (T[c] - cx * T[6 + c]);
+        R[3 + c] = s * (T[3 + c] - cy * T[6 + c]);
+        R[6 + c] = T[6 + c];
+    }
+}
+
+// pi(Gn(th) p) and its derivatives du, dv with respect to th
+template <int KIND>
+__device__ __forceinline__ void adj_project(const double* th, double px, double py, double& U, double& V, double* du, double* dv)
+{
+    if (KIND == 0) {
+        U = px + th[0]; V = py + th[1];
+        du[0] = 1.0; du[1] = 0.0; dv[0] = 0.0; dv[1] = 1.0;
+    } else if (KIND == 1) {
+        U = th[0] * px - th[1] * py + th[2];
+        V = th[1] * px + th[0] * py + th[3];
+        du[0] = px; du[1] = -py; du[2] = 1.0; du[3] = 0.0;
+        dv[0] = py; dv[1] = px; dv[2] = 0.0; dv[3] = 1.0;
+    } else {
+        const double iw = 1.0 / (th[6] * px + th[7] * py + 1.0);
+        U = (th[0] * px + th[1] * py + th[2]) * iw;
+        V = (th[3] * px + th[4] * py + th[5]) * iw;
+        const double a = px * iw, b = py * iw;
+        du[0] = a; du[1] = b; du[2] = iw; du[3] = 0.0; du[4] = 0.0; du[5] = 0.0; du[6] = -U * a; du[7] = -U * b;
+        dv[0] = 0.0; dv[1] = 0.0; dv[2] = 0.0; dv[3] = a; dv[4] = b; dv[5] = iw; dv[6] = -V * a; dv[7] = -V * b;
+    }
+}
+
+// mask points of every link (i < n(l), mask byte != 0)
+__global__ void __launch_bounds__(256) adjust_count_kernel(const Pairs P, const unsigned char* __restrict__ masks, int* __restrict__ npts)
+{
+    __shared__ int tot;
+    const int l = blockIdx.x, n = pair_n(P, l);
+    if (threadIdx.x == 0) tot = 0;
+    __syncthreads();
+    int c = 0;
+    for (int i = threadIdx.x; i < n; i += 256) c += masks[(long long)l * P.max_pts + i] != 0;
+    atomicAdd(&tot, c);                                      // integer: the total does not depend on the order
+    __syncthreads();
+    if (threadIdx.x == 0) npts[l] = tot;
+}
+
+// One CTA.  Initial poses: for k = 1 .. n-1 the smallest d <= span with frame k-d connected and link (k-d, d) usable
+// (status 1, at least M mask points) gives G_k = G_(k-d) . step(H_link) (nm_chain_step, renormalised: place_kernel's
+// chain); without one frame k is disconnected and G_k = G_(k-1).  Then the parameters of N G_k N^-1, the links used,
+// and the LM state.
+template <int KIND>
+__global__ void __launch_bounds__(256) adjust_init_kernel(int n, int span, AdjGeom geo, const float* __restrict__ H_links,
+                                                          const int* __restrict__ link_status, const int* __restrict__ npts,
+                                                          double* __restrict__ G, int* __restrict__ conn, int* __restrict__ used,
+                                                          double* __restrict__ x_cur, double* __restrict__ x_eval, AdjState* state)
+{
+    constexpr int NP = AdjFam<KIND>::P, M = AdjFam<KIND>::M;
+    const int tid = threadIdx.x, L = nm_span_links(n, span);
+    auto usable = [&](int l) { return link_status[(long long)l * 3] == 1 && npts[l] >= M; };
+    if (tid == 0) {
+        for (int i = 0; i < 9; ++i) G[i] = (i % 4 == 0) ? 1.0 : 0.0;
+        conn[0] = 1;
+        for (int k = 1; k < n; ++k) {
+            int found = 0;
+            for (int d = 1; d <= span && d <= k && !found; ++d) {
+                const int l = adj_link(k - d, d, n);
+                if (!conn[k - d] || !usable(l)) continue;
+                double r[9], g[9];
+                nm_chain_step(H_links + (long long)l * 9, true, r);
+                const double* a = G + (long long)(k - d) * 9;
+                for (int row = 0; row < 3; ++row)
+                    for (int c = 0; c < 3; ++c) g[row * 3 + c] = a[row * 3] * r[c] + a[row * 3 + 1] * r[3 + c] + a[row * 3 + 2] * r[6 + c];
+                nm_renormalise(g);
+                for (int i = 0; i < 9; ++i) G[(long long)k * 9 + i] = g[i];
+                found = 1;
+            }
+            if (!found)
+                for (int i = 0; i < 9; ++i) G[(long long)k * 9 + i] = G[(long long)(k - 1) * 9 + i];
+            conn[k] = found;
+        }
+        AdjState st;
+        st.lambda = -1.0; st.cost = st.cost0 = 0.0;
+        st.first = 1; st.done = 0; st.accepted = 0; st.pad = 0;
+        *state = st;
+    }
+    __syncthreads();
+    for (int k = tid; k < n; k += 256) {
+        double th[NP];
+        if (k == 0) adj_identity<KIND>(th);
+        else {
+            double Gn[9];
+            adj_conj(geo, G + (long long)k * 9, Gn, true);
+            adj_params<KIND>(Gn, th);
+        }
+        for (int i = 0; i < NP; ++i) x_cur[k * NP + i] = x_eval[k * NP + i] = th[i];
+    }
+    for (int l = tid; l < L; l += 256) {
+        int t, d;
+        nm_link_decode(l, n, t, d);
+        used[l] = conn[t] && conn[t + d] && usable(l);
+    }
+}
+
+// One CTA per (link, slice): the slice's share of the link's J^T J blocks, J^T r and cost at x_eval.  A pass stages
+// kAdjThreads correspondences (residual and projection derivatives) in shared memory; thread e then adds entry e of
+// every staged point in index order, so the sums have a fixed order.  Entry e is +/-(a1 b1 + a2 b2) of staged values.
+template <int KIND>
+__global__ void __launch_bounds__(kAdjThreads) adjust_build_kernel(const Pairs P, const unsigned char* __restrict__ masks, int n,
+                                                                   AdjGeom geo, const int* __restrict__ used,
+                                                                   const double* __restrict__ x_eval, const AdjState* __restrict__ state,
+                                                                   double* __restrict__ partial)
+{
+    constexpr int NP = AdjFam<KIND>::P, E = AdjFam<KIND>::E, W = AdjFam<KIND>::W;
+    constexpr int NE = (E + kAdjThreads - 1) / kAdjThreads;
+    __shared__ double sp[kAdjThreads * W];
+    __shared__ unsigned char sv[kAdjThreads];
+    const int l = blockIdx.x, slice = blockIdx.y, tid = threadIdx.x;
+    if (state->done || !used[l]) return;
+    int t, d;
+    nm_link_decode(l, n, t, d);
+    double tht[NP], thu[NP];
+    for (int i = 0; i < NP; ++i) { tht[i] = x_eval[t * NP + i]; thu[i] = x_eval[(t + d) * NP + i]; }
+    // entries owned by this thread: (a1, b1, a2, b2, negate)
+    int ea[NE][4];
+    bool neg[NE];
+    for (int r = 0; r < NE; ++r) {
+        const int e = tid + r * kAdjThreads;
+        int a1 = 0, b1 = 0, a2 = 1, b2 = 1;
+        bool ng = false;
+        const int ot = 2, ovt = 2 + NP, ou = 2 + 2 * NP, ovu = 2 + 3 * NP;    // du_t, dv_t, du_u, dv_u
+        if (e < NP * NP) { const int i = e / NP, j = e % NP; a1 = ot + i; b1 = ot + j; a2 = ovt + i; b2 = ovt + j; }
+        else if (e < 2 * NP * NP) { const int i = (e - NP * NP) / NP, j = e % NP; a1 = ou + i; b1 = ou + j; a2 = ovu + i; b2 = ovu + j; }
+        else if (e < 3 * NP * NP) { const int i = (e - 2 * NP * NP) / NP, j = e % NP; a1 = ot + i; b1 = ou + j; a2 = ovt + i; b2 = ovu + j; ng = true; }
+        else if (e < 3 * NP * NP + NP) { const int i = e - 3 * NP * NP; a1 = ot + i; b1 = 0; a2 = ovt + i; b2 = 1; }
+        else if (e < 3 * NP * NP + 2 * NP) { const int i = e - 3 * NP * NP - NP; a1 = ou + i; b1 = 0; a2 = ovu + i; b2 = 1; ng = true; }
+        ea[r][0] = a1; ea[r][1] = b1; ea[r][2] = a2; ea[r][3] = b2;
+        neg[r] = ng;
+    }
+    double acc[NE];
+    for (int r = 0; r < NE; ++r) acc[r] = 0.0;
+    const int cnt = pair_n(P, l), len = (cnt + kAdjSlices - 1) / kAdjSlices;
+    const int lo = slice * len, hi = min(cnt, lo + len);
+    const long long off = (long long)l * P.stride;
+    const unsigned char* __restrict__ mask = masks + (long long)l * P.max_pts;
+    for (int base = lo; base < hi; base += kAdjThreads) {
+        const int i = base + tid;
+        const bool ok = i < hi && mask[i] != 0;
+        if (ok) {
+            double* q = sp + tid * W;
+            const double2 a = geo.norm(P.sx[off + i], P.sy[off + i]), b = geo.norm(P.dx[off + i], P.dy[off + i]);
+            double Ut, Vt, Uu, Vu;
+            adj_project<KIND>(tht, a.x, a.y, Ut, Vt, q + 2, q + 2 + NP);
+            adj_project<KIND>(thu, b.x, b.y, Uu, Vu, q + 2 + 2 * NP, q + 2 + 3 * NP);
+            q[0] = Ut - Uu;
+            q[1] = Vt - Vu;
+        }
+        sv[tid] = ok;
+        __syncthreads();
+        const int np = min(kAdjThreads, hi - base);
+        for (int k = 0; k < np; ++k) {
+            if (!sv[k]) continue;
+            const double* q = sp + k * W;
+#pragma unroll
+            for (int r = 0; r < NE; ++r) acc[r] += q[ea[r][0]] * q[ea[r][1]] + q[ea[r][2]] * q[ea[r][3]];
+        }
+        __syncthreads();
+    }
+    for (int r = 0; r < NE; ++r) {
+        const int e = tid + r * kAdjThreads;
+        if (e < E) partial[((long long)l * kAdjSlices + slice) * E + e] = neg[r] ? -acc[r] : acc[r];
+    }
+}
+
+// One CTA: the Levenberg-Marquardt step.  Link totals (slices in order), the cost at x_eval (links in index order);
+// x_eval is accepted when it is the first point or lowers the cost (lambda / 10), else rejected (lambda * 10).  After an
+// acceptance the banded normal equations of the unknowns (frame-major, half-bandwidth bw = P (span + 1) - 1; a
+// disconnected frame's rows are the identity with zero right-hand side) are assembled in link index order.  Unless the
+// run is over, (J^T J + lambda I) delta = -J^T r is solved by a banded Cholesky factorisation -- the last bw + 1 rows of
+// the factor kept in shared memory, the forward substitution folded into it, the back substitution by warp 0 -- and
+// x_eval = x_cur + delta.  A failed factorisation counts as a rejection.
+template <int KIND>
+__global__ void __launch_bounds__(kAdjSolveThreads) adjust_solve_kernel(int n, int span, const int* __restrict__ used,
+                                                                        const int* __restrict__ conn, const double* __restrict__ partial,
+                                                                        double* __restrict__ link_tot, double* __restrict__ A,
+                                                                        double* __restrict__ rhs, double* __restrict__ U,
+                                                                        double* __restrict__ x_cur, double* __restrict__ x_eval,
+                                                                        AdjState* state, int last)
+{
+    constexpr int NP = AdjFam<KIND>::P, E = AdjFam<KIND>::E;
+    extern __shared__ double sm[];
+    __shared__ int s_accept, s_stop, s_fail;
+    const int tid = threadIdx.x, L = nm_span_links(n, span), m = (n - 1) * NP, bw = NP * (span + 1) - 1, bw1 = bw + 1;
+    double* W = sm;                                          // [bw1][bw1] rows of the factor, row k at slot k % bw1
+    double* tmp = W + bw1 * bw1;                             // [bw1 + 1]
+    double* y = tmp + bw1 + 1;                               // [m] forward, then back substitution
+    if (state->done) return;
+    for (int idx = tid; idx < L * E; idx += kAdjSolveThreads) {
+        const int l = idx / E, e = idx - l * E;
+        if (!used[l]) continue;
+        const double* q = partial + (long long)l * kAdjSlices * E + e;
+        double s = q[0];
+        for (int sl = 1; sl < kAdjSlices; ++sl) s += q[sl * E];
+        link_tot[idx] = s;
+    }
+    __syncthreads();
+    if (tid == 0) {
+        double c = 0.0;
+        for (int l = 0; l < L; ++l)
+            if (used[l]) c += link_tot[(long long)l * E + E - 1];
+        AdjState st = *state;
+        bool accept = false;
+        if (st.first) { accept = true; st.cost0 = c; st.first = 0; }
+        else if (c < st.cost) {
+            accept = true;
+            if (st.cost - c < 1e-12 * st.cost) st.done = 1;
+            st.lambda *= 0.1;
+            ++st.accepted;
+        } else {
+            st.lambda *= 10.0;
+            if (st.lambda > 1e16) st.done = 1;
+        }
+        if (accept) st.cost = c;
+        *state = st;
+        s_accept = accept;
+        s_stop = st.done || last;
+    }
+    __syncthreads();
+    const bool accept = s_accept;
+    if (accept)
+        for (int i = tid; i < n * NP; i += kAdjSolveThreads) x_cur[i] = x_eval[i];
+    if (s_stop) return;
+    if (accept) {
+        for (long long idx = tid; idx < (long long)m * bw1; idx += kAdjSolveThreads) {
+            const int i = (int)(idx / bw1), c = (int)(idx - (long long)i * bw1), j = i + c;
+            double v = 0.0;
+            if (j < m) {
+                const int k = i / NP + 1, a = i % NP, k2 = j / NP + 1, b = j % NP, dd = k2 - k;
+                if (!conn[k] || !conn[k2]) v = c == 0 ? 1.0 : 0.0;
+                else if (dd == 0) {
+                    for (int d = 1; d <= span; ++d) {
+                        if (k - d >= 0) { const int l = adj_link(k - d, d, n); if (used[l]) v += link_tot[(long long)l * E + NP * NP + a * NP + b]; }
+                        if (k + d < n) { const int l = adj_link(k, d, n); if (used[l]) v += link_tot[(long long)l * E + a * NP + b]; }
+                    }
+                } else if (dd <= span) {
+                    const int l = adj_link(k, dd, n);
+                    if (used[l]) v = link_tot[(long long)l * E + 2 * NP * NP + a * NP + b];
+                }
+            }
+            A[idx] = v;
+        }
+        for (int i = tid; i < m; i += kAdjSolveThreads) {
+            const int k = i / NP + 1, a = i % NP;
+            double v = 0.0;
+            if (conn[k])
+                for (int d = 1; d <= span; ++d) {
+                    if (k - d >= 0) { const int l = adj_link(k - d, d, n); if (used[l]) v += link_tot[(long long)l * E + 3 * NP * NP + NP + a]; }
+                    if (k + d < n) { const int l = adj_link(k, d, n); if (used[l]) v += link_tot[(long long)l * E + 3 * NP * NP + a]; }
+                }
+            rhs[i] = v;
+        }
+        __syncthreads();
+        if (tid == 0 && state->lambda < 0.0) {
+            double mx = 0.0;
+            for (int i = 0; i < m; ++i)
+                if (conn[i / NP + 1]) mx = fmax(mx, A[(long long)i * bw1]);
+            state->lambda = mx > 0.0 ? 1e-3 * mx : 1e-3;
+        }
+        __syncthreads();
+    }
+    for (;;) {
+        const double lambda = state->lambda;
+        bool fail = false;
+        for (int j = 0; j < m && !fail; ++j) {
+            if (tid <= bw) {
+                const int i = j + tid;
+                if (i < m) {
+                    double s = A[(long long)j * bw1 + tid] + (tid == 0 ? lambda : 0.0);
+                    const int k0 = max(0, i - bw);
+                    int slot = k0 % bw1;
+                    for (int k = k0; k < j; ++k) {
+                        s -= W[slot * bw1 + (j - k)] * W[slot * bw1 + (i - k)];
+                        slot = slot + 1 == bw1 ? 0 : slot + 1;
+                    }
+                    tmp[tid] = s;
+                }
+            } else if (tid == bw1) {
+                double s = -rhs[j];
+                const int k0 = max(0, j - bw);
+                int slot = k0 % bw1;
+                for (int k = k0; k < j; ++k) {
+                    s -= W[slot * bw1 + (j - k)] * y[k];
+                    slot = slot + 1 == bw1 ? 0 : slot + 1;
+                }
+                tmp[bw1] = s;
+            }
+            __syncthreads();
+            const double dj = tmp[0];
+            fail = !(dj > 0.0) || !isfinite(dj);
+            if (!fail) {
+                const double r = sqrt(dj);
+                if (tid <= bw && j + tid < m) {
+                    const double v = tid == 0 ? r : tmp[tid] / r;
+                    W[(j % bw1) * bw1 + tid] = v;
+                    U[(long long)j * bw1 + tid] = v;
+                } else if (tid == bw1) y[j] = tmp[bw1] / r;
+            }
+            __syncthreads();
+        }
+        if (!fail && tid < 32) {
+            // back substitution U delta = y, in place; lane c handles the columns i + 1 + c + 32 q
+            for (int i = m - 1; i >= 0; --i) {
+                double s = 0.0;
+                for (int c = 1 + tid; c <= bw && i + c < m; c += 32) s += U[(long long)i * bw1 + c] * y[i + c];
+#pragma unroll
+                for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
+                const double v = (y[i] - s) / U[(long long)i * bw1];
+                __syncwarp();
+                if (tid == 0) y[i] = v;
+                __syncwarp();
+                if (!isfinite(v)) fail = true;
+            }
+            if (tid == 0) s_fail = fail;
+        } else if (tid == 0) s_fail = fail;
+        __syncthreads();
+        fail = s_fail;
+        if (!fail) {
+            for (int i = tid; i < n * NP; i += kAdjSolveThreads) {
+                const int k = i / NP;
+                x_eval[i] = (k == 0 || !conn[k]) ? x_cur[i] : x_cur[i] + y[i - NP];
+            }
+            return;
+        }
+        if (tid == 0) {
+            state->lambda *= 10.0;
+            if (state->lambda > 1e16) state->done = 1;
+        }
+        __syncthreads();
+        if (state->done) return;
+    }
+}
+
+// One CTA per pair p: H_out[p] = G_(p+1)^-1 G_p rounded to float (divided by its [8]) and status {1, inliers of it on link
+// (p, 1), LM steps accepted} when frame p + 1 is connected; H_in[p] and {0, 0, 0} otherwise (nm_mosaic_place_f32 then
+// keeps frame p + 1 at G_p).  chain_out[p + 1] (and [0] by CTA 0) = G; CTA 0 writes the report.
+template <int KIND>
+__global__ void __launch_bounds__(256) adjust_finish_kernel(const Pairs P, float thr, int n, int span, AdjGeom geo,
+                                                            const float* H_in, const int* __restrict__ conn,
+                                                            const int* __restrict__ used, const int* __restrict__ npts,
+                                                            const double* __restrict__ x_cur, const AdjState* __restrict__ state,
+                                                            float* H_out, int* status_out, double* __restrict__ chain_out,
+                                                            double* __restrict__ report)
+{
+    constexpr int NP = AdjFam<KIND>::P;
+    __shared__ float Hs[9];
+    __shared__ int s_cnt;
+    const int p = blockIdx.x, k = p + 1, tid = threadIdx.x;
+    if (tid == 0) {
+        // a disconnected frame sits at the adjusted pose of its nearest connected predecessor
+        int ep = p, ek = k;
+        while (!conn[ep]) --ep;
+        if (!conn[ek]) ek = ep;
+        double thp[NP], thk[NP], Gp[9], Gk[9], Gki[9], Mn[9], M[9];
+        for (int i = 0; i < NP; ++i) { thp[i] = x_cur[ep * NP + i]; thk[i] = x_cur[ek * NP + i]; }
+        adj_matrix<KIND>(thp, Gp);
+        adj_matrix<KIND>(thk, Gk);
+        if (chain_out) {
+            double C[9];
+            adj_conj(geo, Gk, C, false);
+            for (int i = 0; i < 9; ++i) chain_out[(long long)k * 9 + i] = C[i];
+            if (p == 0) for (int i = 0; i < 9; ++i) chain_out[i] = (i % 4 == 0) ? 1.0 : 0.0;
+        }
+        nm_inv3d(Gk, nm_det3d(Gk), Gki);
+        for (int r = 0; r < 3; ++r)
+            for (int c = 0; c < 3; ++c) Mn[r * 3 + c] = Gki[r * 3] * Gp[c] + Gki[r * 3 + 1] * Gp[3 + c] + Gki[r * 3 + 2] * Gp[6 + c];
+        adj_conj(geo, Mn, M, false);
+        for (int i = 0; i < 9; ++i) Hs[i] = conn[k] ? (float)(M[i] / M[8]) : H_in[(long long)p * 9 + i];
+        s_cnt = 0;
+        if (p == 0 && report) {
+            long long pts = 0;
+            int links = 0;
+            for (int l = 0; l < nm_span_links(n, span); ++l)
+                if (used[l]) { pts += npts[l]; ++links; }
+            const double scale = 1.0 / (geo.s * geo.s * (double)(pts > 0 ? pts : 1));
+            report[0] = state->cost0 * scale;
+            report[1] = state->cost * scale;
+            report[2] = (double)pts;
+            report[3] = (double)links;
+        }
+    }
+    __syncthreads();
+    if (!conn[k]) {
+        if (tid < 9) H_out[(long long)p * 9 + tid] = Hs[tid];
+        if (tid == 0) status_out[p * 3] = status_out[p * 3 + 1] = status_out[p * 3 + 2] = 0;
+        return;
+    }
+    float H[9];
+    for (int i = 0; i < 9; ++i) H[i] = Hs[i];
+    const int cnt = pair_n(P, p);
+    const long long off = (long long)p * P.stride;
+    int c = 0;
+    for (int i = tid; i < cnt; i += 256) c += transfer_inlier(H, make_float4(P.sx[off + i], P.sy[off + i], P.dx[off + i], P.dy[off + i]), thr);
+    atomicAdd(&s_cnt, c);
+    __syncthreads();
+    if (tid < 9) H_out[(long long)p * 9 + tid] = H[tid];
+    if (tid == 0) {
+        status_out[p * 3] = 1;
+        status_out[p * 3 + 1] = s_cnt;
+        status_out[p * 3 + 2] = state->accepted;
+    }
+}
+
+template <int KIND>
+int adjust_chain(const Pairs& P, float thr, int n, int span, int fw, int fh, const unsigned char* masks, const float* H_links,
+                 const int* link_status, int iterations, float* H_out, int* status_out, double* chain_out, double* report,
+                 cudaStream_t st)
+{
+    constexpr int NP = AdjFam<KIND>::P, E = AdjFam<KIND>::E;
+    const int L = nm_span_links(n, span), m = (n - 1) * NP, bw1 = NP * (span + 1);
+    const size_t smem = sizeof(double) * ((size_t)bw1 * bw1 + bw1 + 1 + m);
+    static NmDeviceOnce once;
+    if (once.first()) {
+        NM_CUDA_TRY(cudaFuncSetAttribute(adjust_solve_kernel<KIND>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                         (int)(sizeof(double) * ((size_t)(8 * (kAdjMaxSpan + 1)) * (8 * (kAdjMaxSpan + 1)) +
+                                                                 8 * (kAdjMaxSpan + 1) + 1 + (kAdjMaxFrames - 1) * 8))));
+        once.done();
+    }
+    // one stream-ordered block: state | G | x_cur | x_eval | partial | link_tot | A | U | rhs (doubles), conn | used | npts
+    const size_t nd = 8 + 9 * (size_t)n + 2 * (size_t)n * NP + (size_t)L * kAdjSlices * E + (size_t)L * E +
+                      2 * (size_t)m * bw1 + (size_t)m;
+    const size_t total = sizeof(double) * nd + sizeof(int) * ((size_t)n + 2 * (size_t)L);
+    char* ws = nullptr;
+    NM_CUDA_TRY(nm_ws_alloc(&ws, total, st));
+    double* d = reinterpret_cast<double*>(ws);
+    AdjState* state = reinterpret_cast<AdjState*>(d);
+    double* G = d + 8;
+    double* x_cur = G + 9 * (size_t)n;
+    double* x_eval = x_cur + (size_t)n * NP;
+    double* partial = x_eval + (size_t)n * NP;
+    double* link_tot = partial + (size_t)L * kAdjSlices * E;
+    double* A = link_tot + (size_t)L * E;
+    double* U = A + (size_t)m * bw1;
+    double* rhs = U + (size_t)m * bw1;
+    int* conn = reinterpret_cast<int*>(rhs + m);
+    int* used = conn + n;
+    int* npts = used + L;
+    const double ext = (double)(fw > fh ? fw : fh);
+    const AdjGeom geo{0.5 * (fw - 1), 0.5 * (fh - 1), 2.0 / ext};
+    adjust_count_kernel<<<L, 256, 0, st>>>(P, masks, npts);
+    adjust_init_kernel<KIND><<<1, 256, 0, st>>>(n, span, geo, H_links, link_status, npts, G, conn, used, x_cur, x_eval, state);
+    for (int it = 0; it < iterations; ++it) {
+        adjust_build_kernel<KIND><<<dim3(L, kAdjSlices), kAdjThreads, 0, st>>>(P, masks, n, geo, used, x_eval, state, partial);
+        adjust_solve_kernel<KIND><<<1, kAdjSolveThreads, smem, st>>>(n, span, used, conn, partial, link_tot, A, rhs, U, x_cur, x_eval,
+                                                                     state, it == iterations - 1);
+    }
+    adjust_finish_kernel<KIND><<<n - 1, 256, 0, st>>>(P, thr, n, span, geo, H_links, conn, used, npts, x_cur, state, H_out, status_out,
+                                                      chain_out, report);
+    const cudaError_t e = cudaGetLastError();
+    const cudaError_t f = cudaFreeAsync(ws, st);
+    return nm_cuda_err(e != cudaSuccess ? e : f);
+}
+
 int min_points(int kind) { return kind == 2 ? 4 : 2; }        // ransac.cu:541, :606, :656 (translation also asks for 2)
 int sample_size(int kind) { return kind == 0 ? 1 : kind == 1 ? 2 : 4; }
 
@@ -985,16 +1518,24 @@ extern "C" int nm_align_points_f32(const float* src_x, const float* src_y, const
     return NM_OK;
 }
 
+extern "C" int nm_align_pairs_span_f32(const float* x, const float* y, const int* matches, const int* counts_dev, int n_frames,
+                                       int capacity, int span, float* c_src_x, float* c_src_y, float* c_dst_x, float* c_dst_y,
+                                       nm_stream_t stream)
+{
+    if (!x || !y || !matches || !counts_dev || !c_src_x || !c_src_y || !c_dst_x || !c_dst_y || n_frames < 2 || capacity <= 0)
+        return NM_ERR_INVALID;
+    if (span < 1 || span > 8 || span > n_frames - 1 || nm_span_links(n_frames, span) > 65535) return NM_ERR_INVALID;
+    align_pairs_kernel<<<dim3(nm_div_up(capacity, 256), nm_span_links(n_frames, span)), 256, 0, (cudaStream_t)stream>>>(
+        x, y, matches, counts_dev, n_frames, capacity, c_src_x, c_src_y, c_dst_x, c_dst_y);
+    NM_LAUNCH_CHECK();
+    return NM_OK;
+}
+
 extern "C" int nm_align_pairs_f32(const float* x, const float* y, const int* matches, const int* counts_dev, int n_frames,
                                   int capacity, float* c_src_x, float* c_src_y, float* c_dst_x, float* c_dst_y,
                                   nm_stream_t stream)
 {
-    if (!x || !y || !matches || !counts_dev || !c_src_x || !c_src_y || !c_dst_x || !c_dst_y || n_frames < 2 || capacity <= 0)
-        return NM_ERR_INVALID;
-    align_pairs_kernel<<<dim3(nm_div_up(capacity, 256), n_frames - 1), 256, 0, (cudaStream_t)stream>>>(
-        x, y, matches, counts_dev, capacity, c_src_x, c_src_y, c_dst_x, c_dst_y);
-    NM_LAUNCH_CHECK();
-    return NM_OK;
+    return nm_align_pairs_span_f32(x, y, matches, counts_dev, n_frames, capacity, 1, c_src_x, c_src_y, c_dst_x, c_dst_y, stream);
 }
 
 extern "C" int nm_ransac_hypotheses_f32(int kind, const float* src_x, const float* src_y, const float* dst_x,
@@ -1046,4 +1587,25 @@ extern "C" int nm_ransac_refine_batch_f32(int kind, const float* src_x, const fl
     else refine_kernel<2><<<n_pairs, kRefineThreads, 0, st>>>(P, inlier_threshold, H_in, status_in, rounds, H_out, status_out, inlier_mask);
     NM_LAUNCH_CHECK();
     return NM_OK;
+}
+
+extern "C" int nm_ransac_adjust_chain_f32(int kind, const float* src_x, const float* src_y, const float* dst_x, const float* dst_y,
+                                          long long pair_stride, const int* counts, int max_pts, float inlier_threshold,
+                                          int n_frames, int span, int frame_w, int frame_h, const unsigned char* masks,
+                                          const float* H_links, const int* link_status, int iterations, float* H_out,
+                                          int* status_out, double* chain_out, double* report_out, nm_stream_t stream)
+{
+    if (kind < 0 || kind > 2 || max_pts <= 0 || pair_stride < 0 || iterations < 1 || frame_w <= 0 || frame_h <= 0) return NM_ERR_INVALID;
+    if (n_frames < 2 || n_frames > kAdjMaxFrames || span < 1 || span > kAdjMaxSpan || span >= n_frames) return NM_ERR_INVALID;
+    if (!src_x || !src_y || !dst_x || !dst_y || !masks || !H_links || !link_status || !H_out || !status_out) return NM_ERR_INVALID;
+    const Pairs P{src_x, src_y, dst_x, dst_y, pair_stride, counts, max_pts};
+    const cudaStream_t st = (cudaStream_t)stream;
+    if (kind == 0)
+        return adjust_chain<0>(P, inlier_threshold, n_frames, span, frame_w, frame_h, masks, H_links, link_status, iterations, H_out,
+                               status_out, chain_out, report_out, st);
+    if (kind == 1)
+        return adjust_chain<1>(P, inlier_threshold, n_frames, span, frame_w, frame_h, masks, H_links, link_status, iterations, H_out,
+                               status_out, chain_out, report_out, st);
+    return adjust_chain<2>(P, inlier_threshold, n_frames, span, frame_w, frame_h, masks, H_links, link_status, iterations, H_out,
+                           status_out, chain_out, report_out, st);
 }

@@ -128,16 +128,27 @@ class StreamRegistrar:
     leave the device and nothing synchronises; consecutive chunks share one frame (recomputed), so no state is carried
     between chunks or between GPUs.  Pair t -> t + 1 draws with seed + t: the result does not depend on the chunking or
     on how the stream is sharded over ranks (frame_range(..., overlap=1)).  refine_rounds > 0 refits each chunk's models
-    on their inliers in place (nm_ransac_refine_batch_f32) right after its RANSAC; status[:, 2] is then the refits kept."""
+    on their inliers in place (nm_ransac_refine_batch_f32) right after its RANSAC; status[:, 2] is then the refits kept.
+
+    span > 1 (at most 8) registers every frame t of a chunk also to t + 2 ... t + span and adjusts the chunk's poses
+    jointly: each chunk [c0, c1) is one adjustment window of the span layout (span min(span, c1 - c0 - 1)), run as
+    match_pairs_span, align_pairs_span, one ransac_batch per d (link (t, d), t in stream coordinates, draws with
+    seed + t + ((d - 1) << 40)), refine_batch on all links (rounds = refine_rounds, 0 = masks only) and adjust_chain, whose
+    pairwise models and status [connected, inliers, LM steps accepted] are returned (status[:, 2] counts LM steps here,
+    not refits kept; adjust_iterations bounds the LM builds per window).  A frame that no usable link reaches
+    keeps its predecessor's pose (status 0).  The result then depends on the window boundaries -- lo and the chunk
+    size -- and on nothing else.  span = 1 calls nothing new."""
 
     def __init__(self, sift_batch, chunk=None, kind: int = 2, ambiguity: float = 0.8, inlier_threshold: float = 4.0,
-                 iterations: int = 1024, seed: int = 0, refine_rounds: int = 0):
+                 iterations: int = 1024, seed: int = 0, refine_rounds: int = 0, span: int = 1, adjust_iterations: int = 10):
         import torch
         self.sb = sift_batch
         self.chunk = min(chunk or sift_batch.max_batch, sift_batch.max_batch)
         assert self.chunk >= 2 and sift_batch.capacity % 256 == 0
         self.kind, self.ambiguity, self.thr, self.iters, self.seed = kind, ambiguity, inlier_threshold, iterations, seed
         self.refine_rounds = refine_rounds
+        assert 1 <= span <= 8
+        self.span, self.adjust_iterations = span, adjust_iterations
         cap, n = sift_batch.capacity, self.chunk - 1
         dev = torch.device("cuda", torch.cuda.current_device())
         self.match = torch.empty((n, cap), dtype=torch.int32, device=dev)
@@ -171,12 +182,18 @@ class StreamRegistrar:
                 sb.run_bgra(chunk)
             else:
                 sb.run(chunk)
+            k = c0 - lo
+            if self.span > 1:
+                adjust_window(r, n, min(self.span, n - 1), chunk.shape[2], chunk.shape[1], self.kind, self.ambiguity, self.thr,
+                              self.iters, self.seed + c0, self.refine_rounds, out=(H[k: k + n - 1], st[k: k + n - 1]),
+                              adjust_iterations=self.adjust_iterations)
+                c0 = c1 - 1
+                continue
             self.match[: n - 1].fill_(-1)
             check(lib.nm_match_pairs_f32(p(r["desc"]), p(r["counts"]), n, cap, self.ambiguity, p(self.match), None, None,
                                          _stream_ptr()), "nm_match_pairs_f32")
             check(lib.nm_align_pairs_f32(p(r["x"]), p(r["y"]), p(self.match), p(r["counts"]), n, cap, *[p(c) for c in self.corr],
                                          _stream_ptr()), "nm_align_pairs_f32")
-            k = c0 - lo
             check(lib.nm_ransac_batch_f32(self.kind, *[p(c) for c in self.corr], cap, p(r["counts"]), cap, n - 1, self.thr,
                                           self.iters, (self.seed + c0) & 0xFFFFFFFFFFFFFFFF, p(H[k:]), p(st[k:]), _stream_ptr()),
                   "nm_ransac_batch_f32")
@@ -186,3 +203,26 @@ class StreamRegistrar:
                                                      None, _stream_ptr()), "nm_ransac_refine_batch_f32")
             c0 = c1 - 1
         return H[:n_pairs], st[:n_pairs]
+
+
+def adjust_window(res, n, span, frame_w, frame_h, kind, ambiguity, inlier_threshold, iterations, seed, refine_rounds, out,
+                  adjust_iterations: int = 10):
+    """One adjustment window of StreamRegistrar(span > 1): frames 0 .. n-1 of the SIFT results `res` (SiftBatch.results())
+    through the five public calls.  seed = the stream seed + the window's first frame.  Writes the window's n - 1 pairwise
+    models and status into out = (H, status); returns adjust_chain's (H, status, chain, report)."""
+    import torch
+    from .match import match_pairs_span, link_row
+    from .ransac import align_pairs_span, ransac_batch, refine_batch, adjust_chain
+    counts = res["counts"][:n]
+    m = match_pairs_span(res["desc"][:n], counts, span, ambiguity)
+    corr = align_pairs_span(res["x"][:n], res["y"][:n], m, counts, span)
+    HL, SL = [], []
+    for d in range(1, span + 1):
+        r0 = link_row(n, 0, d)
+        Hd, Sd = ransac_batch(kind, *[c[r0: r0 + n - d] for c in corr], counts[: n - d], inlier_threshold, iterations,
+                              seed + ((d - 1) << 40))
+        HL.append(Hd)
+        SL.append(Sd)
+    link_counts = torch.cat([counts[: n - d] for d in range(1, span + 1)])
+    HL, SL, mask = refine_batch(kind, *corr, link_counts, torch.cat(HL), torch.cat(SL), inlier_threshold, refine_rounds)
+    return adjust_chain(kind, *corr, link_counts, span, mask, HL, SL, frame_w, frame_h, inlier_threshold, adjust_iterations, out=out)

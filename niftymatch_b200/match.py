@@ -96,6 +96,37 @@ def match_pairs(desc, counts, ambiguity: float = 0.8, match_out=None, want_recor
     return (match_out, rec, fb) if want_records else match_out
 
 
+def span_links(n_frames: int, span: int) -> int:
+    """Rows of the span layout over n_frames frames: the links (t, t + d), 1 <= d <= span, d-major (include/nm_b200.h)."""
+    return span * n_frames - span * (span + 1) // 2
+
+
+def link_row(n_frames: int, t: int, d: int) -> int:
+    """Row of link (t, t + d) in the span layout."""
+    return (d - 1) * n_frames - (d - 1) * d // 2 + t
+
+
+def match_pairs_span(desc, counts, span, ambiguity: float = 0.8, match_out=None, want_records: bool = False):
+    """nm_match_pairs_span_f32: match_pairs for every link (t, t + d), d <= span, of the span layout.  Returns match
+    indices (span_links(n_frames, span), capacity) int32; row link_row(n, t, d) holds frame t's matches into frame t + d.
+    Span 1 is match_pairs.  No host synchronisation."""
+    import torch
+    assert desc.is_cuda and desc.dtype == torch.float32 and desc.is_contiguous() and desc.dim() == 3 and desc.shape[2] == 128
+    n_frames, cap = desc.shape[0], desc.shape[1]
+    _i32(counts, "counts", n_frames)
+    L = span_links(n_frames, span)
+    if match_out is None:
+        match_out = torch.full((max(L, 0), cap), -1, dtype=torch.int32, device=desc.device)
+    rec = torch.zeros((L, cap, 4), dtype=torch.float32, device=desc.device) if want_records else None
+    fb = torch.zeros(1, dtype=torch.int32, device=desc.device) if want_records else None
+    check(_lib.load().nm_match_pairs_span_f32(C.c_void_p(desc.data_ptr()), C.c_void_p(counts.data_ptr()), n_frames, cap, span,
+                                              ambiguity, C.c_void_p(match_out.data_ptr()),
+                                              C.c_void_p(rec.data_ptr()) if rec is not None else None,
+                                              C.c_void_p(fb.data_ptr()) if fb is not None else None, _stream_ptr()),
+          "nm_match_pairs_span_f32")
+    return (match_out, rec, fb) if want_records else match_out
+
+
 def tc_probe(A, B, want_candidates: bool = False):
     """Diagnostics of the tensor-core engine (nm_match_tc_probe): exact records (nA,4), the number
     of rows whose exactness certificate failed (re-scanned by the exact engine), and optionally

@@ -43,6 +43,21 @@ def align_points(src_x, src_y, dst_x, dst_y, matches):
     return tuple(out)
 
 
+def align_pairs_span(x, y, matches, counts, span):
+    """nm_align_pairs_span_f32: the correspondences of every link of the span layout.  x, y: (n_frames, capacity) cuda
+    float32 keypoint coordinates, matches: (L, capacity) int32 as match_pairs_span returns them, counts: (n_frames,) int32.
+    Returns (c_src_x, c_src_y, c_dst_x, c_dst_y), each (L, capacity)."""
+    import torch
+    _f32(x, y); _int32(matches, "matches"); _int32(counts, "counts")
+    n_frames, cap = x.shape
+    L = matches.shape[0]
+    assert tuple(matches.shape) == (span * n_frames - span * (span + 1) // 2, cap) and counts.numel() == n_frames
+    out = [torch.empty((L, cap), dtype=torch.float32, device=x.device) for _ in range(4)]
+    check(_lib.load().nm_align_pairs_span_f32(_p(x), _p(y), _p(matches), _p(counts), n_frames, cap, span, *[_p(o) for o in out],
+                                              _stream_ptr()), "nm_align_pairs_span_f32")
+    return tuple(out)
+
+
 def ransac_hypotheses(kind, src_x, src_y, dst_x, dst_y, rand_list, inlier_threshold):
     """All hypotheses of a caller-supplied index list: (iterations, 9) homographies and inlier counts."""
     import torch
@@ -126,3 +141,45 @@ def refine(kind, src_x, src_y, dst_x, dst_y, H, status, inlier_threshold, rounds
     Hb, sb, mb = refine_batch(kind, src_x[None], src_y[None], dst_x[None], dst_y[None], None, H.reshape(1, 9),
                               None if status is None else status.reshape(1, 3), inlier_threshold, rounds)
     return Hb[0], sb[0], mb[0]
+
+
+def adjust_chain(kind, src_x, src_y, dst_x, dst_y, counts, span, masks, H, link_status, frame_w, frame_h, inlier_threshold,
+                 iterations=10, out=None):
+    """nm_ransac_adjust_chain_f32 (arguments in its order): joint least-squares adjustment of the poses of a window of n
+    frames from the links of its span layout.  src_x ... dst_y (L, max_pts) and counts (L,) or None as for refine_batch;
+    masks (L, max_pts) bool, H (L, 9) the link models and link_status (L, 3), as refine_batch returns them (rows 0 .. n-2
+    are the consecutive pairs).  inlier_threshold: the RANSAC rule that counts status[:, 1].  out = (H_out, status_out), (n - 1, 9) and
+    (n - 1, 3): written there (they may be H[: n - 1] and link_status[: n - 1]).  Returns (H (n - 1, 9) pairwise models that
+    nm_mosaic_place_f32 chains into the adjusted poses, status (n - 1, 3) = [frame p + 1 connected, inliers, LM steps
+    accepted], chain (n, 9) float64 frame -> frame-0 transforms, report (4,) float64 = [mean squared residual before,
+    after (px^2), residual points, links used])."""
+    import torch
+    _f32(src_x, src_y, dst_x, dst_y)
+    if counts is not None:
+        _int32(counts, "counts")
+    L, max_pts = src_x.shape
+    n = next((m for m in range(2, 1026) if span * m - span * (span + 1) // 2 == L), None) if span >= 1 else None
+    if n is None:
+        raise ValueError(f"{L} links do not form a span-{span} layout")
+    if not (masks.is_cuda and masks.dtype == torch.bool and masks.is_contiguous() and tuple(masks.shape) == (L, max_pts)):
+        raise TypeError("masks: expected a contiguous cuda bool tensor of shape (L, max_pts)")
+    _int32(link_status, "link_status")
+    if not (isinstance(H, torch.Tensor) and H.is_cuda and H.dtype == torch.float32 and H.is_contiguous()
+            and tuple(H.shape) == (L, 9) and tuple(link_status.shape) == (L, 3)):
+        raise TypeError("H, link_status: expected contiguous cuda tensors of shapes (L, 9) float32 and (L, 3) int32")
+    if out is None:
+        H_out = torch.empty((n - 1, 9), dtype=torch.float32, device=H.device)
+        st_out = torch.empty((n - 1, 3), dtype=torch.int32, device=H.device)
+    else:
+        H_out, st_out = out
+        _f32(H_out, H[: n - 1])
+        _int32(st_out, "status_out")
+        if tuple(st_out.shape) != (n - 1, 3):
+            raise TypeError("status_out: expected shape (n - 1, 3)")
+    chain = torch.empty((n, 9), dtype=torch.float64, device=H.device)
+    report = torch.empty(4, dtype=torch.float64, device=H.device)
+    check(_lib.load().nm_ransac_adjust_chain_f32(kind, _p(src_x), _p(src_y), _p(dst_x), _p(dst_y), max_pts,
+                                                 _p(counts) if counts is not None else None, max_pts, inlier_threshold, n, span,
+                                                 frame_w, frame_h, _p(masks), _p(H), _p(link_status), iterations, _p(H_out),
+                                                 _p(st_out), _p(chain), _p(report), _stream_ptr()), "nm_ransac_adjust_chain_f32")
+    return H_out, st_out, chain, report

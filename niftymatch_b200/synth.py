@@ -116,3 +116,57 @@ def descriptors(n: int, seed: int, planted_from: np.ndarray | None = None,
         noise = 2.0 * np.sqrt(-2.0 * np.log(1.0 - w1)) * np.cos(2.0 * np.pi * w2)
         a[rows] = np.maximum(planted_from[src].astype(np.float64) + noise.reshape(k, 128), 0.0)
     return a.astype(np.float32)
+
+
+# ---- synthetic registration windows (tests/test_gpu_chain_adjust.py, tools/ransac_report.py --adjust) ----------------
+def map_points(G, p):
+    """Points p (k, 2) mapped through the 3 x 3 matrix G, in float64."""
+    q = np.c_[p, np.ones(len(p))] @ np.asarray(G, np.float64).reshape(3, 3).T
+    return q[:, :2] / q[:, 2:]
+
+
+def camera_chain(kind, n, w, h, seed, step=0.1):
+    """Frame k -> frame 0 transforms (n, 3, 3) of a camera path in the family of `kind` (0 translation, 1 similarity,
+    2 homography): steps of about step * w px along a slowly turning heading, rotations of up to 0.5 deg, scale changes
+    of up to 0.4 % and small perspective terms per frame."""
+    rng = np.random.default_rng(seed)
+    cx, cy = (w - 1) / 2, (h - 1) / 2
+    T = lambda x, y: np.array([[1, 0, x], [0, 1, y], [0, 0, 1.0]])
+    G, phi = [np.eye(3)], rng.uniform(0, 2 * np.pi)
+    for _ in range(n - 1):
+        phi += rng.normal(0, 0.3)
+        dd = step * w * rng.uniform(0.6, 1.2)
+        M = np.eye(3)
+        if kind >= 1:
+            a, s = np.deg2rad(rng.uniform(-0.5, 0.5)), 1 + rng.uniform(-0.004, 0.004)
+            M = np.array([[s * np.cos(a), -s * np.sin(a), 0], [s * np.sin(a), s * np.cos(a), 0], [0, 0, 1.0]])
+        if kind == 2:
+            sg = rng.choice([-1, 1])
+            M[2, :2] = [sg * 2e-5 * 64 / w, -sg * 2e-5 * 48 / h]
+        H = T(cx + dd * np.cos(phi), cy + dd * np.sin(phi)) @ M @ T(-cx, -cy)      # frame k -> frame k + 1
+        G.append(G[-1] @ np.linalg.inv(H))
+    return np.array(G)
+
+
+def span_window(kind, n, span, w, h, npts, seed, noise=0.3, outliers=0.3, dtype=np.float32):
+    """A window of camera_chain(kind, n, w, h, seed) in the span layout (include/nm_b200.h): for every link (t, t + d) npts
+    correspondences, points of frame t that frame t + d also sees, dst with Gaussian noise of `noise` px and a fraction
+    `outliers` replaced by random points.  Returns (G, [src_x, src_y, dst_x, dst_y] each (L, npts))."""
+    rng = np.random.default_rng(seed + 1000)
+    G = camera_chain(kind, n, w, h, seed)
+    L = span * n - span * (span + 1) // 2
+    arrs = [np.full((L, npts), -1.0, dtype) for _ in range(4)]
+    for l, (t, d) in enumerate((t, d) for d in range(1, span + 1) for t in range(n - d)):
+        M = np.linalg.inv(G[t + d]) @ G[t]
+        src = np.empty((0, 2))
+        while len(src) < npts:
+            p = rng.uniform([0, 0], [w - 1, h - 1], (4 * npts, 2))
+            q = map_points(M, p)
+            ok = (q[:, 0] >= 0) & (q[:, 0] <= w - 1) & (q[:, 1] >= 0) & (q[:, 1] <= h - 1)
+            src = np.concatenate([src, p[ok]])[:npts]
+        dst = map_points(M, src) + rng.normal(0, noise, (npts, 2)) if noise else map_points(M, src)
+        bad = rng.random(npts) < outliers
+        dst[bad] = rng.uniform([0, 0], [w - 1, h - 1], (bad.sum(), 2))
+        for a, v in zip(arrs, (src[:, 0], src[:, 1], dst[:, 0], dst[:, 1])):
+            a[l] = v
+    return G, arrs

@@ -4,7 +4,13 @@ oracle on the fixture scene of tests/_util.py (development aid).
 --refine: the refit leg instead (nm_ransac_refine_batch_f32): time of the batched RANSAC alone and followed by 1 or 2
 refit rounds (64 pairs x 8 192 correspondences, 70 % inliers, 1 024 hypotheses; CUDA events, the three variants in
 alternating windows), corner error against the ground truth of the RANSAC model, the refit and a float64 fit to the
-true inliers, and the 2 048-frame 1080p StreamRegistrar rate of bench.py with refine_rounds 0 and 2."""
+true inliers, and the 2 048-frame 1080p StreamRegistrar rate of bench.py with refine_rounds 0 and 2.
+
+--adjust: the skip-link leg (nm_match_pairs_span_f32 ... nm_ransac_adjust_chain_f32): time per 64-frame 1080p window of
+each stage at span 1, 2, 3 (the frames of bench.py's stream, CUDA events, the spans in alternating windows), the
+2 048-frame 1080p StreamRegistrar rate at span 1, 2, 3 with refine_rounds 0 and 2, and the last frame's corner error on
+the synthetic 64-frame windows of tests/test_gpu_chain_adjust.py for chained span-1 refits and the span-2 / span-3
+adjustment."""
 import os
 import subprocess
 import sys
@@ -95,6 +101,103 @@ def refine_leg():
     sb.close()
 
 
+def _card():
+    card = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit", "--format=csv,noheader", "-i", "0"],
+                          capture_output=True, text=True).stdout.strip()
+    print("card:", card)
+
+
+def adjust_leg():
+    import bench
+    from niftymatch_b200.dist import StreamRegistrar
+    from niftymatch_b200.match import link_row
+    from niftymatch_b200.synth import map_points, span_window
+    _card()
+    stream_np = bench.render_frames(bench.stream_jobs(0, 32))
+    P = nm.SiftParams(bench.W, bench.H)
+    sb = nm.SiftBatch(P, bench.BATCH, bench.CAPACITY)
+    base = torch.from_numpy(stream_np).cuda()
+    frames_of = lambda t0, t1: base.index_select(0, torch.arange(t0, t1, device="cuda") % base.shape[0])
+    # stages of one 64-frame window
+    n, kind, thr, iters = sb.max_batch, 2, 4.0, 1024
+    sb.run(frames_of(0, n))
+    r = sb.results()
+    cnt = r["counts"][:n]
+    state = {}
+
+    def stage(span, name):
+        if name == "match":
+            state["m"] = nm.match_pairs_span(r["desc"][:n], cnt, span, 0.8)
+        elif name == "align":
+            state["c"] = nm.align_pairs_span(r["x"][:n], r["y"][:n], state["m"], cnt, span)
+        elif name == "ransac":
+            out = [nm.ransac_batch(kind, *[c[link_row(n, 0, d): link_row(n, 0, d) + n - d] for c in state["c"]], cnt[: n - d], thr,
+                                   iters, (d - 1) << 40) for d in range(1, span + 1)]
+            state["H"], state["S"] = torch.cat([o[0] for o in out]), torch.cat([o[1] for o in out])
+            state["lc"] = torch.cat([cnt[: n - d] for d in range(1, span + 1)])
+        elif name == "refine":
+            state["H"], state["S"], state["k"] = nm.refine_batch(kind, *state["c"], state["lc"], state["H"], state["S"], thr, 2)
+        else:
+            nm.adjust_chain(kind, *state["c"], state["lc"], span, state["k"], state["H"], state["S"], bench.W, bench.H, thr)
+    names = ("match", "align", "ransac", "refine", "adjust")
+    times = {(s, k): [] for s in (1, 2, 3) for k in names}
+    for rep in range(6):
+        for span in (1, 2, 3):
+            for k in names:
+                e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+                e0.record()
+                stage(span, k)
+                e1.record()
+                torch.cuda.synchronize()
+                if rep >= 1:
+                    times[(span, k)].append(e0.elapsed_time(e1))
+    for span in (1, 2, 3):
+        tot = sum(np.median(times[(span, k)]) for k in names)
+        print(f"span {span}, one 64-frame 1080p window: " + ", ".join(f"{k} {np.median(times[(span, k)]):.2f} ms" for k in names)
+              + f"; sum {tot:.2f} ms")
+    # the stream leg of bench.py
+    n_stream = 2048
+    for rep in range(2):
+        for span in (1, 2, 3):
+            for rounds in (0, 2):
+                reg = StreamRegistrar(sb, chunk=sb.max_batch, refine_rounds=rounds, span=span)
+                reg.run(frames_of, 0, sb.max_batch + 1)
+                torch.cuda.synchronize()
+                e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+                e0.record()
+                Hs, sts = reg.run(frames_of, 0, n_stream)
+                e1.record()
+                torch.cuda.synchronize()
+                ms = e0.elapsed_time(e1)
+                print(f"stream {n_stream} frames 1080p, span {span}, refine_rounds {rounds}: {n_stream / ms * 1e3:.0f} frames/s "
+                      f"({ms:.1f} ms), connected pairs {int((sts[:, 0] == 1).sum())}")
+    sb.close()
+    # synthetic accuracy: windows of synth.span_window through RANSAC per d (link seeds as StreamRegistrar) and 2 refits
+    w, h, n, thr = 640, 480, 64, 4.0
+    c = np.array([[0, 0], [w - 1, 0], [0, h - 1], [w - 1, h - 1]], np.float64)
+    for kind in (0, 1, 2):
+        e = {1: [], 2: [], 3: []}
+        for wnd in range(4):
+            seed = 90 + 10 * wnd + kind
+            G, arrs = span_window(kind, n, 3, w, h, 2000, seed)
+            d_ = [torch.from_numpy(a).cuda() for a in arrs]
+            out = [nm.ransac_batch(kind, *[a[link_row(n, 0, d): link_row(n, 0, d) + n - d] for a in d_], None, thr, 512,
+                                   seed + ((d - 1) << 40)) for d in (1, 2, 3)]
+            HL, SL, mask = nm.refine_batch(kind, *d_, None, torch.cat([o[0] for o in out]), torch.cat([o[1] for o in out]), thr, 2)
+            last = lambda Gk: np.hypot(*(map_points(Gk[-1], c) - map_points(G[-1], c)).T).mean()
+            e[1].append(last(nm.place(HL[: n - 1].contiguous(), SL[: n - 1].contiguous(), w, h).chain.cpu().numpy().reshape(n, 3, 3)))
+            for span in (2, 3):                  # the span-2 layout is the first rows of the span-3 one
+                L = span * n - span * (span + 1) // 2
+                _, _, chain, _ = nm.adjust_chain(kind, *[a[:L] for a in d_], None, span, mask[:L], HL[:L], SL[:L], w, h, thr)
+                e[span].append(last(chain.cpu().numpy().reshape(n, 3, 3)))
+        m = {k: float(np.mean(v)) for k, v in e.items()}
+        print(f"synthetic 64-frame windows (4), kind {kind}: last frame mean corner error, chained span-1 refits "
+              f"{m[1]:.4f} px, span 2 {m[2]:.4f} px ({m[2] / m[1]:.3f}), span 3 {m[3]:.4f} px ({m[3] / m[1]:.3f})")
+
+
+if "--adjust" in sys.argv:
+    adjust_leg()
+    sys.exit(0)
 if "--refine" in sys.argv:
     refine_leg()
     sys.exit(0)
