@@ -8,21 +8,21 @@
 //                       3x thrust::fill + detect_keypoints, keypoint.cu:183-200)
 //   PyramidData::gpu_collate_keypoints_for_level (gpu/sift/pyramidata.cu:84-91, copy_if)
 //
-// Design: one fused stencil pass reads the 6 Gaussian levels of a tile once, forms the 5
-// DoG values in shared memory (never materialised in HBM), tests the 3 detection levels,
-// refines/rejects candidates and writes (a) the 3 gradient maps and (b) ONE BIT per pixel
-// and level (warp ballot -> one 32-bit store per 32 pixels).  The ordered keypoint list
-// ("copy_if order": raster within a level, levels ascending, octaves ascending) is then
-// produced from the bitmaps: a per-segment popcount scan gives every word its rank, a tiny
-// planning kernel applies the reference's early-return and capacity rules, and an emit
-// kernel re-runs the (deterministic) refinement for the set bits only and writes each
-// keypoint at its final slot.  No dense float4 maps (16 B/pixel/level in the reference),
-// no thrust::fill, no device->host count round trips.
+// Design: the stencil pass (extrema_kernel) reads the 6 Gaussian levels of a tile once, forms
+// the 5 DoG values in registers (never materialised in HBM), tests the 3 detection levels and
+// lists the extremum candidates; refine_list_kernel refines/rejects them and sets ONE BIT per
+// accepted pixel and level.  The ordered keypoint list ("copy_if order": raster within a
+// level, levels ascending, octaves ascending) is then produced from the bitmaps: a per-segment
+// popcount scan gives every word its rank, a tiny planning kernel applies the reference's
+// early-return and capacity rules, an emit kernel writes each set bit's pixel at its final
+// slot, and kprefine_kernel re-runs the (deterministic) refinement there and marks the
+// gradient-map blocks the keypoint's windows read.  gradmap_kernel then computes only those
+// blocks.  No dense float4 maps (16 B/pixel/level in the reference), no thrust::fill, no
+// device->host count round trips.
 #include "nm_sift_internal.cuh"
 #include "nm_pyramid.cuh"
 #include "nm_refine.cuh"
 #include "nm_kpgeom.cuh"
-#include <cstdlib>
 
 namespace {
 
@@ -31,180 +31,7 @@ namespace {
 constexpr int EX_TW = 32, EX_TH = 32, EX_HL = 4, EX_P = EX_TW + 2 * EX_HL, EX_ROWS = EX_TH + 2;
 constexpr uint32_t EX_TILE_BYTES = 6u * EX_ROWS * EX_P * sizeof(float);   // 32 640
 
-struct SmemDogFetch {
-    const float (*dog)[EX_ROWS][EX_P];     // [5]
-    int l, r, c;                           // detection level (0..2), tile row/col of the centre
-    __device__ __forceinline__ float cur(int dx, int dy) const { return dog[l + 1][r + dy][c + dx]; }
-    __device__ __forceinline__ float down(int dx, int dy) const { return dog[l][r + dy][c + dx]; }
-    __device__ __forceinline__ float up(int dx, int dy) const { return dog[l + 2][r + dy][c + dx]; }
-};
-
 __device__ __forceinline__ uint32_t ex_smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-
-// One CTA = one 32 x 32 pixel tile of one frame.  The six Gaussian levels of the 34 x 36 window (1-pixel
-// halo; 40 columns keep the window start 16-byte aligned) arrive by ONE bulk tensor load (x, y, level) with hardware
-// zero fill outside the image.  Phase 1 turns levels 1..3 into the three gradient maps; phase 2 replaces the
-// window in place by the five DoG levels (cudamath.cu:34); phase 3 is the 26-neighbour test, the refinement
-// and the 1-bit-per-pixel result.
-template <bool TMA>
-__global__ void __launch_bounds__(256, 4) extrema_grad_kernel(const NmOctave oc, const NmDetectParams dp,
-                                                              const __grid_constant__ CUtensorMap tmap)
-{
-    __shared__ __align__(128) float s_tile[6][EX_ROWS][EX_P];
-    __shared__ __align__(8) uint64_t s_bar;
-    const int tid = threadIdx.y * 32 + threadIdx.x;
-    const int f = blockIdx.z, x0 = blockIdx.x * EX_TW, y0 = blockIdx.y * EX_TH;
-
-    if (TMA) {
-        if (tid == 0) {
-            const uint32_t bar = ex_smem_u32(&s_bar);
-            asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(bar));
-            asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-            asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(EX_TILE_BYTES) : "memory");
-            asm volatile(
-                "cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3, %4}], [%5];"
-                ::"r"(ex_smem_u32(&s_tile[0][0][0])), "l"(reinterpret_cast<uint64_t>(&tmap)), "r"(x0 - EX_HL), "r"(y0 - 1),
-                  "r"(f * 6), "r"(bar) : "memory");
-        }
-        __syncthreads();                                   // barrier initialised before anyone polls it
-        asm volatile(
-            "{\n"
-            ".reg .pred p;\n"
-            "LAB_WAIT_%=:\n"
-            "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], 0;\n"
-            "@p bra LAB_DONE_%=;\n"
-            "bra LAB_WAIT_%=;\n"
-            "LAB_DONE_%=:\n"
-            "}\n" ::"r"(ex_smem_u32(&s_bar)) : "memory");
-    } else {
-        const float* __restrict__ L = oc.levels + (long long)f * 6 * oc.level_elems;
-        for (int i = tid; i < EX_ROWS * EX_P; i += 256) {
-            const int r = i / EX_P, c = i - r * EX_P;
-            const int gy = y0 - 1 + r, gx = x0 - EX_HL + c;
-            const bool in = gy >= 0 && gy < oc.h && gx >= 0 && gx < oc.w;
-#pragma unroll
-            for (int k = 0; k < 6; ++k)
-                s_tile[k][r][c] = in ? __ldg(L + k * oc.level_elems + (long long)gy * oc.pitch + gx) : 0.f;
-        }
-        __syncthreads();
-    }
-
-    const int lane = threadIdx.x;
-    const int gx = x0 + lane;
-    float2* __restrict__ G = oc.grad + (long long)f * 3 * oc.level_elems;
-    const long long bm_words = (long long)oc.h * oc.wpr;
-    uint32_t* __restrict__ BM = oc.bitmap + (long long)f * 3 * bm_words;
-
-    // ---- phase 1: gradient maps of levels 1..3 (cudamath.cu:38-54; border pixels = (0, 0)) ----------
-    {
-        const bool inx = gx < oc.w, intx = gx >= 1 && gx <= oc.w - 2;
-        const int c = lane + EX_HL;
-#pragma unroll 1
-        for (int i = 0; i < EX_TH / 8; ++i) {
-            const int ly = threadIdx.y * (EX_TH / 8) + i, gy = y0 + ly, r = ly + 1;
-            if (gy >= oc.h) break;                              // warp uniform
-            const bool interior = intx && gy >= 1 && gy <= oc.h - 2;
-#pragma unroll
-            for (int l = 0; l < 3; ++l) {
-                float2 g = make_float2(0.f, 0.f);
-                if (interior)
-                    g = nm_gradient_at(s_tile[l + 1][r][c + 1], s_tile[l + 1][r][c - 1], s_tile[l + 1][r + 1][c], s_tile[l + 1][r - 1][c]);
-                if (inx) G[l * oc.level_elems + (long long)gy * oc.pitch + gx] = g;
-            }
-        }
-    }
-    __syncthreads();
-
-    // ---- phase 2: levels -> DoG in place: slot k = level k+1 - level k (k = 0..4), four columns per item ----
-    {
-        float4 (*t4)[EX_ROWS][EX_P / 4] = reinterpret_cast<float4 (*)[EX_ROWS][EX_P / 4]>(s_tile);
-        for (int i = tid; i < EX_ROWS * (EX_P / 4); i += 256) {
-            const int r = i / (EX_P / 4), q = i - r * (EX_P / 4);
-            float4 v[6];
-#pragma unroll
-            for (int k = 0; k < 6; ++k) v[k] = t4[k][r][q];
-#pragma unroll
-            for (int k = 0; k < 5; ++k)
-                t4[k][r][q] = make_float4(__fsub_rn(v[k + 1].x, v[k].x), __fsub_rn(v[k + 1].y, v[k].y),
-                                          __fsub_rn(v[k + 1].z, v[k].z), __fsub_rn(v[k + 1].w, v[k].w));
-        }
-    }
-    __syncthreads();
-    const float (*s_dog)[EX_ROWS][EX_P] = s_tile;
-
-    // ---- phase 3: 26-neighbour extremum test for the thread's 4 pixels x 3 levels, separably --------
-    // 3-wide row maxima / minima of every DoG level (with and without the centre column) are shared
-    // by the vertically adjacent pixels of the thread, so a pixel costs ~46 FMNMX3 + 23 LDS instead of
-    // 78 + 81 (the kernel is issue bound).  Same comparisons as keypoint.cu:19-105: strict, against the
-    // max / min of the 26 neighbours.
-    unsigned extmask = 0;                      // bit l * 4 + i
-    {
-        const int c = lane + EX_HL, rbase = threadIdx.y * (EX_TH / 8);      // tile row of the first pixel's upper neighbour
-        const float t = __fmul_rn(0.8f, dp.peak);
-        // levels are walked bottom-up with a 3-deep window of the 3x3 (centre included) maxima, so that
-        // detection level l = k - 2 is decided as soon as DoG level k is reduced (keeps ~50 values live)
-        float m9x[3][4], m9n[3][4];            // ring over k % 3
-        float m8x[4], m8n[4], cv[4];           // DoG level k - 1 (centre excluded) and its centre values
-        float p8x[4], p8n[4], pcv[4];
-#pragma unroll
-        for (int k = 0; k < 5; ++k) {
-            float hx[6], hn[6], gxm[6], gnm[6], ctr[6];
-#pragma unroll
-            for (int rr = 0; rr < 6; ++rr) {
-                const float a = s_dog[k][rbase + rr][c - 1], b = s_dog[k][rbase + rr][c], d = s_dog[k][rbase + rr][c + 1];
-                hx[rr] = fmaxf(fmaxf(a, b), d);
-                hn[rr] = fminf(fminf(a, b), d);
-                gxm[rr] = fmaxf(a, d);
-                gnm[rr] = fminf(a, d);
-                ctr[rr] = b;
-            }
-#pragma unroll
-            for (int j = 0; j < 4; ++j) {
-                m9x[k % 3][j] = fmaxf(fmaxf(hx[j], hx[j + 1]), hx[j + 2]);
-                m9n[k % 3][j] = fminf(fminf(hn[j], hn[j + 1]), hn[j + 2]);
-                p8x[j] = m8x[j]; p8n[j] = m8n[j]; pcv[j] = cv[j];          // those of DoG level k - 1
-                m8x[j] = fmaxf(fmaxf(hx[j], gxm[j + 1]), hx[j + 2]);
-                m8n[j] = fminf(fminf(hn[j], gnm[j + 1]), hn[j + 2]);
-                cv[j] = ctr[j + 1];
-            }
-            if (k >= 2) {
-                const int l = k - 2;           // down = k - 2, current = k - 1, up = k
-#pragma unroll
-                for (int j = 0; j < 4; ++j) {
-                    const float mx = fmaxf(fmaxf(m9x[(k - 2) % 3][j], p8x[j]), m9x[k % 3][j]);
-                    const float mn = fminf(fminf(m9n[(k - 2) % 3][j], p8n[j]), m9n[k % 3][j]);
-                    const float c0 = pcv[j];
-                    if ((c0 <= t && c0 < mn) || (c0 >= t && c0 > mx)) extmask |= 1u << (l * 4 + j);   // keypoint.cu:195-196
-                }
-            }
-        }
-    }
-#pragma unroll 1
-    for (int i = 0; i < EX_TH / 8; ++i) {
-        const int ly = threadIdx.y * (EX_TH / 8) + i;
-        const int gy = y0 + ly;
-        if (gy >= oc.h) break;                                  // warp uniform
-        const bool interior = gx >= 1 && gx <= oc.w - 2 && gy >= 1 && gy <= oc.h - 2;
-        const int r = ly + 1, c = lane + EX_HL;
-#pragma unroll
-        for (int l = 0; l < 3; ++l) {
-            bool acc = false;
-            if (interior && ((extmask >> (l * 4 + i)) & 1u)) {
-                // compute_keypoints_with_mask: pixels whose mask sample is < 1 are skipped (keypoint.cu:214; the
-                // reference tests it first, the outcome is the same) -- one texture fetch per extremum candidate
-                const bool masked_out = dp.mask != 0 &&
-                    tex2D<float>((cudaTextureObject_t)dp.mask, (gx + 0.5f) * oc.xper, (gy + 0.5f) * oc.xper) < 1.f;
-                if (!masked_out) {
-                    SmemDogFetch ft{s_dog, l, r, c};
-                    float4 out;
-                    acc = nm_refine(ft, gx, gy, dp.peak, dp.edge, oc.xper, dp.sigma_0, dp.num_dogs, l, out);
-                }
-            }
-            const unsigned m = __ballot_sync(0xffffffffu, acc);
-            if (lane == 0) BM[l * bm_words + (long long)gy * oc.wpr + blockIdx.x] = m;
-        }
-    }
-}
 
 struct GlobalDogFetch {
     const float* L;            // frame's level 0 at the candidate pixel
@@ -220,7 +47,7 @@ struct GlobalDogFetch {
     __device__ __forceinline__ float up(int dx, int dy) const { return dogv(l + 2, dx, dy); }
 };
 
-// ------------------------- split pipeline: extrema without gradients -------------------------
+// ------------------------- extrema and their refinement -------------------------
 // DoG values formed on the fly from the staged Gaussian levels (cudamath.cu:34: next - this).
 struct SmemLevelFetch {
     const float (*lv)[EX_ROWS][EX_P];      // [6]
@@ -677,7 +504,7 @@ __global__ void __launch_bounds__(256) emit_kernel(const NmOctave oc, int octave
 // per-word kernel above would run the ~400-instruction refinement (double pow) with one live lane.
 __global__ void __launch_bounds__(256) kprefine_kernel(const NmOctaveTable tab, const NmDetectParams dp, int capacity,
                                                        const int* __restrict__ counts, float4* __restrict__ kpts,
-                                                       const int* __restrict__ meta, int mark)
+                                                       const int* __restrict__ meta)
 {
     const int j = blockIdx.x * 256 + threadIdx.x, f = blockIdx.y;
     if (j >= counts[f]) return;
@@ -689,7 +516,7 @@ __global__ void __launch_bounds__(256) kprefine_kernel(const NmOctaveTable tab, 
     float4 out = make_float4(-1.f, -1.f, -1.f, -1.f);
     nm_refine(ft, x, y, dp.peak, dp.edge, oc.xper, dp.sigma_0, dp.num_dogs, l, out);
     kpts[kidx] = out;
-    if (mark && oc.need != nullptr && out.w >= 0.f) mark_gradient_need(oc, f, out);
+    if (out.w >= 0.f) mark_gradient_need(oc, f, out);
 }
 
 // ------------------------- compat: dense per-pixel maps -------------------------
@@ -805,51 +632,34 @@ bool nm_extrema_make_tma(NmBlurTma* t, const NmOctave& oc, int batch)
     return nm_tma_encode_3d(t, oc.levels, dims, strides, box);
 }
 
-// Split pipeline (default): extrema_kernel here, gradmap_kernel after the compaction.  The fused round-1 kernel
-// stays as the path for levels TMA cannot describe; it writes dense gradient maps itself.  NM_EXTREMA_FUSED=1 forces
-// it (test hook: the parity tests are re-run on this path).  Returns through *fused which one ran.
-static bool extrema_use_fused(const NmBlurTma* tma)
+// extrema_kernel + refine_list_kernel over one octave; the gradient maps follow the compaction (nm_gradmap_launch).
+// The window is staged by TMA only: `tma` is the descriptor nm_extrema_make_tma made for these levels.
+int nm_extrema_launch(const NmOctave& oc, const NmDetectParams& dp, int batch, cudaStream_t stream, const NmBlurTma* tma)
 {
-    static const bool forced = getenv("NM_EXTREMA_FUSED") != nullptr;
-    return forced || !(tma && tma->valid);
-}
-
-bool nm_extrema_is_fused(const NmBlurTma* tma) { return extrema_use_fused(tma); }
-
-int nm_extrema_launch(const NmOctave& oc, int, int, const NmDetectParams& dp, int batch, cudaStream_t stream,
-                      const NmBlurTma* tma, bool fused)
-{
+    if (!tma || !tma->valid) return NM_ERR_UNSUPPORTED;
     dim3 block(32, 8), grid(nm_div_up(oc.w, EX_TW), nm_div_up(oc.h, EX_TH), batch);
-    if (!fused) {
-        if (extrema_use_fused(tma) && !(tma && tma->valid)) return NM_ERR_INVALID;
-        static NmDeviceOnce once;
-        static std::atomic<int> ctas_cfg{2};
-        if (once.first()) {
-            int per_sm = 2;
-            NM_CUDA_TRY(cudaFuncSetAttribute(extrema_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, EX2_SMEM));
-            NM_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, extrema_kernel, 256, EX2_SMEM));
-            ctas_cfg.store(per_sm < 1 ? 1 : per_sm);
-            once.done();
-        }
-        const int n_sms = nm_sm_count(), ctas_per_sm = ctas_cfg.load();
-        if (n_sms <= 0) return NM_ERR_NO_DEVICE;
-        const long long n_tiles = (long long)grid.x * grid.y * grid.z;
-        if (n_tiles >= (1LL << 31) / EX2_LIST || !oc.cand_n || !oc.cand) return NM_ERR_OVERFLOW;
-        // 4x the resident count: co-resident CTAs do not advance evenly, and with exactly-resident persistent CTAs the
-        // launch ends on half-empty SMs; the hardware hands an SM its next CTA as one retires (64 x 1080p: 1.27 -> 1.21 ms,
-        // 2x 1.23, 8x 1.21; B200).
-        const long long want = (long long)n_sms * ctas_per_sm * 4;
-        const int ctas = (int)(n_tiles < want ? n_tiles : want);
-        extrema_kernel<<<ctas, block, EX2_SMEM, stream>>>(oc, dp, tma->map, (int)grid.x, (int)grid.y, (int)n_tiles, oc.cand_n, oc.cand);
-        NM_LAUNCH_CHECK();
-        refine_list_kernel<<<(unsigned)nm_div_up64(n_tiles, 8), 256, 0, stream>>>(oc, dp, (int)grid.x, (int)grid.y, (int)n_tiles,
-                                                                                oc.cand_n, oc.cand);
-    } else if (tma && tma->valid) {
-        extrema_grad_kernel<true><<<grid, block, 0, stream>>>(oc, dp, tma->map);
-    } else {
-        CUtensorMap none{};
-        extrema_grad_kernel<false><<<grid, block, 0, stream>>>(oc, dp, none);
+    static NmDeviceOnce once;
+    static std::atomic<int> ctas_cfg{2};
+    if (once.first()) {
+        int per_sm = 2;
+        NM_CUDA_TRY(cudaFuncSetAttribute(extrema_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, EX2_SMEM));
+        NM_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, extrema_kernel, 256, EX2_SMEM));
+        ctas_cfg.store(per_sm < 1 ? 1 : per_sm);
+        once.done();
     }
+    const int n_sms = nm_sm_count(), ctas_per_sm = ctas_cfg.load();
+    if (n_sms <= 0) return NM_ERR_NO_DEVICE;
+    const long long n_tiles = (long long)grid.x * grid.y * grid.z;
+    if (n_tiles >= (1LL << 31) / EX2_LIST || !oc.cand_n || !oc.cand) return NM_ERR_OVERFLOW;
+    // 4x the resident count: co-resident CTAs do not advance evenly, and with exactly-resident persistent CTAs the
+    // launch ends on half-empty SMs; the hardware hands an SM its next CTA as one retires (64 x 1080p: 1.27 -> 1.21 ms,
+    // 2x 1.23, 8x 1.21; B200).
+    const long long want = (long long)n_sms * ctas_per_sm * 4;
+    const int ctas = (int)(n_tiles < want ? n_tiles : want);
+    extrema_kernel<<<ctas, block, EX2_SMEM, stream>>>(oc, dp, tma->map, (int)grid.x, (int)grid.y, (int)n_tiles, oc.cand_n, oc.cand);
+    NM_LAUNCH_CHECK();
+    refine_list_kernel<<<(unsigned)nm_div_up64(n_tiles, 8), 256, 0, stream>>>(oc, dp, (int)grid.x, (int)grid.y, (int)n_tiles,
+                                                                            oc.cand_n, oc.cand);
     NM_LAUNCH_CHECK();
     return NM_OK;
 }
@@ -894,10 +704,10 @@ int nm_emit_launch(const NmOctave& oc, int octave_index, int n_oct, int batch,
 }
 
 int nm_kprefine_launch(const NmOctaveTable& tab, const NmDetectParams& dp, int batch, int capacity, const int* counts,
-                       float4* kpts, const int* meta, int mark, cudaStream_t stream)
+                       float4* kpts, const int* meta, cudaStream_t stream)
 {
     dim3 grid(nm_div_up(capacity, 256), batch);
-    kprefine_kernel<<<grid, 256, 0, stream>>>(tab, dp, capacity, counts, kpts, meta, mark);
+    kprefine_kernel<<<grid, 256, 0, stream>>>(tab, dp, capacity, counts, kpts, meta);
     NM_LAUNCH_CHECK();
     return NM_OK;
 }

@@ -407,16 +407,13 @@ static int sift_run_range(nm_sift_ctx* c, const float* frames_dev, int first, in
         NM_CUDA_TRY(cudaStreamWaitEvent(st, c->ev_side_join, 0));
     }
     if (timing) cudaEventRecord(c->ev[1], st);
-    // ---- DoG + extrema + refinement (+ dense gradient maps in the fused fallback) ----------
-    bool fused = false;
-    for (int o = 0; o < c->n_oct; ++o) fused = fused || nm_extrema_is_fused(&ts->ex[o]);
-    if (fused) for (int o = 0; o < c->n_oct; ++o) tab.o[o].need = nullptr;      // emit_kernel does not mark
+    // ---- DoG + extrema + refinement -----------------------------------------------------
     for (int o = 0; o < c->n_oct; ++o) {
-        if ((rc = nm_extrema_launch(tab.o[o], o, c->n_oct, dp, n, st, &ts->ex[o], fused)) != NM_OK) return rc;
-        launches += fused ? 1 : 2;
+        if ((rc = nm_extrema_launch(tab.o[o], dp, n, st, &ts->ex[o])) != NM_OK) return rc;
+        launches += 2;
     }
     if (timing) cudaEventRecord(c->ev[2], st);
-    // ---- ordered compaction (emit also marks the gradient blocks the keypoint windows read) ----
+    // ---- ordered compaction (kprefine also marks the gradient blocks the keypoint windows read) ----
     if ((rc = nm_rank_launch(tab, n, seg_raw, st)) != NM_OK) return rc;
     if ((rc = nm_plan_launch(seg_raw, seg_cnt, seg_off, counts, c->n_oct, n, c->capacity, st)) != NM_OK) return rc;
     launches += 2;
@@ -424,14 +421,12 @@ static int sift_run_range(nm_sift_ctx* c, const float* frames_dev, int first, in
         if ((rc = nm_emit_launch(tab.o[o], o, c->n_oct, n, seg_cnt, seg_off, c->capacity, kpts, meta, st)) != NM_OK) return rc;
         ++launches;
     }
-    if ((rc = nm_kprefine_launch(tab, dp, n, c->capacity, counts, kpts, meta, fused ? 0 : 1, st)) != NM_OK) return rc;
+    if ((rc = nm_kprefine_launch(tab, dp, n, c->capacity, counts, kpts, meta, st)) != NM_OK) return rc;
     ++launches;
     if (timing) cudaEventRecord(c->ev[3], st);
     // ---- gradient maps of the marked blocks ----------------------------------------------
-    if (!fused) {
-        if ((rc = nm_gradmap_launch(tab, n, c->dense_grad, st)) != NM_OK) return rc;
-        launches += c->n_oct;
-    }
+    if ((rc = nm_gradmap_launch(tab, n, c->dense_grad, st)) != NM_OK) return rc;
+    launches += c->n_oct;
     if (timing) cudaEventRecord(c->ev[4], st);
     // ---- orientation, descriptor -----------------------------------------------------
     if ((rc = nm_orient_launch(tab, n, c->capacity, counts, kpts, meta, orient, st)) != NM_OK) return rc;

@@ -47,26 +47,22 @@ struct NmDetectParams {
 // nm_extrema.cu
 struct NmBlurTma;
 // TMA descriptor of an octave's level planes for `batch` frames (oc.levels = first frame): box = the
-// extrema kernel's 36 x 34 x 6 window.  Without a valid descriptor the kernel stages the window with plain loads.
+// extrema kernel's 40 x 34 x 6 window.
 bool nm_extrema_make_tma(NmBlurTma* t, const NmOctave& oc, int batch);
-// fused = true: the round-1 kernel that also writes dense gradient maps (the only one for sources TMA cannot
-// describe); fused = false: extrema_kernel (needs a valid descriptor), gradient maps by nm_gradmap_launch.
-int nm_extrema_launch(const NmOctave& oc, int octave_index, int n_oct, const NmDetectParams& dp,
-                      int batch, cudaStream_t stream, const NmBlurTma* tma, bool fused);
-// true when nm_extrema_launch takes the fused round-1 kernel (which also writes dense gradient maps) for this source
-bool nm_extrema_is_fused(const NmBlurTma* tma);
+// extrema + refinement of one octave into NmOctave::bitmap; NM_ERR_UNSUPPORTED without a valid descriptor
+int nm_extrema_launch(const NmOctave& oc, const NmDetectParams& dp, int batch, cudaStream_t stream, const NmBlurTma* tma);
 // gradient maps of levels 1..3 for all octaves; dense = 0: only the blocks marked in NmOctave::need
 int nm_gradmap_launch(const NmOctaveTable& tab, int batch, int dense, cudaStream_t stream);
 int nm_rank_launch(const NmOctaveTable& tab, int batch, int* seg_raw, cudaStream_t stream);
 int nm_plan_launch(const int* seg_raw, int* seg_cnt, int* seg_off, int* counts, int n_oct, int batch,
                    int capacity, cudaStream_t stream);
 // emit: slot <- pixel (x, y, level) of every set bit, in copy_if order; kprefine: slot <- refined keypoint payload
-// (one thread per keypoint), mark != 0 also marks NmOctave::need from the keypoint's windows
+// (one thread per keypoint), which also marks NmOctave::need from the keypoint's windows
 int nm_emit_launch(const NmOctave& oc, int octave_index, int n_oct, int batch,
                    const int* seg_cnt, const int* seg_off, int capacity, float4* kpts, int* meta,
                    cudaStream_t stream);
 int nm_kprefine_launch(const NmOctaveTable& tab, const NmDetectParams& dp, int batch, int capacity, const int* counts,
-                       float4* kpts, const int* meta, int mark, cudaStream_t stream);
+                       float4* kpts, const int* meta, cudaStream_t stream);
 
 // nm_orient_desc.cu
 int nm_orient_launch(const NmOctaveTable& tab, int batch, int capacity, const int* counts,

@@ -459,22 +459,6 @@ def test_sparse_gradient_maps_give_identical_results(nm):
         sb.close()
 
 
-def test_fused_extrema_fallback_parity_suite():
-    """NM_EXTREMA_FUSED=1 selects the fused round-1 kernel (DoG + extrema + dense gradient maps in one pass), which
-    is also the path for levels TMA cannot describe; the SIFT parity tests are re-run that way in a child process."""
-    import subprocess
-    import sys
-    if os.environ.get("NM_EXTREMA_FUSED"):
-        pytest.skip("already the forced run")
-    env = dict(os.environ, NM_EXTREMA_FUSED="1")
-    sel = ("test_sift_vs_oracle or test_sift_vs_reference_golden or test_forced_octave_count or "
-           "test_masked_detector_batched_vs_reference_and_oracle or test_sparse_gradient_maps_give_identical_results")
-    r = subprocess.run([sys.executable, "-m", "pytest", "-x", "-q", "-m", "gpu", "-p", "no:cacheprovider", __file__, "-k", sel],
-                       env=env, capture_output=True, text=True, cwd=os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
-    assert r.returncode == 0, r.stdout[-3000:] + r.stderr[-2000:]
-    assert " passed" in r.stdout
-
-
 @pytest.mark.parametrize("stream", ["1", "0"])
 def test_forced_strip_blur_parity_suite(stream):
     """The strip-walking blur kernels are only chosen for large launches; NM_BLUR_STRIP_MIN=1 forces them for every
