@@ -390,8 +390,8 @@ int nm_ransac_refine_batch_f32(int kind, const float* src_x, const float* src_y,
  *   Initial poses: for k = 1 .. n-1 the smallest d <= span with frame k-d connected, link_status[(k-d, d)][0] == 1 and
  *     at least 1 / 2 / 4 mask points gives G_k = G_(k-d) . H^-1 (the chaining rule of nm_mosaic_place_f32); without one
  *     frame k is disconnected: G_k = G_(k-1), fixed, and its links are ignored.
- *   Cost: sum over the links usable that way (both frames connected) and their mask points of
- *     |pi(G_t s_i) - pi(G_(t+d) d_i)|^2, in frame-0 pixels.
+ *   Cost (nm_ransac_adjust_chain_f32: NM_ADJUST_MOSAIC): sum over the links usable that way (both frames connected)
+ *     and their mask points of |pi(G_t s_i) - pi(G_(t+d) d_i)|^2, in frame-0 pixels.
  *   Solver: Levenberg-Marquardt, lambda0 = 1e-3 max diag(J^T J), / 10 after an accepted step, * 10 after a rejected one,
  *     at most `iterations` (>= 1) builds of the banded normal equations, banded Cholesky in one CTA; the final cost is
  *     never above the initial one.
@@ -408,6 +408,24 @@ int nm_ransac_adjust_chain_f32(int kind, const float* src_x, const float* src_y,
                                int n_frames, int span, int frame_w, int frame_h, const unsigned char* masks,
                                const float* H_links, const int* link_status, int iterations, float* H_out,
                                int* status_out, double* chain_out, double* report_out, nm_stream_t stream);
+
+/* Residual of the chain adjustment (nm_ransac_adjust_chain_cost_f32). */
+#define NM_ADJUST_MOSAIC   0   /* pi(G_t s_i) - pi(G_(t+d) d_i), frame-0 (mosaic) pixels: nm_ransac_adjust_chain_f32 */
+#define NM_ADJUST_TRANSFER 1   /* pi(G_(t+d)^-1 G_t s_i) - d_i, pixels of frame t + d (the RANSAC rule's direction) */
+
+/* nm_ransac_adjust_chain_f32 with a choice of residual; cost NM_ADJUST_MOSAIC is bitwise nm_ransac_adjust_chain_f32.
+ * NM_ADJUST_TRANSFER measures every link's residual in the pixels of its own target frame t + d, so it depends only on
+ * the relative poses G_(t+d)^-1 G_t: unlike the mosaic cost it gains nothing from shrinking the frames far from frame 0,
+ * which on long windows of similarity or homography models contracts the chain.  Unknowns, gauge, initial poses, links
+ * used, solver and outputs are those of nm_ransac_adjust_chain_f32; report_out is in pixels of the target frames.  A point
+ * with a non-positive third coordinate of G_(t+d)^-1 G_t s_i, or a non-finite residual, makes the cost of a trial point
+ * +inf (the step is rejected); at the initial poses it leaves the window unadjusted (initial chain, 0 LM steps, both
+ * costs in report_out +inf).  cost outside {NM_ADJUST_MOSAIC, NM_ADJUST_TRANSFER}: NM_ERR_INVALID. */
+int nm_ransac_adjust_chain_cost_f32(int kind, int cost, const float* src_x, const float* src_y, const float* dst_x,
+                                    const float* dst_y, long long pair_stride, const int* counts, int max_pts,
+                                    float inlier_threshold, int n_frames, int span, int frame_w, int frame_h,
+                                    const unsigned char* masks, const float* H_links, const int* link_status, int iterations,
+                                    float* H_out, int* status_out, double* chain_out, double* report_out, nm_stream_t stream);
 
 /* ------------------------------------------------------------------------ */
 /* Batched SIFT detect+describe: the client loop of the reference             */

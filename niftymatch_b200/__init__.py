@@ -10,6 +10,6 @@ from ._lib import load, NmError, LIB_PATH, SiftParamsC  # noqa: F401
 from .sift import SiftParams, SiftBatch, gaussian_taps, grayscale, cast_u8, undistort_map  # noqa: F401
 from .match import match, match_top2, merge_top2, match_pairs, match_pairs_span, set_engine, get_engine, tc_probe  # noqa: F401
 from .ransac import (align_points, align_pairs_span, ransac, ransac_batch, ransac_hypotheses, refine, refine_batch,  # noqa: F401
-                     adjust_chain, TRANSLATION, SIMILARITY, HOMOGRAPHY)
+                     adjust_chain, TRANSLATION, SIMILARITY, HOMOGRAPHY, MOSAIC, TRANSFER)
 from .dist import shard_bounds, match_sharded, frame_range, register_stream  # noqa: F401
 from .mosaic import Mosaic, Placement, place, render_stream  # noqa: F401

@@ -927,6 +927,10 @@ __global__ void __launch_bounds__(kRefineThreads, 1) refine_kernel(const Pairs P
 // ---- joint adjustment of a window's chain (nm_ransac_adjust_chain_f32; no reference counterpart) -------------------
 // Unknowns: G_k, frame k -> frame-0 pixels, k = 1 .. n-1, G_0 = I.  G_k = N^-1 Gn_k N with N = the frame centred and
 // scaled by 2 / max(w, h); Gn_k has P = 2 / 4 / 8 parameters (translation / similarity / homography with Gn[8] = 1).
+// Residual of correspondence (a, b) on link (t, u = t + d), normalised, by cost:
+//   NM_ADJUST_MOSAIC (0):   pi(Gn_t a) - pi(Gn_u b), the disagreement in frame-0 (mosaic) coordinates;
+//   NM_ADJUST_TRANSFER (1): pi(Gn_u^-1 Gn_t a) - b, the forward transfer error in frame u, which depends on the
+//     relative pose only.  A point with p3 <= 0 or a non-finite residual makes the cost of that point +inf.
 // Every sum below is fp64 and is formed in a fixed order, so a window's result is bit-reproducible.
 constexpr int kAdjMaxFrames = 1024, kAdjMaxSpan = 8;
 constexpr int kAdjSlices = 4;               // CTAs per link in the normal-equation build
@@ -942,7 +946,8 @@ template <int KIND> struct AdjFam {
 
 struct AdjState {
     double lambda, cost, cost0;             // lambda < 0: not initialised yet
-    int first, done, accepted, pad;
+    int first, done, accepted;
+    int nonfinite;                          // set by a transfer-cost build: a point at x_eval has p3 <= 0 or a non-finite residual
 };
 
 struct AdjGeom {
@@ -1025,6 +1030,46 @@ __device__ __forceinline__ void adj_project(const double* th, double px, double 
     }
 }
 
+// The two rows of A . dGn/dth . v (times sg = +/-1) for A 2 x 3 and a homogeneous v: dGn/dth v is linear in v.
+template <int KIND>
+__device__ __forceinline__ void adj_dproj(const double* A, const double* v, double sg, double* du, double* dv)
+{
+    for (int r = 0; r < 2; ++r) {
+        const double* a = A + 3 * r;
+        double* o = r ? dv : du;
+        if (KIND == 0) { o[0] = sg * (a[0] * v[2]); o[1] = sg * (a[1] * v[2]); }
+        else if (KIND == 1) {
+            o[0] = sg * (a[0] * v[0] + a[1] * v[1]);
+            o[1] = sg * (a[1] * v[0] - a[0] * v[1]);
+            o[2] = sg * (a[0] * v[2]);
+            o[3] = sg * (a[1] * v[2]);
+        } else
+            for (int i = 0; i < 8; ++i) o[i] = sg * (a[i / 3] * v[i % 3]);
+    }
+}
+
+// Transfer residual r = pi(p) - b, p = Gn_u^-1 Gn_t a = M a, into q[0..1], and its derivatives into q[2 ..]: with
+// A = dpi/dp . Gn_u^-1, dr/dth_t = A (dGn_t/dth_t) a and dr/dth_u = -A (dGn_u/dth_u) p.  False when p3 <= 0 or r is
+// not finite.
+template <int KIND>
+__device__ __forceinline__ bool adj_transfer(const double* Gi, const double* M, double2 a, double2 b, double* q)
+{
+    constexpr int NP = AdjFam<KIND>::P;
+    const double p[3] = {M[0] * a.x + M[1] * a.y + M[2], M[3] * a.x + M[4] * a.y + M[5], M[6] * a.x + M[7] * a.y + M[8]};
+    const double iw = 1.0 / p[2], U = p[0] * iw, V = p[1] * iw;
+    q[0] = U - b.x;
+    q[1] = V - b.y;
+    double A[6];                                             // dpi/dp = iw [1 0 -U; 0 1 -V]
+    for (int c = 0; c < 3; ++c) {
+        A[c] = iw * (Gi[c] - U * Gi[6 + c]);
+        A[3 + c] = iw * (Gi[3 + c] - V * Gi[6 + c]);
+    }
+    const double av[3] = {a.x, a.y, 1.0};
+    adj_dproj<KIND>(A, av, 1.0, q + 2, q + 2 + NP);
+    adj_dproj<KIND>(A, p, -1.0, q + 2 + 2 * NP, q + 2 + 3 * NP);
+    return p[2] > 0.0 && isfinite(q[0]) && isfinite(q[1]);
+}
+
 // mask points of every link (i < n(l), mask byte != 0)
 __global__ void __launch_bounds__(256) adjust_count_kernel(const Pairs P, const unsigned char* __restrict__ masks, int* __restrict__ npts)
 {
@@ -1075,7 +1120,7 @@ __global__ void __launch_bounds__(256) adjust_init_kernel(int n, int span, AdjGe
         }
         AdjState st;
         st.lambda = -1.0; st.cost = st.cost0 = 0.0;
-        st.first = 1; st.done = 0; st.accepted = 0; st.pad = 0;
+        st.first = 1; st.done = 0; st.accepted = 0; st.nonfinite = 0;
         *state = st;
     }
     __syncthreads();
@@ -1099,10 +1144,13 @@ __global__ void __launch_bounds__(256) adjust_init_kernel(int n, int span, AdjGe
 // One CTA per (link, slice): the slice's share of the link's J^T J blocks, J^T r and cost at x_eval.  A pass stages
 // kAdjThreads correspondences (residual and projection derivatives) in shared memory; thread e then adds entry e of
 // every staged point in index order, so the sums have a fixed order.  Entry e is +/-(a1 b1 + a2 b2) of staged values.
-template <int KIND>
+// COST 0 (mosaic) stages dpi(Gn_u b) / dth_u, so the (t, u) block and J^T r of u are negated; COST 1 (transfer) stages
+// dr / dth_u itself and sets state->nonfinite for a point that makes the cost +inf (state is not __restrict__: the
+// kernel reads state->done and a transfer build writes the flag).
+template <int KIND, int COST>
 __global__ void __launch_bounds__(kAdjThreads) adjust_build_kernel(const Pairs P, const unsigned char* __restrict__ masks, int n,
                                                                    AdjGeom geo, const int* __restrict__ used,
-                                                                   const double* __restrict__ x_eval, const AdjState* __restrict__ state,
+                                                                   const double* __restrict__ x_eval, AdjState* state,
                                                                    double* __restrict__ partial)
 {
     constexpr int NP = AdjFam<KIND>::P, E = AdjFam<KIND>::E, W = AdjFam<KIND>::W;
@@ -1115,6 +1163,15 @@ __global__ void __launch_bounds__(kAdjThreads) adjust_build_kernel(const Pairs P
     nm_link_decode(l, n, t, d);
     double tht[NP], thu[NP];
     for (int i = 0; i < NP; ++i) { tht[i] = x_eval[t * NP + i]; thu[i] = x_eval[(t + d) * NP + i]; }
+    double Gi[9], M[9];                                      // transfer: Gn_u^-1 and Gn_u^-1 Gn_t of this link
+    if constexpr (COST == 1) {
+        double Gt[9], Gu[9];
+        adj_matrix<KIND>(tht, Gt);
+        adj_matrix<KIND>(thu, Gu);
+        nm_inv3d(Gu, nm_det3d(Gu), Gi);
+        for (int r = 0; r < 3; ++r)
+            for (int c = 0; c < 3; ++c) M[r * 3 + c] = Gi[r * 3] * Gt[c] + Gi[r * 3 + 1] * Gt[3 + c] + Gi[r * 3 + 2] * Gt[6 + c];
+    }
     // entries owned by this thread: (a1, b1, a2, b2, negate)
     int ea[NE][4];
     bool neg[NE];
@@ -1125,9 +1182,9 @@ __global__ void __launch_bounds__(kAdjThreads) adjust_build_kernel(const Pairs P
         const int ot = 2, ovt = 2 + NP, ou = 2 + 2 * NP, ovu = 2 + 3 * NP;    // du_t, dv_t, du_u, dv_u
         if (e < NP * NP) { const int i = e / NP, j = e % NP; a1 = ot + i; b1 = ot + j; a2 = ovt + i; b2 = ovt + j; }
         else if (e < 2 * NP * NP) { const int i = (e - NP * NP) / NP, j = e % NP; a1 = ou + i; b1 = ou + j; a2 = ovu + i; b2 = ovu + j; }
-        else if (e < 3 * NP * NP) { const int i = (e - 2 * NP * NP) / NP, j = e % NP; a1 = ot + i; b1 = ou + j; a2 = ovt + i; b2 = ovu + j; ng = true; }
+        else if (e < 3 * NP * NP) { const int i = (e - 2 * NP * NP) / NP, j = e % NP; a1 = ot + i; b1 = ou + j; a2 = ovt + i; b2 = ovu + j; ng = COST == 0; }
         else if (e < 3 * NP * NP + NP) { const int i = e - 3 * NP * NP; a1 = ot + i; b1 = 0; a2 = ovt + i; b2 = 1; }
-        else if (e < 3 * NP * NP + 2 * NP) { const int i = e - 3 * NP * NP - NP; a1 = ou + i; b1 = 0; a2 = ovu + i; b2 = 1; ng = true; }
+        else if (e < 3 * NP * NP + 2 * NP) { const int i = e - 3 * NP * NP - NP; a1 = ou + i; b1 = 0; a2 = ovu + i; b2 = 1; ng = COST == 0; }
         ea[r][0] = a1; ea[r][1] = b1; ea[r][2] = a2; ea[r][3] = b2;
         neg[r] = ng;
     }
@@ -1137,17 +1194,21 @@ __global__ void __launch_bounds__(kAdjThreads) adjust_build_kernel(const Pairs P
     const int lo = slice * len, hi = min(cnt, lo + len);
     const long long off = (long long)l * P.stride;
     const unsigned char* __restrict__ mask = masks + (long long)l * P.max_pts;
+    bool bad = false;
     for (int base = lo; base < hi; base += kAdjThreads) {
         const int i = base + tid;
         const bool ok = i < hi && mask[i] != 0;
         if (ok) {
             double* q = sp + tid * W;
             const double2 a = geo.norm(P.sx[off + i], P.sy[off + i]), b = geo.norm(P.dx[off + i], P.dy[off + i]);
-            double Ut, Vt, Uu, Vu;
-            adj_project<KIND>(tht, a.x, a.y, Ut, Vt, q + 2, q + 2 + NP);
-            adj_project<KIND>(thu, b.x, b.y, Uu, Vu, q + 2 + 2 * NP, q + 2 + 3 * NP);
-            q[0] = Ut - Uu;
-            q[1] = Vt - Vu;
+            if constexpr (COST == 0) {
+                double Ut, Vt, Uu, Vu;
+                adj_project<KIND>(tht, a.x, a.y, Ut, Vt, q + 2, q + 2 + NP);
+                adj_project<KIND>(thu, b.x, b.y, Uu, Vu, q + 2 + 2 * NP, q + 2 + 3 * NP);
+                q[0] = Ut - Uu;
+                q[1] = Vt - Vu;
+            } else if (!adj_transfer<KIND>(Gi, M, a, b, q))
+                bad = true;
         }
         sv[tid] = ok;
         __syncthreads();
@@ -1164,10 +1225,13 @@ __global__ void __launch_bounds__(kAdjThreads) adjust_build_kernel(const Pairs P
         const int e = tid + r * kAdjThreads;
         if (e < E) partial[((long long)l * kAdjSlices + slice) * E + e] = neg[r] ? -acc[r] : acc[r];
     }
+    if constexpr (COST == 1)
+        if (bad) state->nonfinite = 1;
 }
 
-// One CTA: the Levenberg-Marquardt step.  Link totals (slices in order), the cost at x_eval (links in index order);
-// x_eval is accepted when it is the first point or lowers the cost (lambda / 10), else rejected (lambda * 10).  After an
+// One CTA: the Levenberg-Marquardt step.  Link totals (slices in order), the cost at x_eval (links in index order, +inf
+// when the build flagged a point); x_eval is accepted when it is the first point or lowers the cost (lambda / 10), else
+// rejected (lambda * 10).  A +inf cost at the first point ends the run there: the window keeps its initial poses.  After an
 // acceptance the banded normal equations of the unknowns (frame-major, half-bandwidth bw = P (span + 1) - 1; a
 // disconnected frame's rows are the identity with zero right-hand side) are assembled in link index order.  Unless the
 // run is over, (J^T J + lambda I) delta = -J^T r is solved by a banded Cholesky factorisation -- the last bw + 1 rows of
@@ -1203,8 +1267,9 @@ __global__ void __launch_bounds__(kAdjSolveThreads) adjust_solve_kernel(int n, i
         for (int l = 0; l < L; ++l)
             if (used[l]) c += link_tot[(long long)l * E + E - 1];
         AdjState st = *state;
+        if (st.nonfinite) c = INFINITY;
         bool accept = false;
-        if (st.first) { accept = true; st.cost0 = c; st.first = 0; }
+        if (st.first) { accept = true; st.cost0 = c; st.first = 0; if (st.nonfinite) st.done = 1; }
         else if (c < st.cost) {
             accept = true;
             if (st.cost - c < 1e-12 * st.cost) st.done = 1;
@@ -1215,6 +1280,7 @@ __global__ void __launch_bounds__(kAdjSolveThreads) adjust_solve_kernel(int n, i
             if (st.lambda > 1e16) st.done = 1;
         }
         if (accept) st.cost = c;
+        st.nonfinite = 0;
         *state = st;
         s_accept = accept;
         s_stop = st.done || last;
@@ -1405,9 +1471,9 @@ __global__ void __launch_bounds__(256) adjust_finish_kernel(const Pairs P, float
 }
 
 template <int KIND>
-int adjust_chain(const Pairs& P, float thr, int n, int span, int fw, int fh, const unsigned char* masks, const float* H_links,
-                 const int* link_status, int iterations, float* H_out, int* status_out, double* chain_out, double* report,
-                 cudaStream_t st)
+int adjust_chain(const Pairs& P, int cost, float thr, int n, int span, int fw, int fh, const unsigned char* masks,
+                 const float* H_links, const int* link_status, int iterations, float* H_out, int* status_out, double* chain_out,
+                 double* report, cudaStream_t st)
 {
     constexpr int NP = AdjFam<KIND>::P, E = AdjFam<KIND>::E;
     const int L = nm_span_links(n, span), m = (n - 1) * NP, bw1 = NP * (span + 1);
@@ -1443,7 +1509,10 @@ int adjust_chain(const Pairs& P, float thr, int n, int span, int fw, int fh, con
     adjust_count_kernel<<<L, 256, 0, st>>>(P, masks, npts);
     adjust_init_kernel<KIND><<<1, 256, 0, st>>>(n, span, geo, H_links, link_status, npts, G, conn, used, x_cur, x_eval, state);
     for (int it = 0; it < iterations; ++it) {
-        adjust_build_kernel<KIND><<<dim3(L, kAdjSlices), kAdjThreads, 0, st>>>(P, masks, n, geo, used, x_eval, state, partial);
+        if (cost == NM_ADJUST_MOSAIC)
+            adjust_build_kernel<KIND, 0><<<dim3(L, kAdjSlices), kAdjThreads, 0, st>>>(P, masks, n, geo, used, x_eval, state, partial);
+        else
+            adjust_build_kernel<KIND, 1><<<dim3(L, kAdjSlices), kAdjThreads, 0, st>>>(P, masks, n, geo, used, x_eval, state, partial);
         adjust_solve_kernel<KIND><<<1, kAdjSolveThreads, smem, st>>>(n, span, used, conn, partial, link_tot, A, rhs, U, x_cur, x_eval,
                                                                      state, it == iterations - 1);
     }
@@ -1589,23 +1658,36 @@ extern "C" int nm_ransac_refine_batch_f32(int kind, const float* src_x, const fl
     return NM_OK;
 }
 
+extern "C" int nm_ransac_adjust_chain_cost_f32(int kind, int cost, const float* src_x, const float* src_y, const float* dst_x,
+                                               const float* dst_y, long long pair_stride, const int* counts, int max_pts,
+                                               float inlier_threshold, int n_frames, int span, int frame_w, int frame_h,
+                                               const unsigned char* masks, const float* H_links, const int* link_status,
+                                               int iterations, float* H_out, int* status_out, double* chain_out, double* report_out,
+                                               nm_stream_t stream)
+{
+    if (kind < 0 || kind > 2 || max_pts <= 0 || pair_stride < 0 || iterations < 1 || frame_w <= 0 || frame_h <= 0) return NM_ERR_INVALID;
+    if (cost != NM_ADJUST_MOSAIC && cost != NM_ADJUST_TRANSFER) return NM_ERR_INVALID;
+    if (n_frames < 2 || n_frames > kAdjMaxFrames || span < 1 || span > kAdjMaxSpan || span >= n_frames) return NM_ERR_INVALID;
+    if (!src_x || !src_y || !dst_x || !dst_y || !masks || !H_links || !link_status || !H_out || !status_out) return NM_ERR_INVALID;
+    const Pairs P{src_x, src_y, dst_x, dst_y, pair_stride, counts, max_pts};
+    const cudaStream_t st = (cudaStream_t)stream;
+    if (kind == 0)
+        return adjust_chain<0>(P, cost, inlier_threshold, n_frames, span, frame_w, frame_h, masks, H_links, link_status, iterations,
+                               H_out, status_out, chain_out, report_out, st);
+    if (kind == 1)
+        return adjust_chain<1>(P, cost, inlier_threshold, n_frames, span, frame_w, frame_h, masks, H_links, link_status, iterations,
+                               H_out, status_out, chain_out, report_out, st);
+    return adjust_chain<2>(P, cost, inlier_threshold, n_frames, span, frame_w, frame_h, masks, H_links, link_status, iterations,
+                           H_out, status_out, chain_out, report_out, st);
+}
+
 extern "C" int nm_ransac_adjust_chain_f32(int kind, const float* src_x, const float* src_y, const float* dst_x, const float* dst_y,
                                           long long pair_stride, const int* counts, int max_pts, float inlier_threshold,
                                           int n_frames, int span, int frame_w, int frame_h, const unsigned char* masks,
                                           const float* H_links, const int* link_status, int iterations, float* H_out,
                                           int* status_out, double* chain_out, double* report_out, nm_stream_t stream)
 {
-    if (kind < 0 || kind > 2 || max_pts <= 0 || pair_stride < 0 || iterations < 1 || frame_w <= 0 || frame_h <= 0) return NM_ERR_INVALID;
-    if (n_frames < 2 || n_frames > kAdjMaxFrames || span < 1 || span > kAdjMaxSpan || span >= n_frames) return NM_ERR_INVALID;
-    if (!src_x || !src_y || !dst_x || !dst_y || !masks || !H_links || !link_status || !H_out || !status_out) return NM_ERR_INVALID;
-    const Pairs P{src_x, src_y, dst_x, dst_y, pair_stride, counts, max_pts};
-    const cudaStream_t st = (cudaStream_t)stream;
-    if (kind == 0)
-        return adjust_chain<0>(P, inlier_threshold, n_frames, span, frame_w, frame_h, masks, H_links, link_status, iterations, H_out,
-                               status_out, chain_out, report_out, st);
-    if (kind == 1)
-        return adjust_chain<1>(P, inlier_threshold, n_frames, span, frame_w, frame_h, masks, H_links, link_status, iterations, H_out,
-                               status_out, chain_out, report_out, st);
-    return adjust_chain<2>(P, inlier_threshold, n_frames, span, frame_w, frame_h, masks, H_links, link_status, iterations, H_out,
-                           status_out, chain_out, report_out, st);
+    return nm_ransac_adjust_chain_cost_f32(kind, NM_ADJUST_MOSAIC, src_x, src_y, dst_x, dst_y, pair_stride, counts, max_pts,
+                                           inlier_threshold, n_frames, span, frame_w, frame_h, masks, H_links, link_status,
+                                           iterations, H_out, status_out, chain_out, report_out, stream);
 }

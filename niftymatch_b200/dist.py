@@ -9,6 +9,8 @@
 """
 from __future__ import annotations
 
+from .ransac import MOSAIC
+
 
 def shard_bounds(n: int, world: int, rank: int):
     """Contiguous range [lo, hi) of shard `rank` out of `world` over n items; the first
@@ -132,15 +134,17 @@ class StreamRegistrar:
 
     span > 1 (at most 8) registers every frame t of a chunk also to t + 2 ... t + span and adjusts the chunk's poses
     jointly: each chunk [c0, c1) is one adjustment window of the span layout (span min(span, c1 - c0 - 1)), run as
-    match_pairs_span, align_pairs_span, one ransac_batch per d (link (t, d), t in stream coordinates, draws with
-    seed + t + ((d - 1) << 40)), refine_batch on all links (rounds = refine_rounds, 0 = masks only) and adjust_chain, whose
+    match_pairs_span, align_pairs_span, one ransac_batch per d (link (t, d), t in stream coordinates, draws with seed +
+    t + ((d - 1) << 40)), refine_batch on all links (rounds = refine_rounds, 0 = masks only) and adjust_chain, whose
     pairwise models and status [connected, inliers, LM steps accepted] are returned (status[:, 2] counts LM steps here,
-    not refits kept; adjust_iterations bounds the LM builds per window).  A frame that no usable link reaches
-    keeps its predecessor's pose (status 0).  The result then depends on the window boundaries -- lo and the chunk
-    size -- and on nothing else.  span = 1 calls nothing new."""
+    not refits kept; adjust_iterations bounds the LM builds per window; adjust_cost is adjust_chain's residual: MOSAIC,
+    the default, or TRANSFER, which keeps long windows of similarity or homography models from contracting).  A frame
+    that no usable link reaches keeps its predecessor's pose (status 0).  The result then depends on the window
+    boundaries -- lo and the chunk size -- and on nothing else.  span = 1 calls nothing new."""
 
     def __init__(self, sift_batch, chunk=None, kind: int = 2, ambiguity: float = 0.8, inlier_threshold: float = 4.0,
-                 iterations: int = 1024, seed: int = 0, refine_rounds: int = 0, span: int = 1, adjust_iterations: int = 10):
+                 iterations: int = 1024, seed: int = 0, refine_rounds: int = 0, span: int = 1, adjust_iterations: int = 10,
+                 adjust_cost: int = MOSAIC):
         import torch
         self.sb = sift_batch
         self.chunk = min(chunk or sift_batch.max_batch, sift_batch.max_batch)
@@ -148,7 +152,7 @@ class StreamRegistrar:
         self.kind, self.ambiguity, self.thr, self.iters, self.seed = kind, ambiguity, inlier_threshold, iterations, seed
         self.refine_rounds = refine_rounds
         assert 1 <= span <= 8
-        self.span, self.adjust_iterations = span, adjust_iterations
+        self.span, self.adjust_iterations, self.adjust_cost = span, adjust_iterations, adjust_cost
         cap, n = sift_batch.capacity, self.chunk - 1
         dev = torch.device("cuda", torch.cuda.current_device())
         self.match = torch.empty((n, cap), dtype=torch.int32, device=dev)
@@ -186,7 +190,7 @@ class StreamRegistrar:
             if self.span > 1:
                 adjust_window(r, n, min(self.span, n - 1), chunk.shape[2], chunk.shape[1], self.kind, self.ambiguity, self.thr,
                               self.iters, self.seed + c0, self.refine_rounds, out=(H[k: k + n - 1], st[k: k + n - 1]),
-                              adjust_iterations=self.adjust_iterations)
+                              adjust_iterations=self.adjust_iterations, adjust_cost=self.adjust_cost)
                 c0 = c1 - 1
                 continue
             self.match[: n - 1].fill_(-1)
@@ -206,10 +210,11 @@ class StreamRegistrar:
 
 
 def adjust_window(res, n, span, frame_w, frame_h, kind, ambiguity, inlier_threshold, iterations, seed, refine_rounds, out,
-                  adjust_iterations: int = 10):
+                  adjust_iterations: int = 10, adjust_cost: int = MOSAIC):
     """One adjustment window of StreamRegistrar(span > 1): frames 0 .. n-1 of the SIFT results `res` (SiftBatch.results())
     through the five public calls.  seed = the stream seed + the window's first frame.  Writes the window's n - 1 pairwise
-    models and status into out = (H, status); returns adjust_chain's (H, status, chain, report)."""
+    models and status into out = (H, status); returns adjust_chain's (H, status, chain, report).  adjust_cost: adjust_chain's
+    cost (MOSAIC or TRANSFER)."""
     import torch
     from .match import match_pairs_span, link_row
     from .ransac import align_pairs_span, ransac_batch, refine_batch, adjust_chain
@@ -225,4 +230,5 @@ def adjust_window(res, n, span, frame_w, frame_h, kind, ambiguity, inlier_thresh
         SL.append(Sd)
     link_counts = torch.cat([counts[: n - d] for d in range(1, span + 1)])
     HL, SL, mask = refine_batch(kind, *corr, link_counts, torch.cat(HL), torch.cat(SL), inlier_threshold, refine_rounds)
-    return adjust_chain(kind, *corr, link_counts, span, mask, HL, SL, frame_w, frame_h, inlier_threshold, adjust_iterations, out=out)
+    return adjust_chain(kind, *corr, link_counts, span, mask, HL, SL, frame_w, frame_h, inlier_threshold, adjust_iterations, out=out,
+                        cost=adjust_cost)

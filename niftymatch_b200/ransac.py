@@ -10,6 +10,7 @@ from ._lib import check
 from .sift import _stream_ptr
 
 TRANSLATION, SIMILARITY, HOMOGRAPHY = 0, 1, 2
+MOSAIC, TRANSFER = 0, 1          # residual of adjust_chain: NM_ADJUST_MOSAIC, NM_ADJUST_TRANSFER
 
 
 def _p(t):
@@ -144,15 +145,19 @@ def refine(kind, src_x, src_y, dst_x, dst_y, H, status, inlier_threshold, rounds
 
 
 def adjust_chain(kind, src_x, src_y, dst_x, dst_y, counts, span, masks, H, link_status, frame_w, frame_h, inlier_threshold,
-                 iterations=10, out=None):
-    """nm_ransac_adjust_chain_f32 (arguments in its order): joint least-squares adjustment of the poses of a window of n
-    frames from the links of its span layout.  src_x ... dst_y (L, max_pts) and counts (L,) or None as for refine_batch;
-    masks (L, max_pts) bool, H (L, 9) the link models and link_status (L, 3), as refine_batch returns them (rows 0 .. n-2
-    are the consecutive pairs).  inlier_threshold: the RANSAC rule that counts status[:, 1].  out = (H_out, status_out), (n - 1, 9) and
-    (n - 1, 3): written there (they may be H[: n - 1] and link_status[: n - 1]).  Returns (H (n - 1, 9) pairwise models that
-    nm_mosaic_place_f32 chains into the adjusted poses, status (n - 1, 3) = [frame p + 1 connected, inliers, LM steps
-    accepted], chain (n, 9) float64 frame -> frame-0 transforms, report (4,) float64 = [mean squared residual before,
-    after (px^2), residual points, links used])."""
+                 iterations=10, out=None, cost=MOSAIC):
+    """nm_ransac_adjust_chain_cost_f32 (arguments in the order of nm_ransac_adjust_chain_f32, then cost): joint
+    least-squares adjustment of the poses of a window of n frames from the links of its span layout.  src_x ... dst_y
+    (L, max_pts) and counts (L,) or None as for refine_batch; masks (L, max_pts) bool, H (L, 9) the link models and
+    link_status (L, 3), as refine_batch returns them (rows 0 .. n-2 are the consecutive pairs).  inlier_threshold: the
+    RANSAC rule that counts status[:, 1].  out = (H_out, status_out), (n - 1, 9) and (n - 1, 3): written there (they may
+    be H[: n - 1] and link_status[: n - 1]).  Returns (H (n - 1, 9) pairwise models that nm_mosaic_place_f32 chains into
+    the adjusted poses, status (n - 1, 3) = [frame p + 1 connected, inliers, LM steps accepted], chain (n, 9) float64
+    frame -> frame-0 transforms, report (4,) float64 = [mean squared residual before, after (px^2), residual points,
+    links used]).  cost: MOSAIC (the default, nm_ransac_adjust_chain_f32) measures a link's residual in frame-0 pixels,
+    TRANSFER in the pixels of its target frame t + d, which does not reward shrinking the frames far from frame 0 (long
+    windows of similarity or homography models).  With TRANSFER a point behind the target camera at the initial poses
+    leaves the window unadjusted (report costs +inf)."""
     import torch
     _f32(src_x, src_y, dst_x, dst_y)
     if counts is not None:
@@ -178,8 +183,9 @@ def adjust_chain(kind, src_x, src_y, dst_x, dst_y, counts, span, masks, H, link_
             raise TypeError("status_out: expected shape (n - 1, 3)")
     chain = torch.empty((n, 9), dtype=torch.float64, device=H.device)
     report = torch.empty(4, dtype=torch.float64, device=H.device)
-    check(_lib.load().nm_ransac_adjust_chain_f32(kind, _p(src_x), _p(src_y), _p(dst_x), _p(dst_y), max_pts,
-                                                 _p(counts) if counts is not None else None, max_pts, inlier_threshold, n, span,
-                                                 frame_w, frame_h, _p(masks), _p(H), _p(link_status), iterations, _p(H_out),
-                                                 _p(st_out), _p(chain), _p(report), _stream_ptr()), "nm_ransac_adjust_chain_f32")
+    check(_lib.load().nm_ransac_adjust_chain_cost_f32(kind, cost, _p(src_x), _p(src_y), _p(dst_x), _p(dst_y), max_pts,
+                                                      _p(counts) if counts is not None else None, max_pts, inlier_threshold, n,
+                                                      span, frame_w, frame_h, _p(masks), _p(H), _p(link_status), iterations,
+                                                      _p(H_out), _p(st_out), _p(chain), _p(report), _stream_ptr()),
+          "nm_ransac_adjust_chain_cost_f32")
     return H_out, st_out, chain, report

@@ -6,11 +6,11 @@ refit rounds (64 pairs x 8 192 correspondences, 70 % inliers, 1 024 hypotheses; 
 alternating windows), corner error against the ground truth of the RANSAC model, the refit and a float64 fit to the
 true inliers, and the 2 048-frame 1080p StreamRegistrar rate of bench.py with refine_rounds 0 and 2.
 
---adjust: the skip-link leg (nm_match_pairs_span_f32 ... nm_ransac_adjust_chain_f32): time per 64-frame 1080p window of
-each stage at span 1, 2, 3 (the frames of bench.py's stream, CUDA events, the spans in alternating windows), the
-2 048-frame 1080p StreamRegistrar rate at span 1, 2, 3 with refine_rounds 0 and 2, and the last frame's corner error on
-the synthetic 64-frame windows of tests/test_gpu_chain_adjust.py for chained span-1 refits and the span-2 / span-3
-adjustment."""
+--adjust: the skip-link leg (nm_match_pairs_span_f32 ... nm_ransac_adjust_chain_cost_f32): time per 64-frame 1080p
+window of each stage at span 1, 2, 3 (the frames of bench.py's stream, CUDA events, the spans in alternating windows),
+the adjustment with the mosaic and the transfer cost, the 2 048-frame 1080p StreamRegistrar rate at span 1, 2, 3 with
+refine_rounds 0 and 2 (span 3 with either cost), and the last frame's corner error on the synthetic 64-frame windows of
+tests/test_gpu_chain_adjust.py for chained span-1 refits and the span-2 / span-3 adjustment with either cost."""
 import os
 import subprocess
 import sys
@@ -138,8 +138,9 @@ def adjust_leg():
         elif name == "refine":
             state["H"], state["S"], state["k"] = nm.refine_batch(kind, *state["c"], state["lc"], state["H"], state["S"], thr, 2)
         else:
-            nm.adjust_chain(kind, *state["c"], state["lc"], span, state["k"], state["H"], state["S"], bench.W, bench.H, thr)
-    names = ("match", "align", "ransac", "refine", "adjust")
+            nm.adjust_chain(kind, *state["c"], state["lc"], span, state["k"], state["H"], state["S"], bench.W, bench.H, thr,
+                            cost=nm.TRANSFER if name == "adjust (transfer)" else nm.MOSAIC)
+    names = ("match", "align", "ransac", "refine", "adjust", "adjust (transfer)")
     times = {(s, k): [] for s in (1, 2, 3) for k in names}
     for rep in range(6):
         for span in (1, 2, 3):
@@ -152,15 +153,15 @@ def adjust_leg():
                 if rep >= 1:
                     times[(span, k)].append(e0.elapsed_time(e1))
     for span in (1, 2, 3):
-        tot = sum(np.median(times[(span, k)]) for k in names)
+        tot = sum(np.median(times[(span, k)]) for k in names[:-1])
         print(f"span {span}, one 64-frame 1080p window: " + ", ".join(f"{k} {np.median(times[(span, k)]):.2f} ms" for k in names)
-              + f"; sum {tot:.2f} ms")
+              + f"; sum with the mosaic cost {tot:.2f} ms")
     # the stream leg of bench.py
     n_stream = 2048
     for rep in range(2):
-        for span in (1, 2, 3):
+        for span, cost in ((1, nm.MOSAIC), (2, nm.MOSAIC), (3, nm.MOSAIC), (3, nm.TRANSFER)):
             for rounds in (0, 2):
-                reg = StreamRegistrar(sb, chunk=sb.max_batch, refine_rounds=rounds, span=span)
+                reg = StreamRegistrar(sb, chunk=sb.max_batch, refine_rounds=rounds, span=span, adjust_cost=cost)
                 reg.run(frames_of, 0, sb.max_batch + 1)
                 torch.cuda.synchronize()
                 e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
@@ -169,14 +170,15 @@ def adjust_leg():
                 e1.record()
                 torch.cuda.synchronize()
                 ms = e0.elapsed_time(e1)
-                print(f"stream {n_stream} frames 1080p, span {span}, refine_rounds {rounds}: {n_stream / ms * 1e3:.0f} frames/s "
+                print(f"stream {n_stream} frames 1080p, span {span}{' (transfer cost)' if cost else ''}, refine_rounds {rounds}: "
+                      f"{n_stream / ms * 1e3:.0f} frames/s "
                       f"({ms:.1f} ms), connected pairs {int((sts[:, 0] == 1).sum())}")
     sb.close()
     # synthetic accuracy: windows of synth.span_window through RANSAC per d (link seeds as StreamRegistrar) and 2 refits
     w, h, n, thr = 640, 480, 64, 4.0
     c = np.array([[0, 0], [w - 1, 0], [0, h - 1], [w - 1, h - 1]], np.float64)
     for kind in (0, 1, 2):
-        e = {1: [], 2: [], 3: []}
+        e = {1: [], (2, 0): [], (3, 0): [], (2, 1): [], (3, 1): []}
         for wnd in range(4):
             seed = 90 + 10 * wnd + kind
             G, arrs = span_window(kind, n, 3, w, h, 2000, seed)
@@ -188,11 +190,15 @@ def adjust_leg():
             e[1].append(last(nm.place(HL[: n - 1].contiguous(), SL[: n - 1].contiguous(), w, h).chain.cpu().numpy().reshape(n, 3, 3)))
             for span in (2, 3):                  # the span-2 layout is the first rows of the span-3 one
                 L = span * n - span * (span + 1) // 2
-                _, _, chain, _ = nm.adjust_chain(kind, *[a[:L] for a in d_], None, span, mask[:L], HL[:L], SL[:L], w, h, thr)
-                e[span].append(last(chain.cpu().numpy().reshape(n, 3, 3)))
+                for cost in (nm.MOSAIC, nm.TRANSFER):
+                    _, _, chain, _ = nm.adjust_chain(kind, *[a[:L] for a in d_], None, span, mask[:L], HL[:L], SL[:L], w, h, thr,
+                                                     cost=cost)
+                    e[span, cost].append(last(chain.cpu().numpy().reshape(n, 3, 3)))
         m = {k: float(np.mean(v)) for k, v in e.items()}
-        print(f"synthetic 64-frame windows (4), kind {kind}: last frame mean corner error, chained span-1 refits "
-              f"{m[1]:.4f} px, span 2 {m[2]:.4f} px ({m[2] / m[1]:.3f}), span 3 {m[3]:.4f} px ({m[3] / m[1]:.3f})")
+        for cost, name in ((nm.MOSAIC, "mosaic"), (nm.TRANSFER, "transfer")):
+            print(f"synthetic 64-frame windows (4), kind {kind}, {name} cost: last frame mean corner error, chained span-1 "
+                  f"refits {m[1]:.4f} px, span 2 {m[2, cost]:.4f} px ({m[2, cost] / m[1]:.3f}), span 3 {m[3, cost]:.4f} px "
+                  f"({m[3, cost] / m[1]:.3f})")
 
 
 if "--adjust" in sys.argv:
