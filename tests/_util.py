@@ -223,6 +223,26 @@ def load_oracle():
     return FrameChecker(C.CDLL(ORACLE_SO), "orc")
 
 
+def orc_orientations(lib, kp, grad, xper=1.0):
+    """orc_orientations (public-API semantics, window clamp 10) on a (levels, oh, ow, 2) gradient buffer."""
+    kp, grad = np.ascontiguousarray(kp, np.float32), np.ascontiguousarray(grad, np.float32)
+    res = np.full((len(kp), 2), -1, np.float32)
+    lib.orc_orientations(_p(kp), _p(grad), len(kp), grad.shape[2], grad.shape[1], C.c_float(1.5), C.c_float(xper),
+                         _p(res), 10)
+    return res
+
+
+def orc_descriptors(lib, kp, orient, grad, num_dogs=3, xper=1.0):
+    """orc_descriptors on a (levels, oh, ow, 2) gradient buffer: desc (n, 128), x, y (zeros where :49 fails)."""
+    kp, grad = np.ascontiguousarray(kp, np.float32), np.ascontiguousarray(grad, np.float32)
+    orient = np.ascontiguousarray(orient, np.float32)
+    n = len(kp)
+    desc, x, y = np.zeros((n, 128), np.float32), np.zeros(n, np.float32), np.zeros(n, np.float32)
+    lib.orc_descriptors(_p(kp), _p(orient), _p(grad), n, grad.shape[2], grad.shape[1], num_dogs, C.c_float(xper),
+                        _p(desc), _p(x), _p(y))
+    return desc, x, y
+
+
 def load_reflib():
     if not os.path.exists(REF_SO):
         return None
