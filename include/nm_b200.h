@@ -427,6 +427,30 @@ int nm_ransac_adjust_chain_cost_f32(int kind, int cost, const float* src_x, cons
                                     const unsigned char* masks, const float* H_links, const int* link_status, int iterations,
                                     float* H_out, int* status_out, double* chain_out, double* report_out, nm_stream_t stream);
 
+/* nm_ransac_adjust_chain_cost_f32 with the poses of frames 0 .. n_fixed-1 held fixed, 1 <= n_fixed <= n_frames - 1: a
+ * window that overlaps the end of an adjusted one is adjusted against that one's poses, so the links that cross the
+ * window boundary are used, and a live session can append frames to a chain it has already shown.
+ *   fixed_chain [n_fixed][9] device doubles: row j maps frame j into any common frame (for example chain_out rows of the
+ *     previous window, chain_out + (n_prev - n_fixed) * 9).  It is rebased on the device: F_j = C_0^-1 C_j, renormalised.
+ *   fixed_conn [n_fixed] device ints, or NULL = all connected; entry 0 is ignored (frame 0 is the gauge).  A fixed frame
+ *     j >= 1 is fixed and disconnected (its links unused, G_j = G_(j-1)) when fixed_conn[j] == 0, when F_j is not finite,
+ *     or when C_0 is not finite or singular (|det| <= 1e-12 max|C_0|^3).  With n_fixed == 1 neither array is read.
+ *   Initial poses: fixed frames take F_j; a free frame k >= n_fixed takes the rule of nm_ransac_adjust_chain_f32 (frame
+ *     k - d may be a fixed frame).  Links used: that rule, and the later frame t + d must be free (a link between two
+ *     fixed frames is constant).  Unknowns: the connected free frames; the rows of a fixed frame are the identity with
+ *     zero right-hand side, like those of a disconnected frame, and lambda0 is taken over the free rows.
+ *   Outputs as nm_ransac_adjust_chain_cost_f32 for every pair and frame: pairs inside the fixed part come from the fixed
+ *     poses, chain_out of a connected fixed frame is F_j up to the rounding of the parameter round trip, and the report
+ *     covers the links used.
+ * n_fixed < 1, n_fixed >= n_frames, or fixed_chain NULL with n_fixed > 1: NM_ERR_INVALID.  No host synchronisation (the
+ * call can be captured in a CUDA graph), bit-reproducible; nm_ransac_adjust_chain_cost_f32 is n_fixed = 1 of it. */
+int nm_ransac_adjust_chain_fixed_f32(int kind, int cost, const float* src_x, const float* src_y, const float* dst_x,
+                                     const float* dst_y, long long pair_stride, const int* counts, int max_pts,
+                                     float inlier_threshold, int n_frames, int span, int frame_w, int frame_h,
+                                     const unsigned char* masks, const float* H_links, const int* link_status, int n_fixed,
+                                     const double* fixed_chain, const int* fixed_conn, int iterations, float* H_out,
+                                     int* status_out, double* chain_out, double* report_out, nm_stream_t stream);
+
 /* ------------------------------------------------------------------------ */
 /* Batched SIFT detect+describe: the client loop of the reference             */
 /* (compute_dog/_gradients/_keypoints/_orientations/_descriptors,             */

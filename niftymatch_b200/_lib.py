@@ -90,6 +90,8 @@ SIGNATURES = {
                                         _vp, _vp, _vp, _vp, _vp]),
     "nm_ransac_adjust_chain_cost_f32": (_i, [_i, _i, _vp, _vp, _vp, _vp, C.c_longlong, _vp, _i, _f, _i, _i, _i, _i, _vp, _vp, _vp,
                                              _i, _vp, _vp, _vp, _vp, _vp]),
+    "nm_ransac_adjust_chain_fixed_f32": (_i, [_i, _i, _vp, _vp, _vp, _vp, C.c_longlong, _vp, _i, _f, _i, _i, _i, _i, _vp, _vp, _vp,
+                                              _i, _vp, _vp, _i, _vp, _vp, _vp, _vp, _vp]),
     "nm_match_set_engine": (_i, [_i]),
     "nm_match_get_engine": (_i, []),
     "nm_sift_create": (_i, [C.POINTER(_vp), C.POINTER(SiftParamsC), _i, _i]),

@@ -1084,14 +1084,19 @@ __global__ void __launch_bounds__(256) adjust_count_kernel(const Pairs P, const 
     if (threadIdx.x == 0) npts[l] = tot;
 }
 
-// One CTA.  Initial poses: for k = 1 .. n-1 the smallest d <= span with frame k-d connected and link (k-d, d) usable
-// (status 1, at least M mask points) gives G_k = G_(k-d) . step(H_link) (nm_chain_step, renormalised: place_kernel's
-// chain); without one frame k is disconnected and G_k = G_(k-1).  Then the parameters of N G_k N^-1, the links used,
-// and the LM state.
+// One CTA.  Fixed frames j = 1 .. nf-1 (nf = n_fixed): G_j = C_0^-1 C_j of fixed_chain, renormalised; frame j is
+// disconnected (G_j = G_(j-1)) when fixed_conn[j] == 0, G_j is not finite, or C_0 is not finite or singular (|det| <=
+// 1e-12 max|C_0|^3, nm_chain_step's rule).  Initial poses of the free frames: for k = nf .. n-1 the smallest d <= span
+// with frame k-d connected and link (k-d, d) usable (status 1, at least M mask points) gives G_k = G_(k-d) .
+// step(H_link) (nm_chain_step, renormalised: place_kernel's chain); without one frame k is disconnected and G_k =
+// G_(k-1).  Then the parameters of N G_k N^-1, the links used (both frames connected, the later one free), and the LM
+// state.
 template <int KIND>
 __global__ void __launch_bounds__(256) adjust_init_kernel(int n, int span, AdjGeom geo, const float* __restrict__ H_links,
                                                           const int* __restrict__ link_status, const int* __restrict__ npts,
-                                                          double* __restrict__ G, int* __restrict__ conn, int* __restrict__ used,
+                                                          int nf, const double* __restrict__ fixed_chain,
+                                                          const int* __restrict__ fixed_conn, double* __restrict__ G,
+                                                          int* __restrict__ conn, int* __restrict__ used,
                                                           double* __restrict__ x_cur, double* __restrict__ x_eval, AdjState* state)
 {
     constexpr int NP = AdjFam<KIND>::P, M = AdjFam<KIND>::M;
@@ -1100,7 +1105,31 @@ __global__ void __launch_bounds__(256) adjust_init_kernel(int n, int span, AdjGe
     if (tid == 0) {
         for (int i = 0; i < 9; ++i) G[i] = (i % 4 == 0) ? 1.0 : 0.0;
         conn[0] = 1;
-        for (int k = 1; k < n; ++k) {
+        if (nf > 1) {
+            double c0[9], c0i[9];
+            bool base = true;
+            for (int i = 0; i < 9; ++i) { c0[i] = fixed_chain[i]; base = base && isfinite(c0[i]); }
+            if (base) {
+                const double m = nm_max_abs9(c0), det = nm_det3d(c0);
+                base = fabs(det) > 1e-12 * m * m * m;
+                if (base) nm_inv3d(c0, det, c0i);
+            }
+            for (int j = 1; j < nf; ++j) {
+                const double* c = fixed_chain + (long long)j * 9;
+                double g[9];
+                bool ok = base && (fixed_conn == nullptr || fixed_conn[j] != 0);
+                if (ok) {
+                    for (int row = 0; row < 3; ++row)
+                        for (int col = 0; col < 3; ++col)
+                            g[row * 3 + col] = c0i[row * 3] * c[col] + c0i[row * 3 + 1] * c[3 + col] + c0i[row * 3 + 2] * c[6 + col];
+                    nm_renormalise(g);
+                    for (int i = 0; i < 9; ++i) ok = ok && isfinite(g[i]);
+                }
+                for (int i = 0; i < 9; ++i) G[(long long)j * 9 + i] = ok ? g[i] : G[(long long)(j - 1) * 9 + i];
+                conn[j] = ok;
+            }
+        }
+        for (int k = nf; k < n; ++k) {
             int found = 0;
             for (int d = 1; d <= span && d <= k && !found; ++d) {
                 const int l = adj_link(k - d, d, n);
@@ -1137,7 +1166,7 @@ __global__ void __launch_bounds__(256) adjust_init_kernel(int n, int span, AdjGe
     for (int l = tid; l < L; l += 256) {
         int t, d;
         nm_link_decode(l, n, t, d);
-        used[l] = conn[t] && conn[t + d] && usable(l);
+        used[l] = t + d >= nf && conn[t] && conn[t + d] && usable(l);
     }
 }
 
@@ -1232,13 +1261,13 @@ __global__ void __launch_bounds__(kAdjThreads) adjust_build_kernel(const Pairs P
 // One CTA: the Levenberg-Marquardt step.  Link totals (slices in order), the cost at x_eval (links in index order, +inf
 // when the build flagged a point); x_eval is accepted when it is the first point or lowers the cost (lambda / 10), else
 // rejected (lambda * 10).  A +inf cost at the first point ends the run there: the window keeps its initial poses.  After an
-// acceptance the banded normal equations of the unknowns (frame-major, half-bandwidth bw = P (span + 1) - 1; a
-// disconnected frame's rows are the identity with zero right-hand side) are assembled in link index order.  Unless the
+// acceptance the banded normal equations of the unknowns (frame-major, half-bandwidth bw = P (span + 1) - 1; the rows
+// of a disconnected or fixed frame k < nf are the identity with zero right-hand side) are assembled in link index order.  Unless the
 // run is over, (J^T J + lambda I) delta = -J^T r is solved by a banded Cholesky factorisation -- the last bw + 1 rows of
 // the factor kept in shared memory, the forward substitution folded into it, the back substitution by warp 0 -- and
 // x_eval = x_cur + delta.  A failed factorisation counts as a rejection.
 template <int KIND>
-__global__ void __launch_bounds__(kAdjSolveThreads) adjust_solve_kernel(int n, int span, const int* __restrict__ used,
+__global__ void __launch_bounds__(kAdjSolveThreads) adjust_solve_kernel(int n, int span, int nf, const int* __restrict__ used,
                                                                         const int* __restrict__ conn, const double* __restrict__ partial,
                                                                         double* __restrict__ link_tot, double* __restrict__ A,
                                                                         double* __restrict__ rhs, double* __restrict__ U,
@@ -1296,7 +1325,7 @@ __global__ void __launch_bounds__(kAdjSolveThreads) adjust_solve_kernel(int n, i
             double v = 0.0;
             if (j < m) {
                 const int k = i / NP + 1, a = i % NP, k2 = j / NP + 1, b = j % NP, dd = k2 - k;
-                if (!conn[k] || !conn[k2]) v = c == 0 ? 1.0 : 0.0;
+                if (k < nf || !conn[k] || !conn[k2]) v = c == 0 ? 1.0 : 0.0;   // k2 >= k is free if k is
                 else if (dd == 0) {
                     for (int d = 1; d <= span; ++d) {
                         if (k - d >= 0) { const int l = adj_link(k - d, d, n); if (used[l]) v += link_tot[(long long)l * E + NP * NP + a * NP + b]; }
@@ -1312,7 +1341,7 @@ __global__ void __launch_bounds__(kAdjSolveThreads) adjust_solve_kernel(int n, i
         for (int i = tid; i < m; i += kAdjSolveThreads) {
             const int k = i / NP + 1, a = i % NP;
             double v = 0.0;
-            if (conn[k])
+            if (k >= nf && conn[k])
                 for (int d = 1; d <= span; ++d) {
                     if (k - d >= 0) { const int l = adj_link(k - d, d, n); if (used[l]) v += link_tot[(long long)l * E + 3 * NP * NP + NP + a]; }
                     if (k + d < n) { const int l = adj_link(k, d, n); if (used[l]) v += link_tot[(long long)l * E + 3 * NP * NP + a]; }
@@ -1323,7 +1352,7 @@ __global__ void __launch_bounds__(kAdjSolveThreads) adjust_solve_kernel(int n, i
         if (tid == 0 && state->lambda < 0.0) {
             double mx = 0.0;
             for (int i = 0; i < m; ++i)
-                if (conn[i / NP + 1]) mx = fmax(mx, A[(long long)i * bw1]);
+                if (i / NP + 1 >= nf && conn[i / NP + 1]) mx = fmax(mx, A[(long long)i * bw1]);
             state->lambda = mx > 0.0 ? 1e-3 * mx : 1e-3;
         }
         __syncthreads();
@@ -1387,7 +1416,7 @@ __global__ void __launch_bounds__(kAdjSolveThreads) adjust_solve_kernel(int n, i
         if (!fail) {
             for (int i = tid; i < n * NP; i += kAdjSolveThreads) {
                 const int k = i / NP;
-                x_eval[i] = (k == 0 || !conn[k]) ? x_cur[i] : x_cur[i] + y[i - NP];
+                x_eval[i] = (k < nf || !conn[k]) ? x_cur[i] : x_cur[i] + y[i - NP];
             }
             return;
         }
@@ -1472,8 +1501,8 @@ __global__ void __launch_bounds__(256) adjust_finish_kernel(const Pairs P, float
 
 template <int KIND>
 int adjust_chain(const Pairs& P, int cost, float thr, int n, int span, int fw, int fh, const unsigned char* masks,
-                 const float* H_links, const int* link_status, int iterations, float* H_out, int* status_out, double* chain_out,
-                 double* report, cudaStream_t st)
+                 const float* H_links, const int* link_status, int n_fixed, const double* fixed_chain, const int* fixed_conn,
+                 int iterations, float* H_out, int* status_out, double* chain_out, double* report, cudaStream_t st)
 {
     constexpr int NP = AdjFam<KIND>::P, E = AdjFam<KIND>::E;
     const int L = nm_span_links(n, span), m = (n - 1) * NP, bw1 = NP * (span + 1);
@@ -1507,14 +1536,15 @@ int adjust_chain(const Pairs& P, int cost, float thr, int n, int span, int fw, i
     const double ext = (double)(fw > fh ? fw : fh);
     const AdjGeom geo{0.5 * (fw - 1), 0.5 * (fh - 1), 2.0 / ext};
     adjust_count_kernel<<<L, 256, 0, st>>>(P, masks, npts);
-    adjust_init_kernel<KIND><<<1, 256, 0, st>>>(n, span, geo, H_links, link_status, npts, G, conn, used, x_cur, x_eval, state);
+    adjust_init_kernel<KIND><<<1, 256, 0, st>>>(n, span, geo, H_links, link_status, npts, n_fixed, fixed_chain, fixed_conn, G, conn,
+                                                used, x_cur, x_eval, state);
     for (int it = 0; it < iterations; ++it) {
         if (cost == NM_ADJUST_MOSAIC)
             adjust_build_kernel<KIND, 0><<<dim3(L, kAdjSlices), kAdjThreads, 0, st>>>(P, masks, n, geo, used, x_eval, state, partial);
         else
             adjust_build_kernel<KIND, 1><<<dim3(L, kAdjSlices), kAdjThreads, 0, st>>>(P, masks, n, geo, used, x_eval, state, partial);
-        adjust_solve_kernel<KIND><<<1, kAdjSolveThreads, smem, st>>>(n, span, used, conn, partial, link_tot, A, rhs, U, x_cur, x_eval,
-                                                                     state, it == iterations - 1);
+        adjust_solve_kernel<KIND><<<1, kAdjSolveThreads, smem, st>>>(n, span, n_fixed, used, conn, partial, link_tot, A, rhs, U,
+                                                                     x_cur, x_eval, state, it == iterations - 1);
     }
     adjust_finish_kernel<KIND><<<n - 1, 256, 0, st>>>(P, thr, n, span, geo, H_links, conn, used, npts, x_cur, state, H_out, status_out,
                                                       chain_out, report);
@@ -1658,6 +1688,31 @@ extern "C" int nm_ransac_refine_batch_f32(int kind, const float* src_x, const fl
     return NM_OK;
 }
 
+extern "C" int nm_ransac_adjust_chain_fixed_f32(int kind, int cost, const float* src_x, const float* src_y, const float* dst_x,
+                                                const float* dst_y, long long pair_stride, const int* counts, int max_pts,
+                                                float inlier_threshold, int n_frames, int span, int frame_w, int frame_h,
+                                                const unsigned char* masks, const float* H_links, const int* link_status,
+                                                int n_fixed, const double* fixed_chain, const int* fixed_conn, int iterations,
+                                                float* H_out, int* status_out, double* chain_out, double* report_out,
+                                                nm_stream_t stream)
+{
+    if (kind < 0 || kind > 2 || max_pts <= 0 || pair_stride < 0 || iterations < 1 || frame_w <= 0 || frame_h <= 0) return NM_ERR_INVALID;
+    if (cost != NM_ADJUST_MOSAIC && cost != NM_ADJUST_TRANSFER) return NM_ERR_INVALID;
+    if (n_frames < 2 || n_frames > kAdjMaxFrames || span < 1 || span > kAdjMaxSpan || span >= n_frames) return NM_ERR_INVALID;
+    if (n_fixed < 1 || n_fixed >= n_frames || (n_fixed > 1 && !fixed_chain)) return NM_ERR_INVALID;
+    if (!src_x || !src_y || !dst_x || !dst_y || !masks || !H_links || !link_status || !H_out || !status_out) return NM_ERR_INVALID;
+    const Pairs P{src_x, src_y, dst_x, dst_y, pair_stride, counts, max_pts};
+    const cudaStream_t st = (cudaStream_t)stream;
+    if (kind == 0)
+        return adjust_chain<0>(P, cost, inlier_threshold, n_frames, span, frame_w, frame_h, masks, H_links, link_status, n_fixed,
+                               fixed_chain, fixed_conn, iterations, H_out, status_out, chain_out, report_out, st);
+    if (kind == 1)
+        return adjust_chain<1>(P, cost, inlier_threshold, n_frames, span, frame_w, frame_h, masks, H_links, link_status, n_fixed,
+                               fixed_chain, fixed_conn, iterations, H_out, status_out, chain_out, report_out, st);
+    return adjust_chain<2>(P, cost, inlier_threshold, n_frames, span, frame_w, frame_h, masks, H_links, link_status, n_fixed,
+                           fixed_chain, fixed_conn, iterations, H_out, status_out, chain_out, report_out, st);
+}
+
 extern "C" int nm_ransac_adjust_chain_cost_f32(int kind, int cost, const float* src_x, const float* src_y, const float* dst_x,
                                                const float* dst_y, long long pair_stride, const int* counts, int max_pts,
                                                float inlier_threshold, int n_frames, int span, int frame_w, int frame_h,
@@ -1665,20 +1720,9 @@ extern "C" int nm_ransac_adjust_chain_cost_f32(int kind, int cost, const float* 
                                                int iterations, float* H_out, int* status_out, double* chain_out, double* report_out,
                                                nm_stream_t stream)
 {
-    if (kind < 0 || kind > 2 || max_pts <= 0 || pair_stride < 0 || iterations < 1 || frame_w <= 0 || frame_h <= 0) return NM_ERR_INVALID;
-    if (cost != NM_ADJUST_MOSAIC && cost != NM_ADJUST_TRANSFER) return NM_ERR_INVALID;
-    if (n_frames < 2 || n_frames > kAdjMaxFrames || span < 1 || span > kAdjMaxSpan || span >= n_frames) return NM_ERR_INVALID;
-    if (!src_x || !src_y || !dst_x || !dst_y || !masks || !H_links || !link_status || !H_out || !status_out) return NM_ERR_INVALID;
-    const Pairs P{src_x, src_y, dst_x, dst_y, pair_stride, counts, max_pts};
-    const cudaStream_t st = (cudaStream_t)stream;
-    if (kind == 0)
-        return adjust_chain<0>(P, cost, inlier_threshold, n_frames, span, frame_w, frame_h, masks, H_links, link_status, iterations,
-                               H_out, status_out, chain_out, report_out, st);
-    if (kind == 1)
-        return adjust_chain<1>(P, cost, inlier_threshold, n_frames, span, frame_w, frame_h, masks, H_links, link_status, iterations,
-                               H_out, status_out, chain_out, report_out, st);
-    return adjust_chain<2>(P, cost, inlier_threshold, n_frames, span, frame_w, frame_h, masks, H_links, link_status, iterations,
-                           H_out, status_out, chain_out, report_out, st);
+    return nm_ransac_adjust_chain_fixed_f32(kind, cost, src_x, src_y, dst_x, dst_y, pair_stride, counts, max_pts, inlier_threshold,
+                                            n_frames, span, frame_w, frame_h, masks, H_links, link_status, 1, nullptr, nullptr,
+                                            iterations, H_out, status_out, chain_out, report_out, stream);
 }
 
 extern "C" int nm_ransac_adjust_chain_f32(int kind, const float* src_x, const float* src_y, const float* dst_x, const float* dst_y,

@@ -140,11 +140,20 @@ class StreamRegistrar:
     not refits kept; adjust_iterations bounds the LM builds per window; adjust_cost is adjust_chain's residual: MOSAIC,
     the default, or TRANSFER, which keeps long windows of similarity or homography models from contracting).  A frame
     that no usable link reaches keeps its predecessor's pose (status 0).  The result then depends on the window
-    boundaries -- lo and the chunk size -- and on nothing else.  span = 1 calls nothing new."""
+    boundaries -- lo and the chunk size -- and on nothing else.  span = 1 calls nothing new.
+
+    overlap O (1 <= O <= span; chunk >= O + 2 when O > 1) is the number of frames consecutive windows share: windows
+    start at lo, then at the previous window's end minus O.  The first window of a call is unanchored; every later one
+    holds its first O frames at the previous window's adjusted poses (adjust_chain(fixed=...): its last O chain rows,
+    connected flags from its status) and writes only the pairs whose later frame is free.  With O = span every link (t, t + d) lies
+    in the window where t + d is free, so no skip link is lost at a window boundary.  The extra cost is the SIFT and
+    matching of O - 1 more frames per window.  O = 1 (the default) is the behaviour above.  Windows are anchored within
+    one call on one rank only: the first window of each rank's range is unanchored, so ranks share no state and need
+    no collective (run(..., resume=True) continues a call on the same registrar)."""
 
     def __init__(self, sift_batch, chunk=None, kind: int = 2, ambiguity: float = 0.8, inlier_threshold: float = 4.0,
                  iterations: int = 1024, seed: int = 0, refine_rounds: int = 0, span: int = 1, adjust_iterations: int = 10,
-                 adjust_cost: int = MOSAIC):
+                 adjust_cost: int = MOSAIC, overlap: int = 1):
         import torch
         self.sb = sift_batch
         self.chunk = min(chunk or sift_batch.max_batch, sift_batch.max_batch)
@@ -153,16 +162,24 @@ class StreamRegistrar:
         self.refine_rounds = refine_rounds
         assert 1 <= span <= 8
         self.span, self.adjust_iterations, self.adjust_cost = span, adjust_iterations, adjust_cost
+        if not 1 <= overlap <= span:
+            raise ValueError(f"overlap {overlap}: expected 1 <= overlap <= span ({span})")
+        if overlap > 1 and self.chunk < overlap + 2:          # overlap 1 keeps the chunk >= 2 of unanchored windows
+            raise ValueError(f"chunk {self.chunk} < overlap + 2 ({overlap + 2})")
+        self.overlap = overlap
+        self._tail = None        # end of the last run: (hi, chain rows, conn, its last overlap - 1 pairs and status)
         cap, n = sift_batch.capacity, self.chunk - 1
         dev = torch.device("cuda", torch.cuda.current_device())
         self.match = torch.empty((n, cap), dtype=torch.int32, device=dev)
         self.corr = [torch.empty((n, cap), dtype=torch.float32, device=dev) for _ in range(4)]
 
-    def run(self, frames_of, lo: int, hi: int):
+    def run(self, frames_of, lo: int, hi: int, resume: bool = False):
         """frames_of(t0, t1) -> frames [t0, t1) of the stream on the device: cuda float32 (t1 - t0, h, w), or BGRA video
         frames, cuda uint8 (t1 - t0, h, w, 4), whose grey conversion is fused into the base blur (nm_sift_run_bgra) --
         the same colour buffer then feeds the mosaic (mosaic.render_stream).  Registers every pair (t, t + 1) with
-        lo <= t < hi - 1.  Returns (homographies (hi - lo - 1, 9), status (hi - lo - 1, 3)) on the device."""
+        lo <= t < hi - 1.  Returns (homographies (hi - lo - 1, 9), status (hi - lo - 1, 3)) on the device.
+        resume=True appends to the previous call (a live session): lo must be that call's hi - overlap, the first window
+        is anchored on the end of that call's last window, and the first overlap - 1 rows returned are that call's."""
         import ctypes as C
         import torch
         from . import _lib
@@ -170,11 +187,19 @@ class StreamRegistrar:
         from .sift import _stream_ptr
         lib = _lib.load()
         sb, cap = self.sb, self.sb.capacity
+        O = self.overlap
+        anchor = None                               # (chain rows, conn) the next window holds fixed
+        if resume:
+            if self._tail is None or lo != self._tail[0] - O or hi <= self._tail[0]:
+                raise ValueError("resume: needs a previous call, lo = its hi - overlap and hi > its hi")
+            anchor = self._tail[1:3] if O > 1 else None
         n_pairs = max(hi - lo - 1, 0)
         H = torch.zeros((max(n_pairs, 1), 9), dtype=torch.float32, device=self.match.device)
         st = torch.zeros((max(n_pairs, 1), 3), dtype=torch.int32, device=self.match.device)
         if n_pairs == 0:
             return H[:0], st[:0]
+        if resume and O > 1:
+            H[: O - 1], st[: O - 1] = self._tail[3], self._tail[4]
         r = sb.results()
         p = lambda t: C.c_void_p(t.data_ptr())
         c0 = lo
@@ -188,10 +213,22 @@ class StreamRegistrar:
                 sb.run(chunk)
             k = c0 - lo
             if self.span > 1:
-                adjust_window(r, n, min(self.span, n - 1), chunk.shape[2], chunk.shape[1], self.kind, self.ambiguity, self.thr,
-                              self.iters, self.seed + c0, self.refine_rounds, out=(H[k: k + n - 1], st[k: k + n - 1]),
-                              adjust_iterations=self.adjust_iterations, adjust_cost=self.adjust_cost)
-                c0 = c1 - 1
+                # an anchored window writes the pairs of its free frames only: the first O - 1 are the last window's
+                a = O - 1 if anchor is not None else 0
+                out = (H[k: k + n - 1], st[k: k + n - 1]) if a == 0 else None
+                Hw, Sw, chain, _ = adjust_window(r, n, min(self.span, n - 1), chunk.shape[2], chunk.shape[1], self.kind,
+                                                 self.ambiguity, self.thr, self.iters, self.seed + c0, self.refine_rounds,
+                                                 out=out, adjust_iterations=self.adjust_iterations,
+                                                 adjust_cost=self.adjust_cost, fixed=anchor)
+                if a:
+                    H[k + a: k + n - 1], st[k + a: k + n - 1] = Hw[a:], Sw[a:]
+                self._tail = (c1,)
+                if O > 1:
+                    anchor = (chain[n - O:], Sw[n - O - 1: n - 1, 0].clone(memory_format=torch.contiguous_format))
+                    self._tail += anchor + (Hw[n - O:].clone(), Sw[n - O:].clone())
+                if c1 >= hi:
+                    break
+                c0 = c1 - O
                 continue
             self.match[: n - 1].fill_(-1)
             check(lib.nm_match_pairs_f32(p(r["desc"]), p(r["counts"]), n, cap, self.ambiguity, p(self.match), None, None,
@@ -205,16 +242,17 @@ class StreamRegistrar:
                 check(lib.nm_ransac_refine_batch_f32(self.kind, *[p(c) for c in self.corr], cap, p(r["counts"]), cap, n - 1,
                                                      self.thr, p(H[k:]), p(st[k:]), self.refine_rounds, p(H[k:]), p(st[k:]),
                                                      None, _stream_ptr()), "nm_ransac_refine_batch_f32")
+            self._tail = (c1,)
             c0 = c1 - 1
         return H[:n_pairs], st[:n_pairs]
 
 
 def adjust_window(res, n, span, frame_w, frame_h, kind, ambiguity, inlier_threshold, iterations, seed, refine_rounds, out,
-                  adjust_iterations: int = 10, adjust_cost: int = MOSAIC):
+                  adjust_iterations: int = 10, adjust_cost: int = MOSAIC, fixed=None):
     """One adjustment window of StreamRegistrar(span > 1): frames 0 .. n-1 of the SIFT results `res` (SiftBatch.results())
     through the five public calls.  seed = the stream seed + the window's first frame.  Writes the window's n - 1 pairwise
-    models and status into out = (H, status); returns adjust_chain's (H, status, chain, report).  adjust_cost: adjust_chain's
-    cost (MOSAIC or TRANSFER)."""
+    models and status into out = (H, status), or new tensors when out is None; returns adjust_chain's (H, status, chain,
+    report).  adjust_cost and fixed: adjust_chain's cost (MOSAIC or TRANSFER) and fixed frames."""
     import torch
     from .match import match_pairs_span, link_row
     from .ransac import align_pairs_span, ransac_batch, refine_batch, adjust_chain
@@ -231,4 +269,4 @@ def adjust_window(res, n, span, frame_w, frame_h, kind, ambiguity, inlier_thresh
     link_counts = torch.cat([counts[: n - d] for d in range(1, span + 1)])
     HL, SL, mask = refine_batch(kind, *corr, link_counts, torch.cat(HL), torch.cat(SL), inlier_threshold, refine_rounds)
     return adjust_chain(kind, *corr, link_counts, span, mask, HL, SL, frame_w, frame_h, inlier_threshold, adjust_iterations, out=out,
-                        cost=adjust_cost)
+                        cost=adjust_cost, fixed=fixed)

@@ -145,8 +145,8 @@ def refine(kind, src_x, src_y, dst_x, dst_y, H, status, inlier_threshold, rounds
 
 
 def adjust_chain(kind, src_x, src_y, dst_x, dst_y, counts, span, masks, H, link_status, frame_w, frame_h, inlier_threshold,
-                 iterations=10, out=None, cost=MOSAIC):
-    """nm_ransac_adjust_chain_cost_f32 (arguments in the order of nm_ransac_adjust_chain_f32, then cost): joint
+                 iterations=10, out=None, cost=MOSAIC, fixed=None):
+    """nm_ransac_adjust_chain_fixed_f32 (arguments in the order of nm_ransac_adjust_chain_f32, then cost and fixed): joint
     least-squares adjustment of the poses of a window of n frames from the links of its span layout.  src_x ... dst_y
     (L, max_pts) and counts (L,) or None as for refine_batch; masks (L, max_pts) bool, H (L, 9) the link models and
     link_status (L, 3), as refine_batch returns them (rows 0 .. n-2 are the consecutive pairs).  inlier_threshold: the
@@ -157,7 +157,10 @@ def adjust_chain(kind, src_x, src_y, dst_x, dst_y, counts, span, masks, H, link_
     links used]).  cost: MOSAIC (the default, nm_ransac_adjust_chain_f32) measures a link's residual in frame-0 pixels,
     TRANSFER in the pixels of its target frame t + d, which does not reward shrinking the frames far from frame 0 (long
     windows of similarity or homography models).  With TRANSFER a point behind the target camera at the initial poses
-    leaves the window unadjusted (report costs +inf)."""
+    leaves the window unadjusted (report costs +inf).  fixed = (chain (n_fixed, 9) float64, conn (n_fixed,) int32 or None),
+    cuda tensors, 1 <= n_fixed <= n - 1: frames 0 .. n_fixed-1 keep the poses chain[j] (any common frame: the rows are
+    rebased on chain[0]) and only links reaching a later frame are used -- for example the last rows of the previous
+    window's chain and its status[:, 0] as conn (entry 0 is ignored).  None: n_fixed = 1, the window on its own."""
     import torch
     _f32(src_x, src_y, dst_x, dst_y)
     if counts is not None:
@@ -181,11 +184,24 @@ def adjust_chain(kind, src_x, src_y, dst_x, dst_y, counts, span, masks, H, link_
         _int32(st_out, "status_out")
         if tuple(st_out.shape) != (n - 1, 3):
             raise TypeError("status_out: expected shape (n - 1, 3)")
+    n_fixed, fchain, fconn = 1, None, None
+    if fixed is not None:
+        fchain, fconn = fixed
+        if not (isinstance(fchain, torch.Tensor) and fchain.is_cuda and fchain.dtype == torch.float64 and fchain.is_contiguous()
+                and fchain.dim() == 2 and fchain.shape[1] == 9):
+            raise TypeError("fixed chain: expected a contiguous cuda float64 tensor of shape (n_fixed, 9)")
+        n_fixed = fchain.shape[0]
+        if fconn is not None:
+            _int32(fconn, "fixed conn")
+            if tuple(fconn.shape) != (n_fixed,):
+                raise TypeError("fixed conn: expected shape (n_fixed,)")
     chain = torch.empty((n, 9), dtype=torch.float64, device=H.device)
     report = torch.empty(4, dtype=torch.float64, device=H.device)
-    check(_lib.load().nm_ransac_adjust_chain_cost_f32(kind, cost, _p(src_x), _p(src_y), _p(dst_x), _p(dst_y), max_pts,
-                                                      _p(counts) if counts is not None else None, max_pts, inlier_threshold, n,
-                                                      span, frame_w, frame_h, _p(masks), _p(H), _p(link_status), iterations,
-                                                      _p(H_out), _p(st_out), _p(chain), _p(report), _stream_ptr()),
-          "nm_ransac_adjust_chain_cost_f32")
+    check(_lib.load().nm_ransac_adjust_chain_fixed_f32(kind, cost, _p(src_x), _p(src_y), _p(dst_x), _p(dst_y), max_pts,
+                                                       _p(counts) if counts is not None else None, max_pts, inlier_threshold, n,
+                                                       span, frame_w, frame_h, _p(masks), _p(H), _p(link_status), n_fixed,
+                                                       _p(fchain) if fchain is not None else None,
+                                                       _p(fconn) if fconn is not None else None, iterations,
+                                                       _p(H_out), _p(st_out), _p(chain), _p(report), _stream_ptr()),
+          "nm_ransac_adjust_chain_fixed_f32")
     return H_out, st_out, chain, report

@@ -10,7 +10,13 @@ true inliers, and the 2 048-frame 1080p StreamRegistrar rate of bench.py with re
 window of each stage at span 1, 2, 3 (the frames of bench.py's stream, CUDA events, the spans in alternating windows),
 the adjustment with the mosaic and the transfer cost, the 2 048-frame 1080p StreamRegistrar rate at span 1, 2, 3 with
 refine_rounds 0 and 2 (span 3 with either cost), and the last frame's corner error on the synthetic 64-frame windows of
-tests/test_gpu_chain_adjust.py for chained span-1 refits and the span-2 / span-3 adjustment with either cost."""
+tests/test_gpu_chain_adjust.py for chained span-1 refits and the span-2 / span-3 adjustment with either cost.
+
+--adjust --overlap O: the window-overlap leg instead (StreamRegistrar(span=3, overlap=O), adjust_chain(fixed=...)):
+time per 64-frame and per 8-frame 1080p window (the five public calls, transfer cost) unanchored against anchored on O
+fixed frames, in alternating windows; the 2 048-frame 1080p StreamRegistrar rate at span 3 (transfer cost, two refit
+rounds) with overlap 1 and O; and the drift figures of tests/test_gpu_chain_adjust_fixed.py (synthetic 120-frame
+streams in 8-frame windows, the SIFT crop stream) with overlap 1 and O."""
 import os
 import subprocess
 import sys
@@ -201,6 +207,76 @@ def adjust_leg():
                   f"({m[3, cost] / m[1]:.3f})")
 
 
+def overlap_leg(O):
+    import bench
+    from niftymatch_b200.dist import StreamRegistrar, adjust_window
+    from tests.test_gpu_chain_adjust import _crop_stream, _stream_errors
+    from tests.test_gpu_chain_adjust_fixed import drift_ratio
+    _card()
+    stream_np = bench.render_frames(bench.stream_jobs(0, 32))
+    P = nm.SiftParams(bench.W, bench.H)
+    sb = nm.SiftBatch(P, bench.BATCH, bench.CAPACITY)
+    base = torch.from_numpy(stream_np).cuda()
+    frames_of = lambda t0, t1: base.index_select(0, torch.arange(t0, t1, device="cuda") % base.shape[0])
+    span, kind, thr, iters = 3, 2, 4.0, 1024
+    sb.run(frames_of(0, sb.max_batch))
+    r = sb.results()
+    for n in (sb.max_batch, 8):
+        win = lambda fixed: adjust_window(r, n, span, bench.W, bench.H, kind, 0.8, thr, iters, 0, 2, None, adjust_cost=nm.TRANSFER,
+                                          fixed=fixed)
+        fixed = (win(None)[2][:O].contiguous(), None)            # frames 0 .. O-1 at their adjusted poses
+        times = {1: [], O: []}
+        for rep in range(7):
+            for o in (1, O):
+                e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+                e0.record()
+                win(None if o == 1 else fixed)
+                e1.record()
+                torch.cuda.synchronize()
+                if rep >= 1:
+                    times[o].append(e0.elapsed_time(e1))
+        print(f"one {n}-frame 1080p window (match, align, RANSAC, refit, adjust; transfer cost): " + ", ".join(
+            f"overlap {o} {np.median(times[o]):.2f} ms (windows {min(times[o]):.2f} - {max(times[o]):.2f}), "
+            f"{np.median(times[o]) / (n - o):.3f} ms per new frame" for o in (1, O)))
+    n_stream = 2048
+    for rep in range(2):
+        for o in (1, O):
+            reg = StreamRegistrar(sb, chunk=sb.max_batch, refine_rounds=2, span=span, adjust_cost=nm.TRANSFER, overlap=o)
+            reg.run(frames_of, 0, sb.max_batch + 1)
+            torch.cuda.synchronize()
+            e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+            e0.record()
+            Hs, sts = reg.run(frames_of, 0, n_stream)
+            e1.record()
+            torch.cuda.synchronize()
+            ms = e0.elapsed_time(e1)
+            print(f"stream {n_stream} frames 1080p, span 3 (transfer cost), refine_rounds 2, overlap {o}: "
+                  f"{n_stream / ms * 1e3:.0f} frames/s ({ms:.1f} ms), connected pairs {int((sts[:, 0] == 1).sum())}")
+    sb.close()
+    for kind, streams in ((0, 64), (1, 16), (2, 16)):
+        a, b = drift_ratio(nm, kind, streams, O=O)
+        print(f"synthetic 120-frame streams ({streams}), kind {kind}, 8-frame windows, span 3, transfer cost: last frame mean "
+              f"squared corner error, overlap 1 {a:.3e} px^2, overlap {O} {b:.3e} px^2, ratio {b / a:.3f}")
+    w, h, n, offs, bgra = _crop_stream()
+    fr = torch.from_numpy(bgra).cuda()
+    Pc = nm.SiftParams(w, h)
+    Pc._peak_threshold = 2.0
+    sbc = nm.SiftBatch(Pc, 8, 8192)
+    for cost in (nm.MOSAIC, nm.TRANSFER):
+        errs = {}
+        for o in (1, O):
+            reg = StreamRegistrar(sbc, chunk=8, kind=nm.HOMOGRAPHY, inlier_threshold=0.25, iterations=512, seed=3, refine_rounds=2,
+                                  span=3, adjust_cost=cost, overlap=o)
+            H, st = reg.run(lambda t0, t1: fr[t0:t1].contiguous(), 0, n)
+            errs[o] = _stream_errors(nm, H, st, w, h, offs)
+        print(f"24-frame SIFT crop stream, homography, chunk 8, span 3, {'transfer' if cost else 'mosaic'} cost: worst corner "
+              f"error, overlap 1 {errs[1]:.3f} px, overlap {O} {errs[O]:.3f} px")
+    sbc.close()
+
+
+if "--adjust" in sys.argv and "--overlap" in sys.argv:
+    overlap_leg(int(sys.argv[sys.argv.index("--overlap") + 1]))
+    sys.exit(0)
 if "--adjust" in sys.argv:
     adjust_leg()
     sys.exit(0)
